@@ -28,6 +28,9 @@ exactly K timed ones, the timed region starting at a fresh solve.
             with the CPU oracle timed on the SAME graph where it can be run in seconds
   cpu_baseline  the CPU oracle (g2o-faithful LM: numeric Jacobians h=1e-9, sparse LDL^T) on a bounded sample
 
+--dump-outputs DIR writes what the last timed step returned (estimates, chi2, lambda, LM history) as DIR/<name>.npy,
+so that two builds run with the same arguments, hence the same seeded graph, can be compared output for output.
+
 --impl reference times the CPU oracle alone (the reference itself cannot be built here: g2o/Eigen/Sophus/TooN
 are absent and there is no network; SURVEY.md 8c): same `config`, every step an LM iteration on a bounded sample
 (s10k) of the workload, `value` scaled to the workload by the edge ratio and flagged `extrapolated`.
@@ -62,6 +65,7 @@ KITTI_DIR = os.path.join(ROOT, "tests", "golden", "kitti00")
 GOLDEN_S10K = os.path.join(ROOT, "tests", "golden", "s10k_oracle100.npz")
 # BASELINE.json north_star tolerances
 TOL_CHI2, TOL_TRANS, TOL_ROT = 1e-4, 1e-4, 1e-5
+DUMP_ROWS = 500_000          # --dump-outputs: 32 MB of float64 estimates at most (the s1m estimates are 64 MB)
 
 
 def parse_args():
@@ -80,7 +84,14 @@ def parse_args():
     ap.add_argument("--no-configs", action="store_true", help="skip the sub-records of the other BASELINE configs")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--seed", type=int, default=42)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 class ClockSampler:
@@ -149,6 +160,19 @@ def common_config(args):
             "free_vertices": nv - 1, "block_dim": 7, "math_mode": "corrected",
             "step": "one LM iteration of a complete solve (initial guess -> the reference's optimize(100) answer)",
             "l2_policy": "inputs larger than L2 (Hessian blocks %.2f GB)" % (392 * (nv - 1 + ne) / 1e9)}
+
+
+def dump_outputs(out_dir, est, chi2, lam, hist):
+    """What the last timed step (one s3o_optimize call) returned to its caller, as float64 .npy files: the estimates
+    (every row up to DUMP_ROWS, else a fixed seeded sample of DUMP_ROWS rows whose indices are in estimate_rows),
+    chi2, lambda and the LM history rows [chi2, lambda, trials, rho, PCG iterations]."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.arange(len(est))
+    if len(est) > DUMP_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(len(est), DUMP_ROWS, replace=False))
+    arrays = {"estimates": est[rows], "estimate_rows": rows, "chi2": [chi2], "lambda": [lam], "lm_history": hist}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def pose_diff(a, b):
@@ -552,6 +576,7 @@ def run_ours(args):
             if self.in_solve == 0:
                 prob.restore_estimates()
             n, chi2, lam, hist = prob.optimize(1, 0.0)
+            self.last = (chi2, lam, hist)
             self.in_solve += 1
             self.cur.append(chi2)
             self.trace.append([float(v) for v in np.asarray(hist).reshape(-1)[:5]])
@@ -600,6 +625,8 @@ def run_ours(args):
         k0 += len(sv)
     st = prob.stats()
     timed_trace = list(drv.trace)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, prob.vertices(), *drv.last)
     if world > 1:
         t = torch.tensor([ms], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
