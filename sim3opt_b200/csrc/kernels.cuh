@@ -117,11 +117,10 @@ int spmv3_tile_blocks(int d);
 void launch_spmv3(int d, const double *H, const StructDev &s, int nf, double lambda, const double *p, double *q1,
                   double *T, double *partials, DevScalars *sc, int pcg_mode, int grid_cap, int dist, cudaStream_t st);
 // v4 (d = 7 only): v3 + descriptor staging, register-pipelined index / vector prefetch, NS-deep ring
-int spmv4_tile_blocks();
-void spmv4_set_cfg(int cfg);
+int spmv4_tile_blocks(int cfg);
 bool spmv4_fits(int ntiles, int grid_cap);
 void launch_spmv4(const double *H, const StructDev &s, int nf, double lambda, const double *p, double *q1, double *T,
-                  double *partials, DevScalars *sc, int pcg_mode, int grid_cap, int dist, cudaStream_t st);
+                  double *partials, DevScalars *sc, int pcg_mode, int cfg, int grid_cap, int dist, cudaStream_t st);
 void launch_spmv2(int d, const double *H, const StructDev &s, int nf, double lambda, const double *p, double *q1,
                   double *T, double *partials, DevScalars *sc, int pcg_mode, int dist, cudaStream_t st);
 

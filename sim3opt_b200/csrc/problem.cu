@@ -173,7 +173,7 @@ void run_spmv(s3o_problem *p, const StructDev &s, double lambda, const double *x
         StructDev s4 = s;
         if (p->p2p && x == p->d_p) s4.ghost_src = p->d_ghost_src;      // ghost columns read from the owners' p
         launch_spmv4(p->d_H, s4, own_rows(p), lambda, x, p->d_q1, p->d_T, p->d_partials, p->d_sc, pcg_mode,
-                     p->spmv_grid_cap, p->dist, p->stream);
+                     p->spmv4_cfg, p->spmv_grid_cap, p->dist, p->stream);
     }
     else if (p->spmv_version >= 3 && p->S.max_row_blocks <= p->S.tile_blocks)
         launch_spmv3(p->d, p->d_H, s, own_rows(p), lambda, x, p->d_q1, p->d_T, p->d_partials, p->d_sc, pcg_mode,
@@ -385,7 +385,7 @@ int upload_structure_arrays(s3o_problem *p, int rows_own, bool on_device) {
     }
     S.max_row_blocks = 0;
     for (int r = 0; r < rows_own; ++r) S.max_row_blocks = std::max(S.max_row_blocks, S.rowptr[r + 1] - S.rowptr[r]);
-    S.tile_blocks = (p->spmv_version == 4 && p->d == 7) ? spmv4_tile_blocks()
+    S.tile_blocks = (p->spmv_version == 4 && p->d == 7) ? spmv4_tile_blocks(p->spmv4_cfg)
                     : (p->spmv_version >= 3 ? spmv3_tile_blocks(p->d) : spmv_tile_blocks(p->d));
     build_tiles(S.rowptr, rows_own, S.tile_blocks, S.tile_row);
     rc = rc ? rc : upload(p, &p->d_tile_row, S.tile_row);
@@ -525,8 +525,14 @@ static int create_impl(int kind, int linear_dim, int device, s3o_problem **out) 
     if (spmv2_configure() != 0) { set_error("s3o_create: cannot configure SpMV shared memory"); delete p; return S3O_ERR_CUDA; }
     if (const char *v = getenv("S3O_TRACE")) { p->trace_state = atoi(v) > 0 ? 1 : 0; p->trace_solve = atoi(v); }    // trace the n-th solve
     if (const char *v = getenv("S3O_SPMV_VERSION")) p->spmv_version = atoi(v);
-    if (const char *v = getenv("S3O_SPMV_GRID")) p->spmv_grid_cap = atoi(v);
-    if (const char *v = getenv("S3O_SPMV4_CFG")) spmv4_set_cfg(atoi(v));
+    if (const char *v = getenv("S3O_SPMV_GRID")) {      // every CTA of the SpMV owns one of the kMaxPartials p.q partials
+        const int g = atoi(v);
+        if (g >= 1 && g <= kMaxPartials) p->spmv_grid_cap = g;
+    }
+    if (const char *v = getenv("S3O_SPMV4_CFG")) {
+        const int c = atoi(v);
+        if (c >= 0 && c <= 2) p->spmv4_cfg = c;
+    }
     if (const char *v = getenv("S3O_PRECOND")) {        // experiment switch; s3o_set_preconditioner overrides it
         const int k = atoi(v);
         if (k >= S3O_PRECOND_AUTO && k <= S3O_PRECOND_MULTILEVEL && (k != S3O_PRECOND_MULTILEVEL || kind != S3O_KIND_BA)) p->precond = k;

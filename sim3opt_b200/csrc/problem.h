@@ -79,7 +79,8 @@ struct s3o_problem {
     int n_peers = 0;
     std::vector<void *> ipc_mapped;            // to cudaIpcCloseMemHandle
     int spmv_version = 4;       // 1: lane-group rows, 2: tiled thread-per-block, 3: v2 + TMA ring, 4: v3 + prefetch pipeline (d = 7)
-    int spmv_grid_cap = 148 * 2;
+    int spmv_grid_cap = 148 * 2;            // persistent SpMV grid; S3O_SPMV_GRID in [1, kMaxPartials]
+    int spmv4_cfg = 0;          // v4 tile / ring: 0: TB=112 NS=2, 1: TB=80 NS=3, 2: TB=56 NS=4; fixes the tiles of this problem
     // linear system
     double *d_H = nullptr, *d_b = nullptr, *d_x = nullptr, *d_r = nullptr, *d_z = nullptr, *d_p = nullptr;
     double *d_q1 = nullptr, *d_T = nullptr, *d_Minv = nullptr, *d_scratch = nullptr, *d_partials = nullptr;

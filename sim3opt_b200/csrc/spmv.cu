@@ -514,9 +514,9 @@ template <int TB, int NS>
 constexpr size_t spmv4_smem_bytes() {
     return sizeof(double) * (size_t)(NS * (TB * 49 + 2) + 2 * TB * 7 + TB) + 8 * NS + 4 * 4 * (Spmv4Cfg::KMAX + 1) + 16;
 }
-static int g_spmv4_cfg = 0;     // 0: TB=112 NS=2, 1: TB=80 NS=3, 2: TB=56 NS=4   (S3O_SPMV4_CFG)
-int spmv4_tile_blocks() { return g_spmv4_cfg == 0 ? 112 : (g_spmv4_cfg == 1 ? 80 : 56); }
-void spmv4_set_cfg(int cfg) { g_spmv4_cfg = cfg < 0 || cfg > 2 ? 0 : cfg; }
+// cfg 0: TB=112 NS=2, 1: TB=80 NS=3, 2: TB=56 NS=4 (S3O_SPMV4_CFG, per problem).  The tiles are cut for the TB of
+// the problem's cfg, so launch_spmv4 must get that same cfg: a smaller TB overruns the ring slot and ys / ts / wt.
+int spmv4_tile_blocks(int cfg) { return cfg == 0 ? 112 : (cfg == 1 ? 80 : 56); }
 // persistent grid: grid_cap CTAs (2 per SM); a graph with more than grid_cap * KMAX tiles gets the next
 // multiple of grid_cap that keeps every CTA's descriptor list within KMAX
 static int spmv4_grid(int ntiles, int grid_cap) {
@@ -530,11 +530,11 @@ bool spmv4_fits(int ntiles, int grid_cap) {
 }
 
 void launch_spmv4(const double *H, const StructDev &s, int nf, double lambda, const double *p, double *q1, double *T,
-                  double *partials, DevScalars *sc, int pcg_mode, int grid_cap, int dist, cudaStream_t st) {
+                  double *partials, DevScalars *sc, int pcg_mode, int cfg, int grid_cap, int dist, cudaStream_t st) {
     if (nf == 0 || s.ntiles == 0) return;
     const int grid = spmv4_grid(s.ntiles, grid_cap);
     constexpr int NT = Spmv4Cfg::NT, KM = Spmv4Cfg::KMAX;
-    switch (g_spmv4_cfg) {
+    switch (cfg) {
     case 0: spmv4_kernel<7, NT, 112, 2, KM><<<grid, NT, spmv4_smem_bytes<112, 2>(), st>>>(H, s, nf, lambda, p, q1, T, partials, sc, pcg_mode, dist); break;
     case 1: spmv4_kernel<7, NT, 80, 3, KM><<<grid, NT, spmv4_smem_bytes<80, 3>(), st>>>(H, s, nf, lambda, p, q1, T, partials, sc, pcg_mode, dist); break;
     case 2: spmv4_kernel<7, NT, 56, 4, KM><<<grid, NT, spmv4_smem_bytes<56, 4>(), st>>>(H, s, nf, lambda, p, q1, T, partials, sc, pcg_mode, dist); break;

@@ -9,6 +9,7 @@ import pytest
 
 from conftest import make_gpu, make_oracle
 from test_gpu_parity import dense_from_blocks
+from test_gpu_spmv_shapes import backward_error
 
 pytestmark = pytest.mark.gpu
 
@@ -128,7 +129,8 @@ def test_scale_null_vector_multilevel(kitti_k118):
 def test_kcycle_fewer_iterations_same_solution():
     """K-cycle (two inner CG steps on the largest coarse levels, one cooperative kernel for the small ones)
     against the V-cycle on a 9k-pose sphere at a late-iteration linearisation point and damping: same solution
-    (backward error against the same H and b), fewer iterations, bitwise reproducible."""
+    (backward error against the same H and b, with a host product independent of the device SpMV the PCG uses), fewer
+    iterations, bitwise reproducible."""
     import os
     import sim3opt_b200 as s3
     from sim3opt_b200 import synth
@@ -144,6 +146,7 @@ def test_kcycle_fewer_iterations_same_solution():
         try:
             gpu = make_gpu(g, jac=1, math_mode=s3.MATH_CORRECTED)
             gpu.set_preconditioner(s3.PRECOND_MULTILEVEL)
+            colptr, rowidx = gpu.build_structure()
             H, b = gpu.linearize()
             lam = 1e-10 * gpu.max_diag()
             gpu.set_pcg(1e-10, 50000)
@@ -153,6 +156,7 @@ def test_kcycle_fewer_iterations_same_solution():
         finally:
             del os.environ["S3O_KCYCLE"]
         assert rc == 0 and rel <= 1e-10
+        assert backward_error(colptr, rowidx, H, lam, x, b) <= 1e-9
         assert np.linalg.norm(y - b) <= 1e-9 * np.linalg.norm(b)
         assert it2 == it and np.array_equal(x, x2)
         res[k] = (x, it)
@@ -167,7 +171,8 @@ def test_kcycle_fewer_iterations_same_solution():
 def test_large_graph_kcycle_with_dense_coarsest_level():
     """Graphs of >= 20 000 free vertices take the production path of the 1M-pose benchmark: K-cycle levels inside the
     persistent kernel and a coarsest level of up to 128 vertices inverted by the row-resident block Gauss-Jordan.
-    A wrong coarse inverse or Galerkin operator shows as a stalled PCG; the solution is checked against H itself."""
+    A wrong coarse inverse or Galerkin operator shows as a stalled PCG; the solution is checked against H itself, with a
+    host product (the device SpMV is what the PCG runs, so it cannot be the judge)."""
     import sim3opt_b200 as s3
     from sim3opt_b200 import synth
     g = dict(synth.sphere(n_laps=30, poses_per_lap=1000, seed=7))
@@ -177,6 +182,7 @@ def test_large_graph_kcycle_with_dense_coarsest_level():
     g["est"] = warm.vertices()
     del warm
     gpu = make_gpu(g, jac=1, math_mode=s3.MATH_CORRECTED)
+    colptr, rowidx = gpu.build_structure()
     H, b = gpu.linearize()
     gpu.set_pcg(1e-10, 5000)
     out = []
@@ -184,6 +190,7 @@ def test_large_graph_kcycle_with_dense_coarsest_level():
         lam = lam_rel * gpu.max_diag()
         rc, x, it, rel = gpu.solve(lam)
         assert rc == 0 and rel <= 1e-10, (lam_rel, rc, it, rel)
+        assert backward_error(colptr, rowidx, H, lam, x, b) <= 1e-9
         y = gpu.hessian_multiply(lam, x)
         assert np.linalg.norm(y - b) <= 1e-9 * np.linalg.norm(b)
         assert it <= 600, (lam_rel, it)
