@@ -9,7 +9,8 @@
 // key-frame order, vertex 0 fixed, loop edges first, then the odometry edges, Omega = I.
 //
 // usage: kitti_pgo direct   <dataDir> <outFile> [--all-loops] [--iters N] [--numeric] [--pcg-tol T] [--precision P]
-//        kitti_pgo stepwise <dataDir> <outFile> [--all-loops] [--stages 2|3] [--no-stepwise] [--iters N]
+//                           [--marginals FILE]
+//        kitti_pgo stepwise <dataDir> <outFile> [--all-loops] [--stages 2|3] [--no-stepwise] [--iters N] [--marginals FILE]
 //        kitti_pgo dry-run  <dataDir> [--all-loops]        (no GPU: loads, builds, prints structure sizes)
 //        kitti_pgo align    <resultFile> <gtPoseFile> [--only-scale]   (kitti_surf.cpp:1381-1452: Umeyama + RMSE)
 //        kitti_pgo reproject <keyFrameDir> <resultFile> <out.bal>       (drawPTAMPoints.cpp:285-456: map -> BAL)
@@ -30,7 +31,7 @@ using std::vector;
 namespace {
 
 struct Options {
-    string mode, dataDir, outFile;
+    string mode, dataDir, outFile, marginalsFile;
     bool oneConstraint = true, stepwise = true, numeric = false;
     int stages = 2, iters = 100, precision = 6;
     double pcgTol = 1e-13;
@@ -114,6 +115,31 @@ void buildSim3Graph(g2o::SparseOptimizer &optimizer, const vector<KeyFrame> &kfs
     }
 }
 
+// --marginals FILE: the d x d block of H^-1 at the final estimates (g2o computeMarginals) of every free key frame,
+// one line each: key-frame id, then the block row by row
+bool writeMarginals(const Options &o, const vector<KeyFrame> &kfs, g2o::SparseOptimizer &opt, int d) {
+    if (o.marginalsFile.empty()) return true;
+    g2o::SparseOptimizer::VertexContainer freeVertices;
+    for (const KeyFrame &kf : kfs)
+        if (!opt.vertex(kf.mnFrameId)->fixed()) freeVertices.push_back(opt.vertex(kf.mnFrameId));
+    g2o::SparseBlockMatrix<g2o::MatrixX> spinv;
+    if (!opt.computeMarginals(spinv, freeVertices)) { std::cerr << "computeMarginals: " << opt.lastError() << "\n"; return false; }
+    FILE *f = std::fopen(o.marginalsFile.c_str(), "w");
+    if (!f) { std::cerr << "cannot write " << o.marginalsFile << "\n"; return false; }
+    std::fprintf(f, "%% marginal covariance of each free key frame: kf id, %dx%d block of H^-1 (row-major)\n", d, d);
+    for (const KeyFrame &kf : kfs) {
+        const g2o::Vertex *v = opt.vertex(kf.mnFrameId);
+        if (v->fixed()) continue;
+        const g2o::MatrixX *b = spinv.block(v->hessianIndex(), v->hessianIndex());
+        std::fprintf(f, "%d", kf.mnId);
+        for (int k = 0; k < d * d; ++k) std::fprintf(f, " %.17g", b->data()[k]);
+        std::fprintf(f, "\n");
+    }
+    std::fclose(f);
+    std::cout << "saved marginals file " << o.marginalsFile << "\n";
+    return true;
+}
+
 template <class GetSim3>
 void writeResult(const Options &o, const vector<KeyFrame> &kfs, const char *header, GetSim3 get) {
     std::ofstream log(o.outFile);
@@ -154,6 +180,7 @@ int runDirect(const Options &o) {
     profiler.stop("optimize");
     if (iters <= 0) { std::cerr << "optimize: " << optimizer.lastError() << "\n"; return 3; }
     report("direct", optimizer, iters);
+    if (!writeMarginals(o, kfs, optimizer, 7)) return 3;
     writeResult(o, kfs, "% sim3 optimization result: kf id, sw2i, scaled tiinw, ri2w(qxyzw):", [&](int id) {
         return static_cast<vio::VertexSim3Expmap *>(optimizer.vertex(id))->estimate();
     });
@@ -251,6 +278,7 @@ int runStepwise(const Options &o) {
         profiler.stop("scale_trans");
         if (it <= 0) { std::cerr << "scale_trans optimize: " << optimizerST.lastError() << "\n"; return 3; }
         report("scale_trans", optimizerST, it);
+        if (num_optimizer != 3 && !writeMarginals(o, kfs, optimizerST, 4)) return 3;
     }
     auto stToSim3 = [&](int id) {
         vio::G2oVertexScaleTrans *vST = static_cast<vio::G2oVertexScaleTrans *>(optimizerST.vertex(id));
@@ -266,6 +294,7 @@ int runStepwise(const Options &o) {
         profiler.stop("sim3_optim");
         if (it <= 0) { std::cerr << "sim3 optimize: " << optimizerSim3.lastError() << "\n"; return 3; }
         report("sim3_optim", optimizerSim3, it);
+        if (!writeMarginals(o, kfs, optimizerSim3, 7)) return 3;
     }
     writeResult(o, kfs, "% sim3 optimization result: kf frameid, sw2i, scaled tiinw, ri2w(qxyzw):", [&](int id) {
         return num_optimizer == 3 ? static_cast<vio::VertexSim3Expmap *>(optimizerSim3.vertex(id))->estimate() : stToSim3(id);
@@ -323,7 +352,7 @@ int main(int argc, char **argv) {
     Options o;
     if (argc < 3) {
         std::cerr << "usage: kitti_pgo direct|stepwise|dry-run <dataDir> [<outFile>] [--all-loops] [--stages 2|3] [--no-stepwise]"
-                     " [--iters N] [--numeric] [--pcg-tol T] [--precision P]\n";
+                     " [--iters N] [--numeric] [--pcg-tol T] [--precision P] [--marginals FILE]\n";
         return 1;
     }
     o.mode = argv[1];
@@ -351,6 +380,7 @@ int main(int argc, char **argv) {
         else if (a == "--iters" && k + 1 < argc) o.iters = std::atoi(argv[++k]);
         else if (a == "--precision" && k + 1 < argc) o.precision = std::atoi(argv[++k]);
         else if (a == "--pcg-tol" && k + 1 < argc) o.pcgTol = std::atof(argv[++k]);
+        else if (a == "--marginals" && k + 1 < argc) o.marginalsFile = argv[++k];
         else { std::cerr << "unknown option " << a << "\n"; return 1; }
     }
     if (o.mode != "dry-run") {

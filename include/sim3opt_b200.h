@@ -200,6 +200,23 @@ int s3o_update(s3o_problem *p, const double *x);
 int s3o_smallest_eigenvector(s3o_problem *p, int max_iter, double tol, double *x, double *lambda_min,
                              double *lambda_max, int *iterations);
 
+/* Marginal covariances: blocks of H^-1, where H = J^T Omega' J is the Gauss-Newton Hessian (robust weights
+ * included, no LM damping) linearised at the CURRENT estimates, in the tangent of the left update S <- exp(d) S
+ * (Sim3 [omega upsilon sigma], scale-trans [s t], scale [s]).  g2o SparseOptimizer::computeMarginals.
+ * rows/cols: n_pairs Hessian indices (s3o_get_hessian_index; fixed vertices have none); out: n_pairs x d x d,
+ * row-major, block (rows[k], cols[k]).  rows == cols == NULL: every diagonal block in Hessian order
+ * (n_pairs must equal n_free).  S3O_ERR_SOLVE when H is singular (a connected component without a fixed
+ * vertex); S3O_ERR_UNSUPPORTED for BA, the partitioned solve, and graphs whose factor exceeds the forced cap.
+ * Every call linearises again at the current estimates, so the result does not depend on what ran before it
+ * (g2o uses the H of its last buildSystem, which is one step behind the estimates optimize() returns).  H is
+ * factorised by the sparse block Cholesky (a plan under the forced cap of s3o_set_linear_solver(DIRECT) when the
+ * linear solver in use has none; the linear solver the LM picks does not change), and the selected inverse gives
+ * every block on the pattern of the factor -- all diagonal blocks and every pair joined by an edge -- for about
+ * twice the block products of the factorisation.  A pair off that pattern costs d triangular solves for each
+ * distinct column vertex among such pairs.  Like s3o_smallest_eigenvector, the call leaves the problem
+ * unlinearised (s3o_solve needs s3o_linearize again). */
+int s3o_compute_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out);
+
 /* ---- the hot call (replaces optimizer.optimize(n)) ------------------------------------- */
 /* hist (may be NULL): per LM iteration [chi2, lambda, trials, rho, pcg_iters]; returns via
  * out-params the number of iterations run (g2o's return value), final chi2 and lambda.

@@ -85,6 +85,53 @@ private:
     double s_;
 };
 
+// ---- g2o::MatrixX and g2o::SparseBlockMatrix<MatrixX>: what computeMarginals fills -------------------------
+class MatrixX {      // dense, row-major
+public:
+    MatrixX() {}
+    MatrixX(int rows, int cols) : rows_(rows), cols_(cols), data_((size_t)rows * cols, 0.0) {}
+    int rows() const { return rows_; }
+    int cols() const { return cols_; }
+    double &operator()(int r, int c) { return data_[(size_t)r * cols_ + c]; }
+    double operator()(int r, int c) const { return data_[(size_t)r * cols_ + c]; }
+    double *data() { return data_.data(); }
+    const double *data() const { return data_.data(); }
+
+private:
+    int rows_ = 0, cols_ = 0;
+    std::vector<double> data_;
+};
+
+template <class MatrixType>
+class SparseBlockMatrix {
+public:
+    SparseBlockMatrix() {}
+    // rbi / cbi: the cumulative row / column index at the end of each block row / column, as in g2o
+    SparseBlockMatrix(const int *rbi, const int *cbi, int rb, int cb, bool /*hasStorage*/ = true)
+        : rbi_(rbi, rbi + rb), cbi_(cbi, cbi + cb) {}
+    // block (r, c), or nullptr when it is not stored; alloc = true creates a zero block
+    MatrixType *block(int r, int c, bool alloc = false) {
+        auto it = blocks_.find({ r, c });
+        if (it != blocks_.end()) return &it->second;
+        if (!alloc || r < 0 || c < 0 || r >= (int)rbi_.size() || c >= (int)cbi_.size()) return nullptr;
+        return &blocks_.emplace(std::make_pair(r, c), MatrixType(rowsOfBlock(r), colsOfBlock(c))).first->second;
+    }
+    const MatrixType *block(int r, int c) const {
+        auto it = blocks_.find({ r, c });
+        return it == blocks_.end() ? nullptr : &it->second;
+    }
+    int rowsOfBlock(int r) const { return r ? rbi_[r] - rbi_[r - 1] : rbi_[0]; }
+    int colsOfBlock(int c) const { return c ? cbi_[c] - cbi_[c - 1] : cbi_[0]; }
+    int rowBaseOfBlock(int r) const { return r ? rbi_[r - 1] : 0; }
+    int colBaseOfBlock(int c) const { return c ? cbi_[c - 1] : 0; }
+    const std::vector<int> &rowBlockIndices() const { return rbi_; }
+    const std::vector<int> &colBlockIndices() const { return cbi_; }
+
+private:
+    std::vector<int> rbi_, cbi_;
+    std::map<std::pair<int, int>, MatrixType> blocks_;
+};
+
 // ---- robust kernels (row a13) ------------------------------------------------------------------
 class RobustKernel {
 public:
@@ -341,6 +388,7 @@ class SparseOptimizer {
 public:
     typedef std::map<int, Vertex *> VertexIDMap;
     typedef std::vector<Edge *> EdgeContainer;
+    typedef std::vector<Vertex *> VertexContainer;
 
     SparseOptimizer() {}
     SparseOptimizer(const SparseOptimizer &) = delete;
@@ -522,6 +570,37 @@ public:
         for (size_t k = 0; k < edges_.size(); ++k) edges_[k]->unpackError(&err[k * dim_]);
         if (s3o_chi2(problem_, &chi2_) != S3O_OK) error_ = s3o_last_error();
     }
+    // SparseOptimizer::computeMarginals [EXT g2o]: blocks (hessianIndex, hessianIndex) of H^-1 at the vertices' current
+    // estimates (s3o_compute_marginals; pose-graph kinds).  spinv gets one block row / column per free vertex and the
+    // requested blocks.  A vertex without a Hessian index (fixed) makes the call fail.
+    bool computeMarginals(SparseBlockMatrix<MatrixX> &spinv, const std::vector<std::pair<int, int>> &blockIndices) {
+        if (!initialized_ || !problem_) return fail("computeMarginals: initializeOptimization() has not succeeded");
+        if (kind_ == S3O_KIND_BA) return fail("computeMarginals: not available for bundle adjustment");
+        if (!uploadEstimates()) return false;
+        const int m = (int)blockIndices.size(), dd = dim_ * dim_;
+        std::vector<int32_t> rows(m), cols(m);
+        for (int k = 0; k < m; ++k) { rows[k] = blockIndices[k].first; cols[k] = blockIndices[k].second; }
+        std::vector<double> out((size_t)m * dd);
+        if (m > 0 && s3o_compute_marginals(problem_, m, rows.data(), cols.data(), out.data()) != S3O_OK) return fail(s3o_last_error());
+        std::vector<int> bi(n_free_);
+        for (int k = 0; k < n_free_; ++k) bi[k] = (k + 1) * dim_;
+        spinv = SparseBlockMatrix<MatrixX>(bi.data(), bi.data(), n_free_, n_free_);
+        for (int k = 0; k < m; ++k) {
+            MatrixX *b = spinv.block(rows[k], cols[k], true);
+            std::copy(out.begin() + (size_t)k * dd, out.begin() + (size_t)(k + 1) * dd, b->data());
+        }
+        return true;
+    }
+    bool computeMarginals(SparseBlockMatrix<MatrixX> &spinv, const Vertex *vertex) {
+        if (!vertex || vertex->hessianIndex() < 0) return false;
+        return computeMarginals(spinv, std::vector<std::pair<int, int>>{ { vertex->hessianIndex(), vertex->hessianIndex() } });
+    }
+    bool computeMarginals(SparseBlockMatrix<MatrixX> &spinv, const VertexContainer &vertices) {
+        std::vector<std::pair<int, int>> indices;
+        for (const Vertex *v : vertices) indices.push_back({ v->hessianIndex(), v->hessianIndex() });
+        return computeMarginals(spinv, indices);
+    }
+
     double activeChi2() const { double s = 0; for (Edge *e : edges_) s += e->chi2(); return s; }
     double activeRobustChi2() const { return chi2_; }
     int numFreeVertices() const { return n_free_; }

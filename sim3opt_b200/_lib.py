@@ -73,6 +73,7 @@ SYMBOLS = {
     "s3o_hessian_multiply": (C.c_int, [C.c_void_p, C.c_double, _dp, _dp]),
     "s3o_update": (C.c_int, [C.c_void_p, _dp]),
     "s3o_smallest_eigenvector": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, _dp, _dp, C.POINTER(C.c_int)]),
+    "s3o_compute_marginals": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _dp]),
     "s3o_optimize": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.POINTER(C.c_int), _dp, _dp, _dp, C.c_int]),
     "s3o_get_vertices": (C.c_int, [C.c_void_p, _dp]),
     "s3o_estimate_slice": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),

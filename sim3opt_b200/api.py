@@ -196,6 +196,22 @@ class Problem:
         self._check(self.L.s3o_smallest_eigenvector(self.h, max_iter, tol, _d(x), C.byref(lmin), C.byref(lmax), C.byref(it)))
         return x, lmin.value, lmax.value, it.value
 
+    def marginals(self, pairs=None):
+        """Marginal covariances (g2o SparseOptimizer::computeMarginals): blocks of H^-1, H the undamped Gauss-Newton
+        Hessian at the current estimates.  pairs=None: the (n_free, d, d) diagonal blocks in Hessian order; otherwise
+        an (m, 2) array of Hessian-index pairs (row, col) -> (m, d, d)."""
+        self.build_structure()
+        if pairs is None:
+            out = np.zeros((self.num_free, self.d, self.d))
+            self._check(self.L.s3o_compute_marginals(self.h, self.num_free, None, None, _d(out)))
+            return out
+        pairs = np.ascontiguousarray(np.asarray(pairs, np.int32).reshape(-1, 2))
+        rows, cols = np.ascontiguousarray(pairs[:, 0]), np.ascontiguousarray(pairs[:, 1])
+        out = np.zeros((len(pairs), self.d, self.d))
+        self._check(self.L.s3o_compute_marginals(self.h, len(pairs), rows.ctypes.data_as(_ip), cols.ctypes.data_as(_ip),
+                                                 _d(out)))
+        return out
+
     # ---- the hot call ------------------------------------------------------------
     def optimize(self, max_iter, stop_rel_gain=0.0):
         hist = np.zeros((max(max_iter, 1), 5))

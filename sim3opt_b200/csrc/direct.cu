@@ -13,6 +13,9 @@
 // host round trip; larger ones run as a cooperative grid (one CTA per SM) with grid barriers.
 #include <cooperative_groups.h>
 
+#include <algorithm>
+#include <climits>
+
 #include "direct.h"
 #include "problem.h"
 #include "reduce.cuh"
@@ -40,6 +43,16 @@ struct DirectState {
     int coop_grid = 0;          // CTAs of the cooperative launch (<= 1: single CTA)
     int wide_levels = 0;        // leading levels wide enough for the whole grid; the rest runs on CTA 0
     bool factored = false;
+    // marginal covariances (direct_marginals), allocated on the first call
+    int32_t *d_sel_ptr = nullptr, *d_sel_sig = nullptr;
+    double *d_Sig = nullptr;    // [nL][D*D] selected inverse, laid out like L
+    double *d_E = nullptr, *d_X = nullptr;      // [D][n*D] unit right-hand sides / solutions of one block column
+    DevScalars *d_msc = nullptr;                // status of those solves (the LM's DevScalars stay untouched)
+    int32_t *d_pick = nullptr, *d_crow = nullptr, *d_cdst = nullptr;
+    double *d_out = nullptr;
+    int out_cap = 0;            // pairs d_pick / d_crow / d_cdst / d_out hold
+    // the plan of the marginals under the forced cap, when the linear solver has none of its own (PCG)
+    DirectState *marg = nullptr;
 };
 
 namespace {
@@ -300,6 +313,174 @@ __global__ void __launch_bounds__(kDirectNT) direct_kernel(DirectDev P, const do
     }
 }
 
+// ---- selected inverse (Takahashi recurrences): Sigma = H^-1 on the pattern of L, from the factor --------------
+// Sigma L = L^-T (upper triangular) gives, column j of L with sub-diagonal row set S(j),
+//   Sigma_ij = -(sum_{k in S(j)} Sigma_ik L_kj) L_jj^-1                  i in S(j)
+//   Sigma_jj = L_jj^-T (L_jj^-1 - sum_{k in S(j)} L_kj^T Sigma_kj)
+// Every Sigma_ik read by column j has i, k in S(j), i.e. belongs to a strictly later round (a round is an independent
+// set), so the rounds run in reverse, each in two phases: its off-diagonal blocks, then its diagonal blocks.
+struct SelinvDev {
+    const int32_t *sel_ptr, *sel_sig;      // selinv_lists (direct_host.cpp)
+    double *Sig;                           // [nL][D*D]
+};
+
+// off-diagonal blocks of the level's columns, one thread per block row: its D sums in registers, fixed order
+template <int D, bool COOP>
+__device__ __forceinline__ void sk_offdiag(const DirectDev &P, const SelinvDev &S, int lev, int tid, int nthreads) {
+    constexpr int DD = D * D;
+    const int c0 = P.lev_ptr[lev], c1 = P.lev_ptr[lev + 1];
+    const int t0 = P.cptr[c0], t1 = P.cptr[c1];
+    for (int item = tid; item < (t1 - t0) * D; item += nthreads) {
+        const int t = t0 + item / D, r = item % D;
+        const int j = P.bcol[t];
+        if (P.brow[t] == j) continue;
+        double acc[D];
+#pragma unroll
+        for (int c = 0; c < D; ++c) acc[c] = 0;
+        const double *Lk = P.L + (size_t)(P.cptr[j] + 1) * DD;      // L_kj of the operands, in list order
+        for (int q = S.sel_ptr[t]; q < S.sel_ptr[t + 1]; ++q, Lk += DD) {
+            const int s = S.sel_sig[q];
+            const double *Sb = S.Sig + (size_t)(s >> 1) * DD;
+            double a[D];                                             // row r of Sigma_ik
+            if (s & 1) {
+#pragma unroll
+                for (int m = 0; m < D; ++m) a[m] = ldw<COOP>(Sb + m * D + r);
+            } else {
+#pragma unroll
+                for (int m = 0; m < D; ++m) a[m] = ldw<COOP>(Sb + r * D + m);
+            }
+#pragma unroll
+            for (int m = 0; m < D; ++m)
+#pragma unroll
+                for (int c = 0; c < D; ++c) acc[c] += a[m] * Lk[m * D + c];
+        }
+        const double *Li = P.Linv + (size_t)j * DD;                  // lower triangular
+        double *out = S.Sig + (size_t)t * DD + r * D;
+#pragma unroll
+        for (int c = 0; c < D; ++c) {
+            double v = 0;
+#pragma unroll
+            for (int m = c; m < D; ++m) v += acc[m] * Li[m * D + c];
+            out[c] = -v;
+        }
+    }
+}
+
+// diagonal blocks of the level's columns, one thread per block column c: W[:, c] = L_jj^-1[:, c] - sum L_kj^T Sigma_kj[:, c],
+// then Sigma_jj[r, c] = (L_jj^-T W)[r, c] for r >= c, written to (r, c) and (c, r): exactly symmetric
+template <int D, bool COOP>
+__device__ __forceinline__ void sk_diag(const DirectDev &P, const SelinvDev &S, int lev, int tid, int nthreads) {
+    constexpr int DD = D * D;
+    const int c0 = P.lev_ptr[lev], c1 = P.lev_ptr[lev + 1];
+    for (int item = tid; item < (c1 - c0) * D; item += nthreads) {
+        const int j = c0 + item / D, c = item % D;
+        const double *Li = P.Linv + (size_t)j * DD;
+        double w[D];
+#pragma unroll
+        for (int m = 0; m < D; ++m) w[m] = Li[m * D + c];
+        for (int t = P.cptr[j] + 1; t < P.cptr[j + 1]; ++t) {
+            const double *Lb = P.L + (size_t)t * DD, *Sb = S.Sig + (size_t)t * DD;
+            double sc[D];
+#pragma unroll
+            for (int q = 0; q < D; ++q) sc[q] = ldw<COOP>(Sb + q * D + c);
+#pragma unroll
+            for (int m = 0; m < D; ++m) {
+                double v = 0;
+#pragma unroll
+                for (int q = 0; q < D; ++q) v += Lb[q * D + m] * sc[q];
+                w[m] -= v;
+            }
+        }
+        double *out = S.Sig + (size_t)P.cptr[j] * DD;
+#pragma unroll
+        for (int r = 0; r < D; ++r) {
+            if (r < c) continue;
+            double v = 0;
+#pragma unroll
+            for (int m = r; m < D; ++m) v += Li[m * D + r] * w[m];
+            out[r * D + c] = v;
+            out[c * D + r] = v;
+        }
+    }
+}
+
+// Schedule of the backward substitution: the narrow tail rounds (the last ones eliminated, so the first ones here) on
+// CTA 0 with CTA barriers while the other CTAs wait at one grid barrier, then the wide leading rounds on the grid.
+// Reads the factor of the preceding direct_kernel launch (L, Linv are read-only here).
+template <int D, bool COOP>
+__global__ void __launch_bounds__(kDirectNT, 1) selinv_kernel(DirectDev P, SelinvDev S, int wide, const GridBarrier gb) {
+    unsigned phase = 0;
+    const int ltid = threadIdx.x;
+    const int gtid = blockIdx.x * kDirectNT + threadIdx.x, gthreads = gridDim.x * kDirectNT;
+    auto gsync = [&]() {
+        if constexpr (COOP) grid_barrier(gb, phase);
+        else __syncthreads();
+    };
+    if (blockIdx.x == 0)
+        for (int lev = P.nlev - 1; lev >= wide; --lev) {
+            sk_offdiag<D, COOP>(P, S, lev, ltid, kDirectNT);
+            __syncthreads();
+            sk_diag<D, COOP>(P, S, lev, ltid, kDirectNT);
+            __syncthreads();
+        }
+    if (wide > 0) {
+        gsync();
+        for (int lev = wide - 1; lev >= 0; --lev) {
+            sk_offdiag<D, COOP>(P, S, lev, gtid, gthreads);
+            gsync();
+            sk_diag<D, COOP>(P, S, lev, gtid, gthreads);
+            if (lev > 0) gsync();
+        }
+    }
+}
+
+// requested blocks on the pattern: out[k] = Sigma block pick[k] >> 1 (transposed if pick[k] & 1); pick[k] < 0: skip
+template <int D>
+__global__ void marg_pick_kernel(const double *__restrict__ Sig, const int32_t *__restrict__ pick, int n_pairs,
+                                 double *__restrict__ out) {
+    constexpr int DD = D * D;
+    for (long long item = blockIdx.x * (long long)blockDim.x + threadIdx.x; item < (long long)n_pairs * DD;
+         item += (long long)gridDim.x * blockDim.x) {
+        const int k = (int)(item / DD), e = (int)(item - (long long)k * DD);
+        const int s = pick[k];
+        if (s < 0) continue;
+        const int a = e / D, b = e - a * D;
+        out[item] = Sig[(size_t)(s >> 1) * DD + ((s & 1) ? b * D + a : e)];
+    }
+}
+
+// D unit right-hand sides of block column `col`: E[m][i] = (i == col * D + m)
+__global__ void marg_unit_kernel(double *__restrict__ E, int nd, int D, int col) {
+    for (long long item = blockIdx.x * (long long)blockDim.x + threadIdx.x; item < (long long)nd * D;
+         item += (long long)gridDim.x * blockDim.x) {
+        const int m = (int)(item / nd), i = (int)(item - (long long)m * nd);
+        E[item] = (i == col * D + m) ? 1.0 : 0.0;
+    }
+}
+
+// requested blocks (row[q], col) of one solved block column: out[dst[q]][a][b] = X[b][row[q] * D + a]
+template <int D>
+__global__ void marg_column_kernel(const double *__restrict__ X, int nd, const int32_t *__restrict__ row,
+                                   const int32_t *__restrict__ dst, int cnt, double *__restrict__ out) {
+    constexpr int DD = D * D;
+    for (int item = blockIdx.x * blockDim.x + threadIdx.x; item < cnt * DD; item += gridDim.x * blockDim.x) {
+        const int q = item / DD, e = item - q * DD;
+        const int a = e / D, b = e - a * D;
+        out[(size_t)dst[q] * DD + e] = X[(size_t)b * nd + (size_t)row[q] * D + a];
+    }
+}
+
+DirectDev device_view(const DirectState *D) {
+    const DirectPlan &Pl = D->plan;
+    DirectDev P{};
+    P.n = Pl.n; P.nlev = Pl.nlev; P.nL = (int)Pl.brow.size();
+    P.perm = D->d_perm; P.lev_ptr = D->d_lev_ptr; P.cptr = D->d_cptr; P.brow = D->d_brow; P.bcol = D->d_bcol; P.src = D->d_src;
+    P.upd_ptr = D->d_upd_ptr; P.upd_a = D->d_upd_a; P.upd_b = D->d_upd_b;
+    P.row_ptr = D->d_row_ptr; P.row_blk = D->d_row_blk; P.row_col = D->d_row_col;
+    P.L = D->d_L; P.Linv = D->d_Linv; P.y = D->d_y; P.fail = D->d_fail;
+    return P;
+}
+
 template <class T>
 int up(s3o_problem *p, T **dst, const std::vector<T> &src) { return upload(p, dst, src); }
 
@@ -307,18 +488,20 @@ void free_direct_arrays(DirectState *D) {
     dev_free(D->d_perm); dev_free(D->d_lev_ptr); dev_free(D->d_cptr); dev_free(D->d_brow); dev_free(D->d_bcol); dev_free(D->d_src);
     dev_free(D->d_upd_ptr); dev_free(D->d_upd_a); dev_free(D->d_upd_b); dev_free(D->d_row_ptr); dev_free(D->d_row_blk);
     dev_free(D->d_row_col); dev_free(D->d_L); dev_free(D->d_Linv); dev_free(D->d_y); dev_free(D->d_fail);
+    dev_free(D->d_sel_ptr); dev_free(D->d_sel_sig); dev_free(D->d_Sig); dev_free(D->d_E); dev_free(D->d_X); dev_free(D->d_msc);
+    dev_free(D->d_pick); dev_free(D->d_crow); dev_free(D->d_cdst); dev_free(D->d_out);
+    D->out_cap = 0;
 }
 
+// one factorisation (do_factor) and/or solve of (H + lambda I) x = b with the plan of S; status in *sc
 template <int D>
-int launch_direct(s3o_problem *p, const DirectDev &P, double lambda, int do_factor) {
-    DirectState *S = p->direct;
+int launch_direct(s3o_problem *p, const DirectState *S, const DirectDev &P, double lambda, int do_factor,
+                  const double *b, double *x, DevScalars *sc) {
     if (S->coop_grid <= 1) {
-        direct_kernel<D, false><<<1, kDirectNT, 0, p->stream>>>(P, p->d_H, lambda, p->d_b, p->d_x, p->d_sc, do_factor, 0, GridBarrier{});
+        direct_kernel<D, false><<<1, kDirectNT, 0, p->stream>>>(P, p->d_H, lambda, b, x, sc, do_factor, 0, GridBarrier{});
         return S3O_OK;
     }
-    const double *H = p->d_H, *b = p->d_b;
-    double *x = p->d_x;
-    DevScalars *sc = p->d_sc;
+    const double *H = p->d_H;
     DirectDev Pc = P;
     int wide = S->wide_levels;
     GridBarrier gb{};
@@ -327,10 +510,25 @@ int launch_direct(s3o_problem *p, const DirectDev &P, double lambda, int do_fact
 }
 
 template <int D>
+int launch_selinv(s3o_problem *p, const DirectState *S, const DirectDev &P, const SelinvDev &Sv) {
+    if (S->coop_grid <= 1) {
+        selinv_kernel<D, false><<<1, kDirectNT, 0, p->stream>>>(P, Sv, 0, GridBarrier{});
+        return S3O_OK;
+    }
+    DirectDev Pc = P;
+    SelinvDev Sc = Sv;
+    int wide = S->wide_levels;
+    GridBarrier gb{};
+    void *args[] = { &Pc, &Sc, &wide, &gb };
+    return launch_persistent(p, (const void *)selinv_kernel<D, true>, S->coop_grid, kDirectNT, args, 4);
+}
+
+template <int D>
 int coop_capacity(int device) {
     int per_sm = 0, sms = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, direct_kernel<D, true>, kDirectNT, 0) != cudaSuccess) return 0;
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess) return 0;
+    // (selinv_kernel runs on the same grid: it has the same launch bounds and no shared memory, so it fits as well)
     return per_sm > 0 ? sms : 0;      // one CTA per SM
 }
 
@@ -338,6 +536,7 @@ int coop_capacity(int device) {
 
 void direct_destroy(s3o_problem *p) {
     if (!p->direct) return;
+    if (DirectState *M = p->direct->marg) { free_direct_arrays(M); delete M; }
     free_direct_arrays(p->direct);
     delete p->direct;
     p->direct = nullptr;
@@ -347,22 +546,13 @@ void direct_destroy(s3o_problem *p) {
 static constexpr long long kAutoMaxPairs = 400000, kForcedMaxPairs = 60000000;
 static constexpr int kAutoMaxLevels = 128;
 
-// Symbolic analysis + upload, once per structure.  Returns S3O_OK also when the factor is too large
-// (direct_available() then says no).
-int direct_setup(s3o_problem *p) {
-    if (p->direct && p->direct->analyzed) return S3O_OK;
-    if (!p->direct) p->direct = new DirectState();
-    DirectState *D = p->direct;
+// Symbolic analysis of p->S into D under the limits and upload; D->available says whether the plan stayed within them.
+static int plan_and_upload(s3o_problem *p, DirectState *D, long long max_pairs, int max_levels) {
     D->analyzed = true;
     D->available = false;
-    if (p->dist || p->S.nf == 0) return S3O_OK;
-    const bool forced = p->linsolver == S3O_LINSOLVER_DIRECT;
-    // AUTO: a factor within kAutoMaxPairs block products cannot have more than ~kAutoMaxPairs / 3 columns (a chain
-    // costs 3 products per column), so larger graphs go to the PCG without paying for the analysis
-    if (!forced && p->S.nf > kAutoMaxPairs / 3) return S3O_OK;
-    if (!direct_analyze(p->S.nf, p->S.rowptr, p->S.colidx, forced ? kForcedMaxPairs : kAutoMaxPairs, D->plan)) return S3O_OK;
+    if (!direct_analyze(p->S.nf, p->S.rowptr, p->S.colidx, max_pairs, D->plan)) return S3O_OK;
     const DirectPlan &P = D->plan;
-    if (!forced && P.nlev > kAutoMaxLevels) return S3O_OK;
+    if (P.nlev > max_levels) return S3O_OK;
     const int nL = (int)P.brow.size(), d = p->d;
     std::vector<int32_t> bcol(nL);
     for (int j = 0; j < P.n; ++j)
@@ -413,8 +603,26 @@ int direct_setup(s3o_problem *p) {
     }
     D->available = true;
     D->factored = false;
-    p->stats.direct_levels = P.nlev;
-    p->stats.direct_blocks = nL;
+    return S3O_OK;
+}
+
+// Symbolic analysis + upload, once per structure.  Returns S3O_OK also when the factor is too large
+// (direct_available() then says no).
+int direct_setup(s3o_problem *p) {
+    if (p->direct && p->direct->analyzed) return S3O_OK;
+    if (!p->direct) p->direct = new DirectState();
+    DirectState *D = p->direct;
+    D->analyzed = true;
+    D->available = false;
+    if (p->dist || p->S.nf == 0) return S3O_OK;
+    const bool forced = p->linsolver == S3O_LINSOLVER_DIRECT;
+    // AUTO: a factor within kAutoMaxPairs block products cannot have more than ~kAutoMaxPairs / 3 columns (a chain
+    // costs 3 products per column), so larger graphs go to the PCG without paying for the analysis
+    if (!forced && p->S.nf > kAutoMaxPairs / 3) return S3O_OK;
+    const int rc = plan_and_upload(p, D, forced ? kForcedMaxPairs : kAutoMaxPairs, forced ? INT_MAX : kAutoMaxLevels);
+    if (rc || !D->available) return rc;
+    p->stats.direct_levels = D->plan.nlev;
+    p->stats.direct_blocks = (int)D->plan.brow.size();
     return S3O_OK;
 }
 
@@ -426,26 +634,151 @@ void direct_invalidate(s3o_problem *p) { if (p->direct) p->direct->factored = fa
 int direct_solve(s3o_problem *p, double lambda, bool reuse_factor) {
     DirectState *D = p->direct;
     if (!D || !D->available) { set_error("direct_solve: no factorisation plan"); return S3O_ERR_INVALID; }
-    const DirectPlan &Pl = D->plan;
-    DirectDev P{};
-    P.n = Pl.n; P.nlev = Pl.nlev; P.nL = (int)Pl.brow.size();
-    P.perm = D->d_perm; P.lev_ptr = D->d_lev_ptr; P.cptr = D->d_cptr; P.brow = D->d_brow; P.bcol = D->d_bcol; P.src = D->d_src;
-    P.upd_ptr = D->d_upd_ptr; P.upd_a = D->d_upd_a; P.upd_b = D->d_upd_b;
-    P.row_ptr = D->d_row_ptr; P.row_blk = D->d_row_blk; P.row_col = D->d_row_col;
-    P.L = D->d_L; P.Linv = D->d_Linv; P.y = D->d_y; P.fail = D->d_fail;
+    const DirectDev P = device_view(D);
     const int do_factor = (reuse_factor && D->factored) ? 0 : 1;
     int rc = S3O_OK;
     switch (p->d) {
-    case 7: rc = launch_direct<7>(p, P, lambda, do_factor); break;
-    case 6: rc = launch_direct<6>(p, P, lambda, do_factor); break;
-    case 4: rc = launch_direct<4>(p, P, lambda, do_factor); break;
-    case 1: rc = launch_direct<1>(p, P, lambda, do_factor); break;
+    case 7: rc = launch_direct<7>(p, D, P, lambda, do_factor, p->d_b, p->d_x, p->d_sc); break;
+    case 6: rc = launch_direct<6>(p, D, P, lambda, do_factor, p->d_b, p->d_x, p->d_sc); break;
+    case 4: rc = launch_direct<4>(p, D, P, lambda, do_factor, p->d_b, p->d_x, p->d_sc); break;
+    case 1: rc = launch_direct<1>(p, D, P, lambda, do_factor, p->d_b, p->d_x, p->d_sc); break;
     default: set_error("direct_solve: block dimension %d", p->d); return S3O_ERR_UNSUPPORTED;
     }
     if (rc) return rc;
     D->factored = true;
     p->stats.direct_solves += 1;
     return check_launch(p, 1);
+}
+
+namespace {
+
+template <int D>
+int marginals_launches(s3o_problem *p, DirectState *S, int n_pairs, const std::vector<int32_t> &col_ptr,
+                       const std::vector<int32_t> &col_id, cudaEvent_t *ev) {
+    const DirectDev P = device_view(S);
+    const SelinvDev Sv{ S->d_sel_ptr, S->d_sel_sig, S->d_Sig };
+    const int nd = S->plan.n * D;
+    int rc = launch_direct<D>(p, S, P, 0.0, 1, S->d_E, S->d_X, S->d_msc);     // H = L L^T (no damping)
+    if (rc) return rc;
+    if (ev) cudaEventRecord(ev[0], p->stream);
+    if ((rc = launch_selinv<D>(p, S, P, Sv))) return rc;
+    if (ev) cudaEventRecord(ev[1], p->stream);
+    int launches = 2;
+    if (n_pairs > 0) {
+        const int grid = (int)std::min<long long>(1024, ((long long)n_pairs * D * D + 255) / 256);
+        marg_pick_kernel<D><<<grid, 256, 0, p->stream>>>(S->d_Sig, S->d_pick, n_pairs, S->d_out);
+        ++launches;
+    }
+    // pairs off the pattern of L: H X = E_c for each distinct block column c, D solves with the factor above
+    for (size_t g = 0; g + 1 < col_ptr.size(); ++g) {
+        marg_unit_kernel<<<(int)std::min<long long>(1024, ((long long)nd * D + 255) / 256), 256, 0, p->stream>>>(S->d_E, nd, D, col_id[g]);
+        for (int m = 0; m < D; ++m)
+            if ((rc = launch_direct<D>(p, S, P, 0.0, 0, S->d_E + (size_t)m * nd, S->d_X + (size_t)m * nd, S->d_msc))) return rc;
+        const int cnt = col_ptr[g + 1] - col_ptr[g];
+        marg_column_kernel<D><<<std::min(1024, (cnt * D * D + 255) / 256), 256, 0, p->stream>>>(
+            S->d_X, nd, S->d_crow + col_ptr[g], S->d_cdst + col_ptr[g], cnt, S->d_out);
+        launches += D + 2;
+    }
+    if (ev) cudaEventRecord(ev[2], p->stream);
+    return check_launch(p, launches);
+}
+
+void free_marginal_arrays(DirectState *S) {
+    dev_free(S->d_sel_ptr); dev_free(S->d_sel_sig); dev_free(S->d_Sig); dev_free(S->d_E); dev_free(S->d_X); dev_free(S->d_msc);
+}
+
+}  // namespace
+
+// Marginal covariances for the H in p->d_H (see problem.h).
+int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev) {
+    // the plan: the linear solver's own when it has one (the same analysis, only the size limits differ), otherwise
+    // one under the forced cap kept for the marginals -- the choice of the linear solver does not move
+    DirectState *S = nullptr;
+    int rc;
+    if (p->linsolver != S3O_LINSOLVER_PCG) {
+        if ((rc = direct_setup(p))) return rc;
+        if (direct_available(p)) S = p->direct;
+    }
+    if (!S) {
+        if (!p->direct) p->direct = new DirectState();
+        DirectState *&M = p->direct->marg;
+        if (!M) {
+            M = new DirectState();
+            if ((rc = plan_and_upload(p, M, kForcedMaxPairs, INT_MAX))) { delete M; M = nullptr; return rc; }
+        }
+        if (!M->available) {
+            set_error("s3o_compute_marginals: the factor of this graph needs more than %lld block products", kForcedMaxPairs);
+            return S3O_ERR_UNSUPPORTED;
+        }
+        S = M;
+    }
+    const DirectPlan &Pl = S->plan;
+    const int n = Pl.n, d = p->d, dd = d * d;
+    if (!S->d_Sig) {      // first marginals call on this plan: gather lists and buffers
+        std::vector<int32_t> sel_ptr, sel_sig;
+        selinv_lists(Pl, sel_ptr, sel_sig);
+        rc = up(p, &S->d_sel_ptr, sel_ptr);
+        rc = rc ? rc : up(p, &S->d_sel_sig, sel_sig);
+        rc = rc ? rc : dev_alloc(&S->d_E, (size_t)n * dd);
+        rc = rc ? rc : dev_alloc(&S->d_X, (size_t)n * dd);
+        rc = rc ? rc : dev_alloc(&S->d_msc, 1);
+        rc = rc ? rc : dev_alloc(&S->d_Sig, Pl.brow.size() * dd);
+        if (!rc && cudaMemsetAsync(S->d_E, 0, sizeof(double) * n * dd, p->stream) != cudaSuccess) rc = S3O_ERR_CUDA;
+        if (!rc && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = S3O_ERR_CUDA;
+        if (rc) { free_marginal_arrays(S); set_error("s3o_compute_marginals: device allocation failed"); return rc; }
+    }
+    // requested pairs -> block of Sigma (elimination order) and transpose flag; the rest by block column
+    std::vector<int32_t> ipos(n);
+    for (int k = 0; k < n; ++k) ipos[Pl.perm[k]] = k;
+    std::vector<int32_t> pick(n_pairs);
+    std::vector<std::pair<int32_t, int32_t>> off;       // (column, pair) of the pairs off the pattern
+    for (int k = 0; k < n_pairs; ++k) {
+        const int r = rows ? rows[k] : k, c = cols ? cols[k] : k;
+        const int pr = ipos[r], pc = ipos[c];
+        const int32_t t = direct_find_block(Pl, std::min(pr, pc), std::max(pr, pc));
+        pick[k] = t >= 0 ? (t << 1) | (pr < pc ? 1 : 0) : -1;
+        if (t < 0) off.push_back({ c, k });
+    }
+    std::sort(off.begin(), off.end());
+    std::vector<int32_t> col_ptr, col_id, crow(off.size()), cdst(off.size());
+    for (size_t q = 0; q < off.size(); ++q) {
+        if (q == 0 || off[q].first != off[q - 1].first) { col_ptr.push_back((int32_t)q); col_id.push_back(off[q].first); }
+        crow[q] = rows[off[q].second];
+        cdst[q] = off[q].second;
+    }
+    if (!off.empty()) col_ptr.push_back((int32_t)off.size());
+    if (n_pairs > S->out_cap) {
+        dev_free(S->d_pick); dev_free(S->d_crow); dev_free(S->d_cdst); dev_free(S->d_out);
+        S->out_cap = 0;
+        rc = dev_alloc(&S->d_pick, (size_t)n_pairs);
+        rc = rc ? rc : dev_alloc(&S->d_crow, (size_t)n_pairs);
+        rc = rc ? rc : dev_alloc(&S->d_cdst, (size_t)n_pairs);
+        rc = rc ? rc : dev_alloc(&S->d_out, (size_t)n_pairs * dd);
+        if (rc) { set_error("s3o_compute_marginals: device allocation failed"); return rc; }
+        S->out_cap = n_pairs;
+    }
+    auto h2d = [&](int32_t *dst, const std::vector<int32_t> &v) -> int {
+        if (v.empty()) return S3O_OK;
+        S3O_CUDA(cudaMemcpyAsync(dst, v.data(), v.size() * sizeof(int32_t), cudaMemcpyHostToDevice, p->stream));
+        p->stats.h2d_bytes += (int64_t)(v.size() * sizeof(int32_t));
+        return S3O_OK;
+    };
+    if ((rc = h2d(S->d_pick, pick)) || (rc = h2d(S->d_crow, crow)) || (rc = h2d(S->d_cdst, cdst))) return rc;
+    switch (d) {
+    case 7: rc = marginals_launches<7>(p, S, n_pairs, col_ptr, col_id, ev); break;
+    case 4: rc = marginals_launches<4>(p, S, n_pairs, col_ptr, col_id, ev); break;
+    case 1: rc = marginals_launches<1>(p, S, n_pairs, col_ptr, col_id, ev); break;
+    default: set_error("s3o_compute_marginals: block dimension %d", d); return S3O_ERR_UNSUPPORTED;
+    }
+    S->factored = false;      // the factor of H without damping: a later solve with reuse_factor factorises again
+    if (rc) return rc;
+    int failed = 0;
+    if (n_pairs > 0) S3O_CUDA(cudaMemcpyAsync(out, S->d_out, sizeof(double) * n_pairs * dd, cudaMemcpyDeviceToHost, p->stream));
+    S3O_CUDA(cudaMemcpyAsync(&failed, S->d_fail, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
+    S3O_CUDA(cudaStreamSynchronize(p->stream));
+    p->stats.d2h_bytes += (int64_t)n_pairs * dd * 8 + 4;
+    if (failed) { set_error("s3o_compute_marginals: the Hessian is not positive definite (a pivot of its factorisation failed)"); return S3O_ERR_SOLVE; }
+    return S3O_OK;
 }
 
 }  // namespace s3o

@@ -45,4 +45,15 @@ struct DirectPlan {
 bool direct_analyze(int n, const std::vector<int32_t> &rowptr, const std::vector<int32_t> &colidx, long long max_pairs,
                     DirectPlan &plan);
 
+// Block index of L(row, col), row >= col (elimination positions), or -1 when the block is not in the pattern.
+int32_t direct_find_block(const DirectPlan &plan, int col, int row);
+
+// Gather lists of the selected inverse Sigma = H^-1 on the pattern of L (Takahashi recurrences, direct.cu), stored
+// like L ([nL][d*d], block t = Sigma(brow[t], col(t))).  For every sub-diagonal block t = (i, j), the operands of
+//   Sigma_ij = -(sum_{k in S(j)} Sigma_ik L_kj) L_jj^-1
+// in the order of column j's sub-diagonal blocks (L_kj is block cptr[j] + 1 + m for the m-th operand):
+// sel_sig[sel_ptr[t] + m] = (Sigma block holding (i, k) << 1) | transposed (i < k: the block holds Sigma_ki).
+// Diagonal blocks have empty lists (their recurrence reads column j's own sub-diagonal blocks).
+void selinv_lists(const DirectPlan &plan, std::vector<int32_t> &sel_ptr, std::vector<int32_t> &sel_sig);
+
 }  // namespace s3o

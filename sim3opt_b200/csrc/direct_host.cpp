@@ -29,6 +29,13 @@ void merge_into(std::vector<int32_t> &a, const std::vector<int32_t> &b, int32_t 
 
 }  // namespace
 
+int32_t direct_find_block(const DirectPlan &P, int col, int row) {
+    if (row == col) return P.cptr[col];
+    const int32_t *b = P.brow.data() + P.cptr[col] + 1, *e = P.brow.data() + P.cptr[col + 1];
+    const int32_t *it = std::lower_bound(b, e, row);
+    return (it != e && *it == row) ? (int32_t)(it - P.brow.data()) : -1;
+}
+
 bool direct_analyze(int n, const std::vector<int32_t> &rowptr, const std::vector<int32_t> &colidx, long long max_pairs,
                     DirectPlan &P) {
     P = DirectPlan();
@@ -94,12 +101,7 @@ bool direct_analyze(int n, const std::vector<int32_t> &rowptr, const std::vector
         for (size_t t = 0; t < N.size(); ++t) dst[1 + t] = pos[N[t]];
         std::sort(dst + 1, dst + 1 + N.size());
     }
-    auto find_block = [&](int col, int row) -> int32_t {     // block (row, col), row >= col
-        if (row == col) return P.cptr[col];
-        const int32_t *b = P.brow.data() + P.cptr[col] + 1, *e = P.brow.data() + P.cptr[col + 1];
-        const int32_t *it = std::lower_bound(b, e, row);
-        return (it != e && *it == row) ? (int32_t)(it - P.brow.data()) : -1;
-    };
+    auto find_block = [&](int col, int row) { return direct_find_block(P, col, row); };
 
     // ---- scatter map from the BSR-upper Hessian
     P.src.assign(nL, -1);
@@ -149,6 +151,27 @@ bool direct_analyze(int n, const std::vector<int32_t> &rowptr, const std::vector
             ++rfill[i];
         }
     return true;
+}
+
+void selinv_lists(const DirectPlan &P, std::vector<int32_t> &sel_ptr, std::vector<int32_t> &sel_sig) {
+    const int n = P.n, nL = (int)P.brow.size();
+    sel_ptr.assign(nL + 1, 0);
+    for (int j = 0; j < n; ++j) {
+        const int ns = P.cptr[j + 1] - P.cptr[j] - 1;
+        for (int t = P.cptr[j]; t < P.cptr[j + 1]; ++t) sel_ptr[t + 1] = sel_ptr[t] + (t == P.cptr[j] ? 0 : ns);
+    }
+    sel_sig.resize((size_t)sel_ptr[nL]);
+    for (int j = 0; j < n; ++j)
+        for (int a = P.cptr[j] + 1; a < P.cptr[j + 1]; ++a) {
+            const int i = P.brow[a];
+            int32_t *dst = sel_sig.data() + sel_ptr[a];
+            for (int b = P.cptr[j] + 1; b < P.cptr[j + 1]; ++b) {
+                const int k = P.brow[b];
+                // S(j) is a clique of the filled graph: (max(i, k), min(i, k)) is always a block of L
+                const int32_t s = direct_find_block(P, std::min(i, k), std::max(i, k));
+                *dst++ = (s << 1) | (i < k ? 1 : 0);
+            }
+        }
 }
 
 }  // namespace s3o

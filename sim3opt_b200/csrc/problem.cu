@@ -1618,6 +1618,58 @@ int s3o_smallest_eigenvector(s3o_problem *p, int max_iter, double tol, double *x
     return S3O_OK;
 }
 
+// Marginal covariances (g2o SparseOptimizer::computeMarginals): H = J^T Omega' J at the current estimates, factorised
+// without damping, and its selected inverse (direct.cu).
+int s3o_compute_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out) {
+    if (!p || n_pairs < 0 || (!rows != !cols) || (n_pairs > 0 && !out)) { set_error("s3o_compute_marginals: bad arguments"); return S3O_ERR_INVALID; }
+    if (p->dist || (p->kind != S3O_KIND_SIM3 && p->kind != S3O_KIND_SCALE_TRANS && p->kind != S3O_KIND_SCALE)) {
+        set_error("s3o_compute_marginals: pose-graph kinds on one GPU only (not bundle adjustment, the partitioned solve or a linear-solver handle)");
+        return S3O_ERR_UNSUPPORTED;
+    }
+    cudaSetDevice(p->device);
+    int rc = ensure_built(p);
+    if (rc) return rc;
+    const int nf = p->S.nf;
+    if (nf == 0) { set_error("s3o_compute_marginals: 0 free vertices"); return S3O_ERR_INVALID; }
+    if (!rows && n_pairs != nf) { set_error("s3o_compute_marginals: the diagonal blocks need n_pairs = n_free = %d", nf); return S3O_ERR_INVALID; }
+    for (int k = 0; rows && k < n_pairs; ++k)
+        if (rows[k] < 0 || rows[k] >= nf || cols[k] < 0 || cols[k] >= nf) {
+            set_error("s3o_compute_marginals: pair %d (%d, %d) is not a pair of Hessian indices in [0, %d) (fixed vertices have none)",
+                      k, rows[k], cols[k], nf);
+            return S3O_ERR_INVALID;
+        }
+    // H is singular when a connected component holds no fixed vertex (its gauge is free)
+    {
+        std::vector<int32_t> root(p->nv);
+        for (int v = 0; v < p->nv; ++v) root[v] = v;
+        auto find = [&](int v) { while (root[v] != v) v = root[v] = root[root[v]]; return v; };
+        for (int e = 0; e < p->ne; ++e) {
+            const int a = find(p->v0[e]), b = find(p->v1[e]);
+            if (a != b) root[std::max(a, b)] = std::min(a, b);
+        }
+        std::vector<uint8_t> anchored(p->nv, 0);
+        for (int v = 0; v < p->nv; ++v) if (p->fixed[v]) anchored[find(v)] = 1;
+        for (int v = 0; v < p->nv; ++v)
+            if (!anchored[find(v)]) {
+                set_error("s3o_compute_marginals: the Hessian is singular: the connected component of vertex %d has no fixed vertex", v);
+                return S3O_ERR_SOLVE;
+            }
+    }
+    cudaEventRecord(p->ev[0], p->stream);
+    if ((rc = do_linearize(p))) return rc;
+    cudaEventRecord(p->ev[1], p->stream);
+    rc = direct_marginals(p, n_pairs, rows, cols, out, p->ev + 2);
+    direct_invalidate(p);
+    p->linearized = false;          // as after s3o_optimize: the next solve linearises again
+    if (rc) return rc;
+    if (getenv("S3O_MARGINALS_TRACE")) {     // per-phase CUDA-event times (tools/marginals_probe.py)
+        float ms[4] = {};
+        for (int k = 0; k < 4; ++k) cudaEventElapsedTime(&ms[k], p->ev[k], p->ev[k + 1]);
+        fprintf(stderr, "s3o_compute_marginals: linearize %.4f factor %.4f selinv %.4f gather %.4f ms\n", ms[0], ms[1], ms[2], ms[3]);
+    }
+    return S3O_OK;
+}
+
 int s3o_get_vertices(s3o_problem *p, double *est) {
     if (p && p->kind == S3O_KIND_BA) { set_error("s3o_get_vertices: a BA problem takes s3o_ba_get_cameras / s3o_ba_get_points"); return S3O_ERR_INVALID; }
     if (!p || !est || !p->d_est[0]) { set_error("s3o_get_vertices: no vertices"); return S3O_ERR_INVALID; }

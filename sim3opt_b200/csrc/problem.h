@@ -163,6 +163,12 @@ bool direct_available(const s3o_problem *p);          // false: the factor would
 int direct_solve(s3o_problem *p, double lambda, bool reuse_factor);
 void direct_invalidate(s3o_problem *p);               // H changed
 void direct_destroy(s3o_problem *p);
+// Marginal covariances: blocks (rows[k], cols[k]) of H^-1 (Hessian indices, validated by the caller) for the H in
+// p->d_H, into out (n_pairs x d x d); rows == cols == nullptr: the n_pairs = n_free diagonal blocks.  Factorises H on
+// the linear solver's plan, or on a plan under the forced cap kept for the marginals (the choice of the linear solver
+// does not change), then runs the selected inverse.  Leaves p->d_b / p->d_x / p->d_sc untouched and no factor held.
+// ev (may be nullptr): 3 events recorded after the factorisation, the selected inverse and the gather.
+int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev);
 // Launches a persistent kernel whose CTAs synchronise through grid_barrier (gridbar.cuh).  The kernel's LAST argument
 // is a GridBarrier; args[nargs - 1] must point to a GridBarrier that this call fills.
 inline int launch_persistent(s3o_problem *p, const void *func, int grid, int block, void **args, int nargs, size_t smem = 0) {

@@ -1,0 +1,97 @@
+"""Times s3o_compute_marginals (every diagonal block of H^-1) on K1, K118, sphere_small and the s10k sphere.
+
+Each call is split by the library's CUDA events (S3O_MARGINALS_TRACE=1: linearise, factorisation, selected inverse,
+gather) and timed end to end on the host; medians over --reps calls after --warmup calls.  Prints the plan's rounds,
+blocks of L and block products, and for K1 / K118 the CPU oracle's dense inverse of the same H as a reference.
+One JSON line per graph.
+
+    python tools/marginals_probe.py [--reps 50] [--warmup 5]
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import tempfile
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+os.environ["S3O_MARGINALS_TRACE"] = "1"
+
+
+def graphs():
+    from oracle import kitti_io
+    from sim3opt_b200 import synth
+    kd = os.path.join(ROOT, "tests", "golden", "kitti00")
+    return {"K1": kitti_io.build_kitti_sim3_graph(kd, use_one_constraint=True),
+            "K118": kitti_io.build_kitti_sim3_graph(kd, use_one_constraint=False),
+            "sphere_small": synth.sphere(n_laps=12, poses_per_lap=40, seed=7),
+            "s10k": synth.sphere(10, 1000, seed=42)}
+
+
+class StderrCapture:
+    """The library writes its trace lines to file descriptor 2: route it to a temporary file."""
+
+    def __enter__(self):
+        sys.stderr.flush()
+        self.f = tempfile.TemporaryFile(mode="w+")
+        self.saved = os.dup(2)
+        os.dup2(self.f.fileno(), 2)
+        return self
+
+    def __exit__(self, *exc):
+        os.dup2(self.saved, 2)
+        os.close(self.saved)
+        self.f.seek(0)
+        self.text = self.f.read()
+        self.f.close()
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reps", type=int, default=50)
+    ap.add_argument("--warmup", type=int, default=5)
+    a = ap.parse_args()
+    import sim3opt_b200 as s3
+    from conftest import make_gpu, make_oracle
+    from test_gpu_parity import dense_from_blocks
+    gpu_info = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"],
+                              capture_output=True, text=True).stdout.strip().splitlines()
+    for name, g in graphs().items():
+        plan = s3.host_direct_plan(len(g["est"]), g["fixed"], g["v0"], g["v1"], max_pairs=60000000)
+        p = make_gpu(g, jac=1)
+        for _ in range(a.warmup):
+            p.marginals()
+        wall = []
+        with StderrCapture() as cap:
+            for _ in range(a.reps):
+                t0 = time.perf_counter()
+                p.marginals()
+                wall.append(time.perf_counter() - t0)
+        phases = np.array([[float(x) for x in line.split()[2:9:2]] for line in cap.text.splitlines()
+                           if line.startswith("s3o_compute_marginals:")])
+        assert len(phases) == a.reps, cap.text[-2000:]
+        med = np.median(phases, 0)
+        rec = {"graph": name, "free": plan["n"], "rounds": plan["rounds"], "blocks_L": len(plan["brow"]),
+               "factor_products": plan["n_pairs"], "selinv_products": 2 * plan["n_pairs"],
+               "ms_linearize": med[0], "ms_factor": med[1], "ms_selinv": med[2], "ms_gather": med[3],
+               "ms_call_wall": 1e3 * float(np.median(wall)), "reps": a.reps, "gpu": gpu_info[:1]}
+        if name in ("K1", "K118"):          # reference, not a target: the oracle's H and a dense LAPACK inverse
+            o = make_oracle(g, jac=1)
+            cp, ri = o.build_structure()
+            ts = []
+            for _ in range(5):
+                t0 = time.perf_counter()
+                H, _ = o.linearize()
+                np.linalg.inv(dense_from_blocks(cp, ri, H, 7))
+                ts.append(time.perf_counter() - t0)
+            rec["ms_cpu_oracle_dense_inverse"] = 1e3 * float(np.median(ts))
+        print(json.dumps(rec), flush=True)
+
+
+if __name__ == "__main__":
+    main()
