@@ -206,7 +206,8 @@ int s3o_smallest_eigenvector(s3o_problem *p, int max_iter, double tol, double *x
  * rows/cols: n_pairs Hessian indices (s3o_get_hessian_index; fixed vertices have none); out: n_pairs x d x d,
  * row-major, block (rows[k], cols[k]).  rows == cols == NULL: every diagonal block in Hessian order
  * (n_pairs must equal n_free).  S3O_ERR_SOLVE when H is singular (a connected component without a fixed
- * vertex); S3O_ERR_UNSUPPORTED for BA, the partitioned solve, and graphs whose factor exceeds the forced cap.
+ * vertex); S3O_ERR_UNSUPPORTED for BA (s3o_ba_compute_marginals), the partitioned solve, and graphs whose factor
+ * exceeds the forced cap.
  * Every call linearises again at the current estimates, so the result does not depend on what ran before it
  * (g2o uses the H of its last buildSystem, which is one step behind the estimates optimize() returns).  H is
  * factorised by the sparse block Cholesky (a plan under the forced cap of s3o_set_linear_solver(DIRECT) when the
@@ -289,6 +290,26 @@ int s3o_ba_get_system(s3o_problem *p, double *Hpp, double *Hll, double *Hpl, dou
 /* damped Schur complement S = (Hpp + lambda I) - sum Hpl (Hll + lambda I)^-1 Hpl^T (blocks in the CCS
  * order of s3o_get_structure) and bs = bp - sum Hpl (Hll + lambda I)^-1 bl */
 int s3o_ba_get_schur(s3o_problem *p, double lambda, double *blocks, double *bs);
+/* Marginal covariances of bundle adjustment (g2o SparseOptimizer::computeMarginals on the BA graph): blocks of
+ * Sigma = H^-1, H = [[Hpp, Hpl], [Hpl^T, Hll]] the full Gauss-Newton Hessian (robust weights and information included,
+ * no LM damping) linearised at the CURRENT estimates, with the same semantics as s3o_compute_marginals.  Tangents:
+ * camera [omega, upsilon] of T <- exp(d) T, point xyz.  Hessian indices: free cameras 0 .. ncf-1 in camera-id order,
+ * then free points ncf .. ncf+npf-1 in point-id order (ncf, npf: s3o_ba_get_sizes); fixed vertices have none.
+ * out: the blocks back to back, block k dim(rows[k]) x dim(cols[k]) row-major (dim 6 for a camera, 3 for a point)
+ * at the sum of the sizes of the blocks before it.  rows == cols == NULL: every diagonal block, cameras then points
+ * (n_pairs must equal ncf + npf; out holds 36 ncf + 9 npf doubles).  Pairs served: any two cameras; the diagonal
+ * block of a point; (camera, point) and (point, camera) when that camera observes that point.  Camera blocks come
+ * from the selected inverse of the Schur complement S = Hpp - Hpl Hll^-1 Hpl^T (s3o_compute_marginals' machinery on
+ * the 6x6 system), points from Sigma(c_a, l) = -Z_a and Sigma(l, l) = Hll^-1 + sum_a Y_a^T Z_a with
+ * Y_a = Hpl_a Hll^-1, Z_a = sum_b S^-1(c_a, c_b) Y_b over the point's observations by free cameras.
+ * Returns S3O_ERR_UNSUPPORTED for two distinct points, a camera-point pair whose camera does not observe the point,
+ * or a Schur factor beyond the forced cap; S3O_ERR_INVALID for bad arguments, an index out of range, or a problem that
+ * is not BA; S3O_ERR_SOLVE, naming a vertex, when H is singular: a connected component of the observation graph fixes
+ * neither a camera and one more vertex nor three points (the 7-DoF gauge of monocular BA is free), or a free point is
+ * seen by fewer than two distinct cameras; S3O_ERR_SOLVE also when a pivot of the factorisation of S fails or a free
+ * point's det(Hll) is not positive.  The LM state (step, lambda, snapshots, direct_solves) is untouched, and the
+ * problem is left unlinearised. */
+int s3o_ba_compute_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out);
 
 /* ---- LinearSolver-level plug-in: g2o::LinearSolver<M>::{init(), solve(A, x, b)} (the innermost slot of
  * OptimizationAlgorithmLevenberg(BlockSolverX(LinearSolverEigen)), kitti_surf.cpp:553-557, bal_example.cpp:73-83) ----

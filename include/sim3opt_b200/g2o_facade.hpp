@@ -571,23 +571,32 @@ public:
         if (s3o_chi2(problem_, &chi2_) != S3O_OK) error_ = s3o_last_error();
     }
     // SparseOptimizer::computeMarginals [EXT g2o]: blocks (hessianIndex, hessianIndex) of H^-1 at the vertices' current
-    // estimates (s3o_compute_marginals; pose-graph kinds).  spinv gets one block row / column per free vertex and the
-    // requested blocks.  A vertex without a Hessian index (fixed) makes the call fail.
+    // estimates (s3o_compute_marginals; for BA s3o_ba_compute_marginals, where a block row / column is 6 wide for a
+    // camera and 3 for a point).  spinv gets one block row / column per free vertex and the requested blocks.  A vertex
+    // without a Hessian index (fixed) makes the call fail.
     bool computeMarginals(SparseBlockMatrix<MatrixX> &spinv, const std::vector<std::pair<int, int>> &blockIndices) {
         if (!initialized_ || !problem_) return fail("computeMarginals: initializeOptimization() has not succeeded");
-        if (kind_ == S3O_KIND_BA) return fail("computeMarginals: not available for bundle adjustment");
         if (!uploadEstimates()) return false;
-        const int m = (int)blockIndices.size(), dd = dim_ * dim_;
+        const bool ba = kind_ == S3O_KIND_BA;
+        const int nb = ba ? n_free_ + n_free_points_ : n_free_;
+        auto dim = [&](int h) { return ba && h >= n_free_ ? 3 : dim_; };
+        const int m = (int)blockIndices.size();
         std::vector<int32_t> rows(m), cols(m);
-        for (int k = 0; k < m; ++k) { rows[k] = blockIndices[k].first; cols[k] = blockIndices[k].second; }
-        std::vector<double> out((size_t)m * dd);
-        if (m > 0 && s3o_compute_marginals(problem_, m, rows.data(), cols.data(), out.data()) != S3O_OK) return fail(s3o_last_error());
-        std::vector<int> bi(n_free_);
-        for (int k = 0; k < n_free_; ++k) bi[k] = (k + 1) * dim_;
-        spinv = SparseBlockMatrix<MatrixX>(bi.data(), bi.data(), n_free_, n_free_);
+        std::vector<size_t> off(m + 1, 0);
+        for (int k = 0; k < m; ++k) {
+            rows[k] = blockIndices[k].first; cols[k] = blockIndices[k].second;
+            off[k + 1] = off[k] + (size_t)dim(rows[k]) * dim(cols[k]);
+        }
+        std::vector<double> out(off[m]);
+        if (m > 0 && (ba ? s3o_ba_compute_marginals(problem_, m, rows.data(), cols.data(), out.data())
+                         : s3o_compute_marginals(problem_, m, rows.data(), cols.data(), out.data())) != S3O_OK)
+            return fail(s3o_last_error());
+        std::vector<int> bi(nb);
+        for (int k = 0; k < nb; ++k) bi[k] = (k ? bi[k - 1] : 0) + dim(k);
+        spinv = SparseBlockMatrix<MatrixX>(bi.data(), bi.data(), nb, nb);
         for (int k = 0; k < m; ++k) {
             MatrixX *b = spinv.block(rows[k], cols[k], true);
-            std::copy(out.begin() + (size_t)k * dd, out.begin() + (size_t)(k + 1) * dd, b->data());
+            std::copy(out.begin() + off[k], out.begin() + off[k + 1], b->data());
         }
         return true;
     }
@@ -667,7 +676,7 @@ private:
         int hc = 0, hp = 0;      // free cameras numbered first, then the marginalised points
         for (Vertex *v : order_) v->hessian_index_ = v->fixed() ? -1 : hc++;
         for (Vertex *v : points_) v->hessian_index_ = v->fixed() ? -1 : hc + hp++;
-        est_dim_ = 7; dim_ = 6; n_free_ = nf; n_blocks_ = nb;
+        est_dim_ = 7; dim_ = 6; n_free_ = nf; n_free_points_ = hp; n_blocks_ = nb;
         initialized_ = true;
         return true;
     }
@@ -705,7 +714,7 @@ private:
     std::vector<double> est_, pts_, hist_;
     std::string error_;
     bool verbose_ = false, initialized_ = false;
-    int device_ = 0, kind_ = 0, est_dim_ = 0, dim_ = 0, n_free_ = 0, n_blocks_ = 0;
+    int device_ = 0, kind_ = 0, est_dim_ = 0, dim_ = 0, n_free_ = 0, n_free_points_ = 0, n_blocks_ = 0;
     int jac_mode_ = S3O_JAC_ANALYTIC, math_mode_ = S3O_MATH_REFERENCE, pcg_max_iter_ = 0;
     double jac_h_ = 1e-9, pcg_tol_ = 0, stop_gain_ = 0, chi2_ = 0;
 };

@@ -93,6 +93,7 @@ SYMBOLS = {
     "s3o_ba_edge_errors": (C.c_int, [C.c_void_p, _dp]),
     "s3o_ba_get_system": (C.c_int, [C.c_void_p, _dp, _dp, _dp, _dp]),
     "s3o_ba_get_schur": (C.c_int, [C.c_void_p, C.c_double, _dp, _dp]),
+    "s3o_ba_compute_marginals": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _dp]),
     "s3o_linsolver_create": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "s3o_linsolver_destroy": (C.c_int, [C.c_void_p]),
     "s3o_linsolver_solve": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _dp, C.c_int, C.c_double, _dp, _dp, C.POINTER(C.c_int), C.POINTER(C.c_int)]),

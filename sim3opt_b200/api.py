@@ -471,6 +471,28 @@ class BAProblem(Problem):
         self._check(self.L.s3o_ba_get_schur(self.h, float(lam), _d(S), _d(bs)))
         return S, bs
 
+    def ba_marginals(self, pairs=None):
+        """Marginal covariances of BA (s3o_ba_compute_marginals): blocks of H^-1, H the full undamped Gauss-Newton Hessian
+        at the current estimates.  Hessian indices: free cameras 0..ncf-1, then free points ncf..ncf+npf-1.
+        pairs=None: (cams (ncf, 6, 6), points (npf, 3, 3)), the diagonal blocks; otherwise an (m, 2) array of index
+        pairs (row, col) -> a list of m arrays, (6 or 3) x (6 or 3) by the kinds of row and col."""
+        self.build_structure()
+        if pairs is None:
+            out = np.zeros(36 * self.ncf + 9 * self.npf)
+            self._check(self.L.s3o_ba_compute_marginals(self.h, self.ncf + self.npf, None, None, _d(out)))
+            return out[:36 * self.ncf].reshape(self.ncf, 6, 6), out[36 * self.ncf:].reshape(self.npf, 3, 3)
+        pairs = np.ascontiguousarray(np.asarray(pairs, np.int32).reshape(-1, 2))
+        rows, cols = np.ascontiguousarray(pairs[:, 0]), np.ascontiguousarray(pairs[:, 1])
+        dims = [(6 if r < self.ncf else 3, 6 if c < self.ncf else 3) for r, c in pairs]
+        out = np.zeros(max(sum(a * b for a, b in dims), 1))
+        self._check(self.L.s3o_ba_compute_marginals(self.h, len(pairs), rows.ctypes.data_as(_ip), cols.ctypes.data_as(_ip),
+                                                    _d(out)))
+        res, o = [], 0
+        for a, b in dims:
+            res.append(out[o:o + a * b].reshape(a, b).copy())
+            o += a * b
+        return res
+
     def solve(self, lam):
         x = np.zeros(6 * self.ncf + 3 * self.npf)
         it, rel = C.c_int(0), C.c_double(0)

@@ -19,8 +19,11 @@
 #include <algorithm>
 #include <cmath>
 #include <cstring>
+#include <map>
+#include <string>
 #include <vector>
 
+#include "direct.h"
 #include "problem.h"
 #include "reduce.cuh"
 #include "sim3_math.cuh"
@@ -49,6 +52,20 @@ struct BaState {
     double *d_Hpp = nullptr, *d_bp = nullptr, *d_Hll = nullptr, *d_bl = nullptr;
     double *d_Dinv = nullptr, *d_dl = nullptr, *d_xl = nullptr;
     double *d_cam_snap = nullptr, *d_pt_snap = nullptr;
+    // marginal covariances (s3o_ba_compute_marginals)
+    std::vector<int32_t> pt_ptr, socam;     // observations sorted by point: per-point ranges and their cameras
+    int marg_check = -1;                    // host checks of this structure: -1 not run, else their return code
+    std::string marg_msg;
+    bool marg_lists = false;                // point gather lists below built, on the plan numbered marg_serial
+    uint64_t marg_serial = 0;
+    int32_t *d_mo_ptr = nullptr, *d_mo_obs = nullptr, *d_mp_sig = nullptr;
+    int64_t *d_mp_ptr = nullptr;
+    // per call: requested points, camera-point slots, output map, staging and result
+    int32_t *d_mrq = nullptr, *d_mcl_ptr = nullptr, *d_mcl_a = nullptr, *d_msrc = nullptr;
+    int64_t *d_mdst = nullptr;
+    double *d_mpt = nullptr, *d_mout = nullptr;
+    int *d_mflag = nullptr;
+    size_t cap_mrq = 0, cap_mcl_ptr = 0, cap_mcl_a = 0, cap_msrc = 0, cap_mdst = 0, cap_mpt = 0, cap_mout = 0;
 };
 
 namespace {
@@ -468,6 +485,99 @@ __global__ void ba_scale_kernel(int n1, const double *__restrict__ xc, const dou
     }
 }
 
+// ---- marginal covariances: the point phase --------------------------------------------------------------------
+// For a free point l with observations O(l) by free cameras, Y_a = Hpl_a Hll^-1 and Sigma_cc = S^-1 (selected inverse):
+//   Z_a = sum_{b in O(l)} Sigma_cc(c_a, c_b) Y_b,   Sigma(c_a, l) = -Z_a,   Sigma(l, l) = Hll^-1 + sum_a Y_a^T Z_a.
+// One warp per requested point; a group of 6 lanes per observation a (5 groups a warp), lane r of the group owns row r
+// of Z_a and sums over b in list order.  Each lane adds its rows' share of Y_a^T Z_a to a lower triangle, which a
+// butterfly over the warp reduces (fixed lanes, fixed order: bitwise reproducible); lane 0 adds Hll^-1 and writes the
+// triangle mirrored, so Sigma(l, l) is exactly symmetric.  The observation lists: mo_ptr / mo_obs (sorted observation
+// index of each free-camera observation, in order); the Sigma_cc operands: mp_sig[mp_ptr[l] + a |O(l)| + b] = (block
+// of the selected inverse << 1) | transposed.  Camera-point blocks: cl_a[q] (q in cl_ptr[s] .. cl_ptr[s+1]) is the
+// observation whose -Z_a goes to slot q.  A first grid-stride pass flags every free point whose det(Hll) is not > 0.
+constexpr int kMargNT = 256;
+__global__ void __launch_bounds__(kMargNT) ba_marginal_points_kernel(
+    int npf, int nrq, const int32_t *__restrict__ rq, const int32_t *__restrict__ mo_ptr, const int32_t *__restrict__ mo_obs,
+    const int64_t *__restrict__ mp_ptr, const int32_t *__restrict__ mp_sig, const double *__restrict__ Sig,
+    const double *__restrict__ Y, const double *__restrict__ Dinv, const double *__restrict__ Hll,
+    const int32_t *__restrict__ cl_ptr, const int32_t *__restrict__ cl_a, double *__restrict__ pdiag,
+    double *__restrict__ pcl, int *fail) {
+    const int gtid = blockIdx.x * kMargNT + threadIdx.x, gthreads = gridDim.x * kMargNT;
+    for (int li = gtid; li < npf; li += gthreads) {      // the determinant as ba_point_inverse_kernel forms it
+        const double *A = Hll + (size_t)li * 9;
+        const double a = A[0], b = A[1], c = A[2], d = A[4], e = A[5], f = A[8];
+        const double det = a * (d * f - e * e) + b * (c * e - b * f) + c * (b * e - c * d);
+        if (!(det > 0) || !isfinite(det)) *fail = 1;
+    }
+    const int lane = threadIdx.x & 31, g = lane / 6, r = lane - 6 * g;
+    for (int s = gtid >> 5; s < nrq; s += gthreads >> 5) {
+        const int li = rq ? rq[s] : s;
+        const int o0 = mo_ptr[li], nO = mo_ptr[li + 1] - o0;
+        const int32_t *sig = mp_sig + mp_ptr[li];
+        double P[6] = { 0, 0, 0, 0, 0, 0 };      // (0,0) (1,0) (1,1) (2,0) (2,1) (2,2)
+        for (int a0 = 0; a0 < nO; a0 += 5) {
+            const int a = a0 + g;
+            if (g >= 5 || a >= nO) continue;
+            double z0 = 0, z1 = 0, z2 = 0;
+            const int32_t *sg = sig + (size_t)a * nO;
+            for (int b = 0; b < nO; ++b) {
+                const int t = sg[b];
+                const double *blk = Sig + (size_t)(t >> 1) * 36;
+                const double *yb = Y + (size_t)mo_obs[o0 + b] * 18;
+                double v[6];
+                if (t & 1) {
+#pragma unroll
+                    for (int m = 0; m < 6; ++m) v[m] = blk[m * 6 + r];
+                } else {
+#pragma unroll
+                    for (int m = 0; m < 6; ++m) v[m] = blk[r * 6 + m];
+                }
+#pragma unroll
+                for (int m = 0; m < 6; ++m) { z0 += v[m] * yb[m * 3]; z1 += v[m] * yb[m * 3 + 1]; z2 += v[m] * yb[m * 3 + 2]; }
+            }
+            const double *ya = Y + (size_t)mo_obs[o0 + a] * 18 + r * 3;
+            P[0] += ya[0] * z0; P[1] += ya[1] * z0; P[2] += ya[1] * z1;
+            P[3] += ya[2] * z0; P[4] += ya[2] * z1; P[5] += ya[2] * z2;
+            if (cl_ptr)
+                for (int q = cl_ptr[s]; q < cl_ptr[s + 1]; ++q)
+                    if (cl_a[q] == a) { double *o = pcl + (size_t)q * 18 + r * 3; o[0] = -z0; o[1] = -z1; o[2] = -z2; }
+        }
+#pragma unroll
+        for (int k = 0; k < 6; ++k)
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) P[k] += __shfl_xor_sync(0xffffffffu, P[k], off);
+        if (lane == 0) {
+            const double *D = Dinv + (size_t)li * 9;
+            const double v00 = D[0] + P[0], v10 = D[3] + P[1], v11 = D[4] + P[2], v20 = D[6] + P[3], v21 = D[7] + P[4], v22 = D[8] + P[5];
+            double *o = pdiag + (size_t)s * 9;
+            o[0] = v00; o[1] = v10; o[2] = v20;
+            o[3] = v10; o[4] = v11; o[5] = v21;
+            o[6] = v20; o[7] = v21; o[8] = v22;
+        }
+    }
+}
+
+// The requested blocks, back to back: src[k] = (index << 2) | kind, kind 0 camera-camera (cc, 6x6), 1 point diagonal
+// (pdiag, 3x3), 2 camera-point (pcl, 6x3), 3 point-camera (pcl transposed, 3x6); dst[k] = offset in out.
+// flag[1] = the factorisation's pivot flag (dfail, may be nullptr).
+__global__ void ba_marginal_gather_kernel(int n_pairs, const int32_t *__restrict__ src, const int64_t *__restrict__ dst,
+                                          const double *__restrict__ cc, const double *__restrict__ pdiag,
+                                          const double *__restrict__ pcl, const int *dfail, int *flag, double *__restrict__ out) {
+    const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (tid == 0) flag[1] = dfail ? *dfail : 0;
+    for (long long item = tid; item < (long long)n_pairs * 36; item += (long long)gridDim.x * blockDim.x) {
+        const int k = (int)(item / 36), e = (int)(item - (long long)k * 36);
+        const int kind = src[k] & 3, idx = src[k] >> 2;
+        double *o = out + dst[k];
+        if (kind == 0) o[e] = cc[(size_t)idx * 36 + e];
+        else if (kind == 1) { if (e < 9) o[e] = pdiag[(size_t)idx * 9 + e]; }
+        else if (e < 18) {
+            if (kind == 2) o[e] = pcl[(size_t)idx * 18 + e];
+            else { const int a = e / 6, b = e - 6 * a; o[e] = pcl[(size_t)idx * 18 + b * 3 + a]; }
+        }
+    }
+}
+
 __global__ void ba_pack_kernel(const double *__restrict__ aos, int n, int n_pad, int dim, double *__restrict__ soa) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n * dim) return;
@@ -494,6 +604,12 @@ void ba_free_device(BaState &B) {
     dev_free(B.d_Hpp); dev_free(B.d_bp); dev_free(B.d_Hll); dev_free(B.d_bl);
     dev_free(B.d_Dinv); dev_free(B.d_dl); dev_free(B.d_xl);
     dev_free(B.d_cam_snap); dev_free(B.d_pt_snap);
+    dev_free(B.d_mo_ptr); dev_free(B.d_mo_obs); dev_free(B.d_mp_sig); dev_free(B.d_mp_ptr);
+    dev_free(B.d_mrq); dev_free(B.d_mcl_ptr); dev_free(B.d_mcl_a); dev_free(B.d_msrc); dev_free(B.d_mdst);
+    dev_free(B.d_mpt); dev_free(B.d_mout); dev_free(B.d_mflag);
+    B.cap_mrq = B.cap_mcl_ptr = B.cap_mcl_a = B.cap_msrc = B.cap_mdst = B.cap_mpt = B.cap_mout = 0;
+    B.marg_lists = false;
+    B.marg_check = -1;
 }
 
 int upload_soa(s3o_problem *p, const std::vector<double> &aos, int n, int n_pad, int dim, double *soa) {
@@ -631,6 +747,8 @@ int ba_build_structure(s3o_problem *p) {
         }
     }
     B.ncon = con.size();
+    B.pt_ptr = pt_ptr;
+    B.socam = socam;
     // ---- device ---------------------------------------------------------------------------
     int rc = 0;
     rc = rc ? rc : upload_structure_arrays(p, S.nf);
@@ -670,8 +788,8 @@ int ba_build_structure(s3o_problem *p) {
         cudaMemsetAsync(B.d_pt[w], 0, (size_t)B.np_pad * 3 * sizeof(double), p->stream);
     }
     cudaMemsetAsync(B.d_uv, 0, (size_t)B.no_pad * 2 * sizeof(double), p->stream);
-    cudaMemsetAsync(B.d_xl, 0, (size_t)std::max(B.npf, 1) * 3 * sizeof(double), p->stream);
-    cudaMemsetAsync(p->d_x, 0, (size_t)std::max(S.nf, 1) * 6 * sizeof(double), p->stream);
+    cudaMemsetAsync(B.d_xl, 0, (size_t)B.npf * 3 * sizeof(double), p->stream);     // (no free point / camera: 0 bytes)
+    cudaMemsetAsync(p->d_x, 0, (size_t)S.nf * 6 * sizeof(double), p->stream);
     p->cur = 0;
     rc = rc ? rc : upload_soa(p, B.cam0, B.nc, B.nc_pad, 7, B.d_cam[0]);
     rc = rc ? rc : upload_soa(p, B.pt0, B.np, B.np_pad, 3, B.d_pt[0]);
@@ -778,6 +896,120 @@ int ba_snapshot(s3o_problem *p, int restore) {
     S3O_CUDA(cudaMemcpyAsync(B.d_pt[p->cur], B.d_pt_snap, pb, cudaMemcpyDeviceToDevice, p->stream));
     return S3O_OK;
 }
+
+namespace {
+
+// Host checks of s3o_ba_compute_marginals, once per structure (B.marg_check / B.marg_msg).  H is singular when
+//  - a connected component of the camera-point observation graph holding a free vertex fixes neither a camera and one
+//    more vertex nor three points: the monocular 7-DoF gauge (scale included) is free;
+//  - a free point is seen by fewer than two distinct cameras: its Hll has rank <= 2.
+int ba_marginal_checks(BaState &B) {
+    if (B.marg_check >= 0) {
+        if (B.marg_check) set_error("%s", B.marg_msg.c_str());
+        return B.marg_check;
+    }
+    char msg[256] = "";
+    const int nv = B.nc + B.np;
+    std::vector<int32_t> root(nv);
+    for (int v = 0; v < nv; ++v) root[v] = v;
+    auto find = [&](int v) { while (root[v] != v) v = root[v] = root[root[v]]; return v; };
+    for (int k = 0; k < B.no; ++k) {
+        const int a = find(B.ocam[k]), b = find(B.nc + B.opt[k]);
+        if (a != b) root[std::max(a, b)] = std::min(a, b);
+    }
+    std::vector<int32_t> fcam(nv, 0), fpt(nv, 0);
+    for (int c = 0; c < B.nc; ++c) if (B.cfix[c]) fcam[find(c)]++;
+    for (int l = 0; l < B.np; ++l) if (B.pfix[l]) fpt[find(B.nc + l)]++;
+    for (int v = 0; v < nv && !msg[0]; ++v) {
+        const bool is_cam = v < B.nc;
+        if (is_cam ? B.cfix[v] : B.pfix[v - B.nc]) continue;
+        const int r = find(v);
+        if ((fcam[r] >= 1 && fcam[r] + fpt[r] >= 2) || fpt[r] >= 3) continue;
+        snprintf(msg, sizeof msg, "s3o_ba_compute_marginals: the Hessian is singular: the connected component of %s %d "
+                 "fixes %d camera(s) and %d point(s), not a camera and one more vertex or three points (its 7-DoF gauge is free)",
+                 is_cam ? "camera" : "point", is_cam ? v : v - B.nc, fcam[r], fpt[r]);
+    }
+    std::vector<int32_t> cams;
+    for (int l = 0; l < B.np && !msg[0]; ++l) {
+        if (B.pfix[l]) continue;
+        cams.assign(B.socam.begin() + B.pt_ptr[l], B.socam.begin() + B.pt_ptr[l + 1]);
+        std::sort(cams.begin(), cams.end());
+        const int distinct = (int)(std::unique(cams.begin(), cams.end()) - cams.begin());
+        if (distinct < 2)
+            snprintf(msg, sizeof msg, "s3o_ba_compute_marginals: the Hessian is singular: free point %d is seen by %d distinct "
+                     "camera(s); a free point needs two", l, distinct);
+    }
+    B.marg_msg = msg;
+    B.marg_check = msg[0] ? S3O_ERR_SOLVE : S3O_OK;
+    if (B.marg_check) set_error("%s", msg);
+    return B.marg_check;
+}
+
+// Point gather lists on the plan of the selected inverse (plan == nullptr: no free camera, empty lists), in point
+// order, then a-major over the point's free-camera observations: mo_ptr / mo_obs / mp_ptr / mp_sig of
+// ba_marginal_points_kernel.  Every pair of cameras co-observing a free point is a block of S, hence of L.
+int ba_marginal_lists(s3o_problem *p, BaState &B, const DirectPlan *plan, uint64_t serial) {
+    if (B.marg_lists && B.marg_serial == serial) return S3O_OK;
+    dev_free(B.d_mo_ptr); dev_free(B.d_mo_obs); dev_free(B.d_mp_sig); dev_free(B.d_mp_ptr);
+    B.marg_lists = false;
+    std::vector<int32_t> ipos(plan ? plan->n : 0);
+    for (int k = 0; plan && k < plan->n; ++k) ipos[plan->perm[k]] = k;
+    std::vector<int32_t> mo_ptr(B.npf + 1, 0), mo_obs, mp_sig, pos;
+    std::vector<int64_t> mp_ptr(B.npf + 1, 0);
+    for (int l = 0; l < B.np; ++l) {
+        const int li = B.phidx[l];
+        if (li < 0) continue;
+        pos.clear();
+        for (int t = B.pt_ptr[l]; t < B.pt_ptr[l + 1]; ++t) {
+            const int ci = B.chidx[B.socam[t]];
+            if (ci < 0) continue;
+            mo_obs.push_back(t);
+            pos.push_back(ipos[ci]);
+        }
+        const int nO = (int)pos.size();
+        mo_ptr[li + 1] = (int32_t)mo_obs.size();
+        mp_ptr[li + 1] = mp_ptr[li] + (int64_t)nO * nO;
+        const size_t base = mp_sig.size();
+        mp_sig.resize(base + (size_t)nO * nO);
+        for (int a = 0; a < nO; ++a)
+            for (int b = 0; b <= a; ++b) {
+                const int32_t t = direct_find_block(*plan, std::min(pos[a], pos[b]), std::max(pos[a], pos[b]));
+                if (t < 0) { set_error("s3o_ba_compute_marginals: internal error (co-observing cameras without a block of L)"); return S3O_ERR_INVALID; }
+                mp_sig[base + (size_t)a * nO + b] = (t << 1) | (pos[a] < pos[b] ? 1 : 0);
+                mp_sig[base + (size_t)b * nO + a] = (t << 1) | (pos[b] < pos[a] ? 1 : 0);
+            }
+    }
+    int rc = upload(p, &B.d_mo_ptr, mo_ptr);
+    rc = rc ? rc : upload(p, &B.d_mo_obs, mo_obs);
+    rc = rc ? rc : upload(p, &B.d_mp_ptr, mp_ptr);
+    rc = rc ? rc : upload(p, &B.d_mp_sig, mp_sig);
+    if (!rc && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = S3O_ERR_CUDA;
+    if (rc) { set_error("s3o_ba_compute_marginals: device allocation failed"); return rc; }
+    B.marg_lists = true;
+    B.marg_serial = serial;
+    return S3O_OK;
+}
+
+// device buffer of at least `need` elements (kept between calls)
+template <class T>
+int ensure_cap(T **ptr, size_t *cap, size_t need) {
+    if (*ptr && need <= *cap) return S3O_OK;
+    dev_free(*ptr);
+    *cap = 0;
+    const int rc = dev_alloc(ptr, need);
+    if (!rc) *cap = need;
+    return rc;
+}
+
+template <class T>
+int h2d(s3o_problem *p, T *dst, const std::vector<T> &v) {
+    if (v.empty()) return S3O_OK;
+    S3O_CUDA(cudaMemcpyAsync(dst, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, p->stream));
+    p->stats.h2d_bytes += (int64_t)(v.size() * sizeof(T));
+    return S3O_OK;
+}
+
+}  // namespace
 
 }  // namespace s3o
 
@@ -955,6 +1187,151 @@ int s3o_ba_get_schur(s3o_problem *p, double lambda, double *blocks, double *bs) 
     if (bs) {
         S3O_CUDA(cudaMemcpyAsync(bs, p->d_b, (size_t)p->S.nf * 6 * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
         S3O_CUDA(cudaStreamSynchronize(p->stream));
+    }
+    return S3O_OK;
+}
+
+// Marginal covariances of bundle adjustment: blocks of H^-1 for the undamped H = [[Hpp, Hpl], [Hpl^T, Hll]] at the
+// current estimates, from the selected inverse of the Schur complement (direct.cu) and the point phase above.
+int s3o_ba_compute_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out) {
+    if (!p || p->kind != S3O_KIND_BA || n_pairs < 0 || (!rows != !cols) || (n_pairs > 0 && !out)) {
+        set_error("s3o_ba_compute_marginals: bad arguments (the problem must be of kind S3O_KIND_BA)");
+        return S3O_ERR_INVALID;
+    }
+    if (p->dist) { set_error("s3o_ba_compute_marginals: not available with the partitioned solve"); return S3O_ERR_UNSUPPORTED; }
+    cudaSetDevice(p->device);
+    int rc = p->built ? S3O_OK : s3o_build_structure(p, nullptr, nullptr);
+    if (rc) return rc;
+    BaState &B = *p->ba;
+    const int ncf = B.ncf, npf = B.npf, n = ncf + npf;
+    if (n == 0) { set_error("s3o_ba_compute_marginals: 0 free vertices"); return S3O_ERR_INVALID; }
+    if (!rows && n_pairs != n) { set_error("s3o_ba_compute_marginals: the diagonal blocks need n_pairs = n_free_cameras + n_free_points = %d", n); return S3O_ERR_INVALID; }
+    for (int k = 0; rows && k < n_pairs; ++k)
+        if (rows[k] < 0 || rows[k] >= n || cols[k] < 0 || cols[k] >= n) {
+            set_error("s3o_ba_compute_marginals: pair %d (%d, %d) is not a pair of Hessian indices in [0, %d) (fixed vertices have none)",
+                      k, rows[k], cols[k], n);
+            return S3O_ERR_INVALID;
+        }
+    // ---- the requested pairs: camera-camera to the selected inverse, the rest to the point phase
+    std::vector<int32_t> src(n_pairs), cc_r, cc_c, rq, rq_slot, pid;
+    std::vector<int64_t> dst(n_pairs);
+    std::map<std::pair<int32_t, int32_t>, int32_t> cl;        // (point slot, observation a) -> camera-point slot
+    std::vector<std::pair<int32_t, int32_t>> pair_cl(n_pairs);
+    int64_t total = 0;
+    if (rows) rq_slot.assign(npf, -1);
+    auto point_slot = [&](int li) {
+        if (rq_slot[li] < 0) { rq_slot[li] = (int32_t)rq.size(); rq.push_back(li); }
+        return rq_slot[li];
+    };
+    for (int k = 0; k < n_pairs; ++k) {
+        const int r = rows ? rows[k] : k, c = cols ? cols[k] : k;
+        const bool rc_cam = r < ncf, cc_cam = c < ncf;
+        dst[k] = total;
+        total += (rc_cam ? 6 : 3) * (cc_cam ? 6 : 3);
+        if (!rows) { src[k] = k < ncf ? (k << 2) : ((k - ncf) << 2) | 1; continue; }
+        if (rc_cam && cc_cam) {
+            src[k] = ((int32_t)cc_r.size() << 2);
+            cc_r.push_back(r); cc_c.push_back(c);
+        } else if (!rc_cam && !cc_cam) {
+            if (r != c) { set_error("s3o_ba_compute_marginals: pair %d (%d, %d) joins two distinct points (not supported)", k, r, c); return S3O_ERR_UNSUPPORTED; }
+            src[k] = (point_slot(r - ncf) << 2) | 1;
+        } else {
+            const int ci = rc_cam ? r : c, li = (rc_cam ? c : r) - ncf;
+            if (pid.empty()) {
+                pid.resize(npf);
+                for (int q = 0; q < B.np; ++q) if (B.phidx[q] >= 0) pid[B.phidx[q]] = q;
+            }
+            const int l = pid[li];
+            int a = -1;
+            for (int t = B.pt_ptr[l], m = 0; t < B.pt_ptr[l + 1] && a < 0; ++t) {
+                const int cf = B.chidx[B.socam[t]];
+                if (cf == ci) a = m;
+                if (cf >= 0) ++m;
+            }
+            if (a < 0) {
+                set_error("s3o_ba_compute_marginals: pair %d (%d, %d): camera %d does not observe point %d (not supported)", k, r, c, ci, li + ncf);
+                return S3O_ERR_UNSUPPORTED;
+            }
+            pair_cl[k] = { point_slot(li), a };
+            cl.emplace(pair_cl[k], 0);
+            src[k] = rc_cam ? 2 : 3;
+        }
+    }
+    if ((rc = ba_marginal_checks(B))) return rc;
+    // camera-point slots grouped by point slot
+    const int nrq = rows ? (int)rq.size() : npf;
+    std::vector<int32_t> cl_ptr, cl_a;
+    if (!cl.empty()) {
+        cl_ptr.assign(nrq + 1, 0);
+        for (auto &kv : cl) { kv.second = (int32_t)cl_a.size(); cl_a.push_back(kv.first.second); cl_ptr[kv.first.first + 1]++; }
+        for (int s = 0; s < nrq; ++s) cl_ptr[s + 1] += cl_ptr[s];
+        for (int k = 0; k < n_pairs; ++k)
+            if ((src[k] & 3) >= 2) src[k] |= cl.at(pair_cl[k]) << 2;
+    }
+    // ---- plan, lists and buffers (host work and uploads, before anything runs)
+    MarginalsRun R;
+    const int n_cc = rows ? (int)cc_r.size() : ncf;
+    if (ncf > 0 && (rc = marginals_open(p, "s3o_ba_compute_marginals", n_cc, rows ? cc_r.data() : nullptr,
+                                        rows ? cc_c.data() : nullptr, &R)))
+        return rc;
+    if ((rc = ba_marginal_lists(p, B, ncf > 0 ? R.plan : nullptr, R.serial))) return rc;
+    rc = ensure_cap(&B.d_msrc, &B.cap_msrc, (size_t)n_pairs);
+    rc = rc ? rc : ensure_cap(&B.d_mdst, &B.cap_mdst, (size_t)n_pairs);
+    rc = rc ? rc : ensure_cap(&B.d_mpt, &B.cap_mpt, (size_t)nrq * 9 + cl_a.size() * 18);
+    rc = rc ? rc : ensure_cap(&B.d_mout, &B.cap_mout, (size_t)total);
+    if (!rc && !B.d_mflag) rc = dev_alloc(&B.d_mflag, 2);
+    if (!rc && rows) rc = ensure_cap(&B.d_mrq, &B.cap_mrq, rq.size());
+    if (!rc && !cl_a.empty()) rc = ensure_cap(&B.d_mcl_ptr, &B.cap_mcl_ptr, cl_ptr.size());
+    if (!rc && !cl_a.empty()) rc = ensure_cap(&B.d_mcl_a, &B.cap_mcl_a, cl_a.size());
+    if (rc) { set_error("s3o_ba_compute_marginals: device allocation failed"); return rc; }
+    if ((rc = h2d(p, B.d_msrc, src)) || (rc = h2d(p, B.d_mdst, dst)) || (rc = h2d(p, B.d_mrq, rq)) ||
+        (rc = h2d(p, B.d_mcl_ptr, cl_ptr)) || (rc = h2d(p, B.d_mcl_a, cl_a)))
+        return rc;
+    S3O_CUDA(cudaMemsetAsync(B.d_mflag, 0, 2 * sizeof(int), p->stream));
+    // ---- linearize | Schur (lambda = 0) | factor | selected inverse | points | gather
+    cudaEvent_t *ev = p->ev;
+    cudaEventRecord(ev[0], p->stream);
+    if ((rc = ba_linearize(p))) return rc;
+    cudaEventRecord(ev[1], p->stream);
+    rc = ba_form_schur(p, 0.0);
+    p->linearized = false;          // p->d_b holds the undamped Schur right-hand side: the next solve linearises again
+    direct_invalidate(p);
+    if (rc) return rc;
+    cudaEventRecord(ev[2], p->stream);
+    if (ncf > 0) {
+        if ((rc = marginals_factor(p, R, ev + 3))) return rc;
+    } else {
+        cudaEventRecord(ev[3], p->stream);
+        cudaEventRecord(ev[4], p->stream);
+    }
+    int launches = 1;
+    if (npf > 0) {
+        const int grid = (int)std::max<long long>(1, std::min<long long>(148 * 8, ((long long)std::max(nrq, npf) * 32 + kMargNT - 1) / kMargNT));
+        ba_marginal_points_kernel<<<grid, kMargNT, 0, p->stream>>>(
+            npf, nrq, rows ? B.d_mrq : nullptr, B.d_mo_ptr, B.d_mo_obs, B.d_mp_ptr, B.d_mp_sig, ncf > 0 ? R.Sig : nullptr,
+            B.d_Y, B.d_Dinv, B.d_Hll, cl_a.empty() ? nullptr : B.d_mcl_ptr, B.d_mcl_a, B.d_mpt, B.d_mpt + (size_t)nrq * 9, B.d_mflag);
+        ++launches;
+    }
+    cudaEventRecord(ev[5], p->stream);
+    if (ncf > 0 && (rc = marginals_pick(p, R, n_cc))) return rc;
+    if (n_pairs > 0)
+        ba_marginal_gather_kernel<<<(int)std::min<long long>(1024, ((long long)n_pairs * 36 + 255) / 256), 256, 0, p->stream>>>(
+            n_pairs, B.d_msrc, B.d_mdst, ncf > 0 ? R.out : nullptr, B.d_mpt, B.d_mpt + (size_t)nrq * 9, ncf > 0 ? R.fail : nullptr,
+            B.d_mflag, B.d_mout);
+    cudaEventRecord(ev[6], p->stream);
+    if ((rc = check_launch(p, launches))) return rc;
+    int flag[2] = { 0, 0 };
+    if (total > 0) S3O_CUDA(cudaMemcpyAsync(out, B.d_mout, sizeof(double) * total, cudaMemcpyDeviceToHost, p->stream));
+    S3O_CUDA(cudaMemcpyAsync(flag, B.d_mflag, sizeof flag, cudaMemcpyDeviceToHost, p->stream));
+    S3O_CUDA(cudaStreamSynchronize(p->stream));
+    p->stats.d2h_bytes += total * 8 + (int64_t)sizeof flag;
+    if (flag[1]) { set_error("s3o_ba_compute_marginals: the Schur complement is not positive definite (a pivot of its factorisation failed)"); return S3O_ERR_SOLVE; }
+    if (flag[0]) { set_error("s3o_ba_compute_marginals: a free point's Hll is not positive definite (det <= 0 or not finite)"); return S3O_ERR_SOLVE; }
+    if (getenv("S3O_MARGINALS_TRACE")) {     // per-phase CUDA-event times (tools/marginals_probe.py --ba)
+        float ms[6] = {};
+        for (int k = 0; k < 6; ++k) cudaEventElapsedTime(&ms[k], ev[k], ev[k + 1]);
+        fprintf(stderr, "s3o_ba_compute_marginals: linearize %.4f schur %.4f factor %.4f selinv %.4f points %.4f gather %.4f ms\n",
+                ms[0], ms[1], ms[2], ms[3], ms[4], ms[5]);
     }
     return S3O_OK;
 }

@@ -51,6 +51,8 @@ struct DirectState {
     int32_t *d_pick = nullptr, *d_crow = nullptr, *d_cdst = nullptr;
     double *d_out = nullptr;
     int out_cap = 0;            // pairs d_pick / d_crow / d_cdst / d_out hold
+    std::vector<int32_t> col_ptr, col_id;       // the requested pairs off the pattern, by block column (marginals_open)
+    uint64_t serial = 0;        // plan_and_upload's count: the plan's identity for gather lists kept elsewhere
     // the plan of the marginals under the forced cap, when the linear solver has none of its own (PCG)
     DirectState *marg = nullptr;
 };
@@ -548,6 +550,8 @@ static constexpr int kAutoMaxLevels = 128;
 
 // Symbolic analysis of p->S into D under the limits and upload; D->available says whether the plan stayed within them.
 static int plan_and_upload(s3o_problem *p, DirectState *D, long long max_pairs, int max_levels) {
+    static uint64_t plans = 0;
+    D->serial = ++plans;
     D->analyzed = true;
     D->available = false;
     if (!direct_analyze(p->S.nf, p->S.rowptr, p->S.colidx, max_pairs, D->plan)) return S3O_OK;
@@ -652,18 +656,26 @@ int direct_solve(s3o_problem *p, double lambda, bool reuse_factor) {
 
 namespace {
 
+// factorisation of H without damping and its selected inverse; ev (may be nullptr): 2 events, after each
 template <int D>
-int marginals_launches(s3o_problem *p, DirectState *S, int n_pairs, const std::vector<int32_t> &col_ptr,
-                       const std::vector<int32_t> &col_id, cudaEvent_t *ev) {
+int factor_launches(s3o_problem *p, DirectState *S, cudaEvent_t *ev) {
     const DirectDev P = device_view(S);
     const SelinvDev Sv{ S->d_sel_ptr, S->d_sel_sig, S->d_Sig };
-    const int nd = S->plan.n * D;
     int rc = launch_direct<D>(p, S, P, 0.0, 1, S->d_E, S->d_X, S->d_msc);     // H = L L^T (no damping)
     if (rc) return rc;
     if (ev) cudaEventRecord(ev[0], p->stream);
     if ((rc = launch_selinv<D>(p, S, P, Sv))) return rc;
     if (ev) cudaEventRecord(ev[1], p->stream);
-    int launches = 2;
+    return check_launch(p, 2);
+}
+
+// the requested blocks into d_out: on the pattern from the selected inverse, off it from column solves
+template <int D>
+int pick_launches(s3o_problem *p, DirectState *S, int n_pairs) {
+    const DirectDev P = device_view(S);
+    const std::vector<int32_t> &col_ptr = S->col_ptr, &col_id = S->col_id;
+    const int nd = S->plan.n * D;
+    int rc, launches = 0;
     if (n_pairs > 0) {
         const int grid = (int)std::min<long long>(1024, ((long long)n_pairs * D * D + 255) / 256);
         marg_pick_kernel<D><<<grid, 256, 0, p->stream>>>(S->d_Sig, S->d_pick, n_pairs, S->d_out);
@@ -679,7 +691,6 @@ int marginals_launches(s3o_problem *p, DirectState *S, int n_pairs, const std::v
             S->d_X, nd, S->d_crow + col_ptr[g], S->d_cdst + col_ptr[g], cnt, S->d_out);
         launches += D + 2;
     }
-    if (ev) cudaEventRecord(ev[2], p->stream);
     return check_launch(p, launches);
 }
 
@@ -689,8 +700,8 @@ void free_marginal_arrays(DirectState *S) {
 
 }  // namespace
 
-// Marginal covariances for the H in p->d_H (see problem.h).
-int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev) {
+// Plan, buffers and pair lists of one marginals call (see problem.h).
+int marginals_open(s3o_problem *p, const char *who, int n_pairs, const int32_t *rows, const int32_t *cols, MarginalsRun *R) {
     // the plan: the linear solver's own when it has one (the same analysis, only the size limits differ), otherwise
     // one under the forced cap kept for the marginals -- the choice of the linear solver does not move
     DirectState *S = nullptr;
@@ -707,7 +718,7 @@ int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int
             if ((rc = plan_and_upload(p, M, kForcedMaxPairs, INT_MAX))) { delete M; M = nullptr; return rc; }
         }
         if (!M->available) {
-            set_error("s3o_compute_marginals: the factor of this graph needs more than %lld block products", kForcedMaxPairs);
+            set_error("%s: the factor of this graph needs more than %lld block products", who, kForcedMaxPairs);
             return S3O_ERR_UNSUPPORTED;
         }
         S = M;
@@ -725,7 +736,7 @@ int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int
         rc = rc ? rc : dev_alloc(&S->d_Sig, Pl.brow.size() * dd);
         if (!rc && cudaMemsetAsync(S->d_E, 0, sizeof(double) * n * dd, p->stream) != cudaSuccess) rc = S3O_ERR_CUDA;
         if (!rc && cudaStreamSynchronize(p->stream) != cudaSuccess) rc = S3O_ERR_CUDA;
-        if (rc) { free_marginal_arrays(S); set_error("s3o_compute_marginals: device allocation failed"); return rc; }
+        if (rc) { free_marginal_arrays(S); set_error("%s: device allocation failed", who); return rc; }
     }
     // requested pairs -> block of Sigma (elimination order) and transpose flag; the rest by block column
     std::vector<int32_t> ipos(n);
@@ -740,13 +751,15 @@ int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int
         if (t < 0) off.push_back({ c, k });
     }
     std::sort(off.begin(), off.end());
-    std::vector<int32_t> col_ptr, col_id, crow(off.size()), cdst(off.size());
+    std::vector<int32_t> crow(off.size()), cdst(off.size());
+    S->col_ptr.clear();
+    S->col_id.clear();
     for (size_t q = 0; q < off.size(); ++q) {
-        if (q == 0 || off[q].first != off[q - 1].first) { col_ptr.push_back((int32_t)q); col_id.push_back(off[q].first); }
+        if (q == 0 || off[q].first != off[q - 1].first) { S->col_ptr.push_back((int32_t)q); S->col_id.push_back(off[q].first); }
         crow[q] = rows[off[q].second];
         cdst[q] = off[q].second;
     }
-    if (!off.empty()) col_ptr.push_back((int32_t)off.size());
+    if (!off.empty()) S->col_ptr.push_back((int32_t)off.size());
     if (n_pairs > S->out_cap) {
         dev_free(S->d_pick); dev_free(S->d_crow); dev_free(S->d_cdst); dev_free(S->d_out);
         S->out_cap = 0;
@@ -754,7 +767,7 @@ int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int
         rc = rc ? rc : dev_alloc(&S->d_crow, (size_t)n_pairs);
         rc = rc ? rc : dev_alloc(&S->d_cdst, (size_t)n_pairs);
         rc = rc ? rc : dev_alloc(&S->d_out, (size_t)n_pairs * dd);
-        if (rc) { set_error("s3o_compute_marginals: device allocation failed"); return rc; }
+        if (rc) { set_error("%s: device allocation failed", who); return rc; }
         S->out_cap = n_pairs;
     }
     auto h2d = [&](int32_t *dst, const std::vector<int32_t> &v) -> int {
@@ -764,17 +777,50 @@ int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int
         return S3O_OK;
     };
     if ((rc = h2d(S->d_pick, pick)) || (rc = h2d(S->d_crow, crow)) || (rc = h2d(S->d_cdst, cdst))) return rc;
-    switch (d) {
-    case 7: rc = marginals_launches<7>(p, S, n_pairs, col_ptr, col_id, ev); break;
-    case 4: rc = marginals_launches<4>(p, S, n_pairs, col_ptr, col_id, ev); break;
-    case 1: rc = marginals_launches<1>(p, S, n_pairs, col_ptr, col_id, ev); break;
-    default: set_error("s3o_compute_marginals: block dimension %d", d); return S3O_ERR_UNSUPPORTED;
+    R->S = S;
+    R->plan = &S->plan;
+    R->serial = S->serial;
+    R->Sig = S->d_Sig;
+    R->out = S->d_out;
+    R->fail = S->d_fail;
+    return S3O_OK;
+}
+
+int marginals_factor(s3o_problem *p, const MarginalsRun &R, cudaEvent_t *ev) {
+    int rc;
+    switch (p->d) {
+    case 7: rc = factor_launches<7>(p, R.S, ev); break;
+    case 6: rc = factor_launches<6>(p, R.S, ev); break;
+    case 4: rc = factor_launches<4>(p, R.S, ev); break;
+    case 1: rc = factor_launches<1>(p, R.S, ev); break;
+    default: set_error("marginals: block dimension %d", p->d); return S3O_ERR_UNSUPPORTED;
     }
-    S->factored = false;      // the factor of H without damping: a later solve with reuse_factor factorises again
+    R.S->factored = false;      // the factor of H without damping: a later solve with reuse_factor factorises again
+    return rc;
+}
+
+int marginals_pick(s3o_problem *p, const MarginalsRun &R, int n_pairs) {
+    switch (p->d) {
+    case 7: return pick_launches<7>(p, R.S, n_pairs);
+    case 6: return pick_launches<6>(p, R.S, n_pairs);
+    case 4: return pick_launches<4>(p, R.S, n_pairs);
+    case 1: return pick_launches<1>(p, R.S, n_pairs);
+    }
+    set_error("marginals: block dimension %d", p->d);
+    return S3O_ERR_UNSUPPORTED;
+}
+
+// Marginal covariances for the H in p->d_H (see problem.h).
+int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev) {
+    MarginalsRun R;
+    int rc = marginals_open(p, "s3o_compute_marginals", n_pairs, rows, cols, &R);
     if (rc) return rc;
+    if ((rc = marginals_factor(p, R, ev)) || (rc = marginals_pick(p, R, n_pairs))) return rc;
+    if (ev) cudaEventRecord(ev[2], p->stream);
+    const int dd = p->d * p->d;
     int failed = 0;
-    if (n_pairs > 0) S3O_CUDA(cudaMemcpyAsync(out, S->d_out, sizeof(double) * n_pairs * dd, cudaMemcpyDeviceToHost, p->stream));
-    S3O_CUDA(cudaMemcpyAsync(&failed, S->d_fail, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
+    if (n_pairs > 0) S3O_CUDA(cudaMemcpyAsync(out, R.out, sizeof(double) * n_pairs * dd, cudaMemcpyDeviceToHost, p->stream));
+    S3O_CUDA(cudaMemcpyAsync(&failed, R.fail, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
     S3O_CUDA(cudaStreamSynchronize(p->stream));
     p->stats.d2h_bytes += (int64_t)n_pairs * dd * 8 + 4;
     if (failed) { set_error("s3o_compute_marginals: the Hessian is not positive definite (a pivot of its factorisation failed)"); return S3O_ERR_SOLVE; }

@@ -28,6 +28,7 @@ void dev_free(T *&ptr) {
 struct BaState;   // bundle adjustment (ba.cu)
 struct AmgState;  // multilevel preconditioner (amg.cu)
 struct DirectState;  // sparse block Cholesky (direct.cu)
+struct DirectPlan;   // its symbolic analysis (direct.h)
 
 }  // namespace s3o
 
@@ -118,7 +119,7 @@ struct s3o_problem {
     int spmv_ev_iter[kSpmvEvents] = {};     // PCG iteration (launch index within the solve) of each sample
     // statistics
     s3o_stats stats{};
-    cudaEvent_t ev[6] = {};
+    cudaEvent_t ev[8] = {};
     // bundle adjustment (kind S3O_KIND_BA): cameras / points / observations live in ba.cu
     s3o::BaState *ba = nullptr;
     // multilevel preconditioner of the pose-graph PCG (amg.cu), built on first use
@@ -169,6 +170,24 @@ void direct_destroy(s3o_problem *p);
 // does not change), then runs the selected inverse.  Leaves p->d_b / p->d_x / p->d_sc untouched and no factor held.
 // ev (may be nullptr): 3 events recorded after the factorisation, the selected inverse and the gather.
 int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev);
+// The same call in steps, so that the BA marginals (ba.cu) can run their point phase on the selected inverse:
+//   marginals_open    plan choice, first-call buffers and gather lists, the requested pairs' lists (host + upload);
+//                     errors are reported as "<who>: ..."
+//   marginals_factor  factorisation of p->d_H without damping and the selected inverse (launches; ev: 2 events)
+//   marginals_pick    the requested blocks into run.out, [n_pairs][d*d] (launches)
+// *fail is set on the device when a pivot fails.  serial identifies the plan: gather lists built on run.plan elsewhere
+// stay valid while it does not change.
+struct MarginalsRun {
+    DirectState *S = nullptr;
+    const DirectPlan *plan = nullptr;
+    uint64_t serial = 0;
+    const double *Sig = nullptr;     // [nL][d*d] selected inverse, laid out like L (elimination order)
+    const double *out = nullptr;
+    const int *fail = nullptr;
+};
+int marginals_open(s3o_problem *p, const char *who, int n_pairs, const int32_t *rows, const int32_t *cols, MarginalsRun *run);
+int marginals_factor(s3o_problem *p, const MarginalsRun &run, cudaEvent_t *ev);
+int marginals_pick(s3o_problem *p, const MarginalsRun &run, int n_pairs);
 // Launches a persistent kernel whose CTAs synchronise through grid_barrier (gridbar.cuh).  The kernel's LAST argument
 // is a GridBarrier; args[nargs - 1] must point to a GridBarrier that this call fills.
 inline int launch_persistent(s3o_problem *p, const void *func, int grid, int block, void **args, int nargs, size_t smem = 0) {

@@ -5,7 +5,12 @@ gather) and timed end to end on the host; medians over --reps calls after --warm
 blocks of L and block products, and for K1 / K118 the CPU oracle's dense inverse of the same H as a reference.
 One JSON line per graph.
 
-    python tools/marginals_probe.py [--reps 50] [--warmup 5]
+--ba: s3o_ba_compute_marginals (every camera and point diagonal block) on the graphs of tests/test_gpu_ba_marginals.py
+(ba_small, ba_medium and the bench-size ba_loop(1000, 500000, 10); cameras 0 and 7 and the points seen by fewer than
+two cameras fixed, Huber 2.5), split into linearise, Schur complement, factorisation, selected inverse, point phase and
+gather.  Also prints sum_l |O(l)|^2, the 6x6-by-6x3 products of the point phase.
+
+    python tools/marginals_probe.py [--ba] [--reps 50] [--warmup 5]
 """
 import argparse
 import json
@@ -51,16 +56,52 @@ class StderrCapture:
         self.f.close()
 
 
+def ba_main(a, gpu_info):
+    from sim3opt_b200 import synth
+    from test_ba_marginals_host import ba_fixings, hessian_indices, point_observations
+    from test_gpu_ba_marginals import make_ba
+    graphs = {"ba_small": synth.ba_loop(24, 300, 5, seed=11), "ba_medium": synth.ba_loop(120, 6000, 8, seed=5),
+              "ba_bench": synth.ba_loop(1000, 500000, 10, seed=42)}
+    names = ["linearize", "schur", "factor", "selinv", "points", "gather"]
+    for name, g in graphs.items():
+        cf, pf = ba_fixings(g)
+        ch, ph = hessian_indices(cf, pf)
+        products = int(sum(len(k) ** 2 for k in point_observations(g, ch, ph)))
+        p = make_ba(g, cf, pf)
+        reps = a.reps if name != "ba_bench" else max(3, a.reps // 5)
+        for _ in range(a.warmup):
+            p.ba_marginals()
+        wall = []
+        with StderrCapture() as cap:
+            for _ in range(reps):
+                t0 = time.perf_counter()
+                p.ba_marginals()
+                wall.append(time.perf_counter() - t0)
+        phases = np.array([[float(x) for x in line.split()[2:13:2]] for line in cap.text.splitlines()
+                           if line.startswith("s3o_ba_compute_marginals:")])
+        assert len(phases) == reps, cap.text[-2000:]
+        med = np.median(phases, 0)
+        st = p.stats()
+        rec = {"graph": name, "free_cameras": p.ncf, "free_points": p.npf, "schur_blocks": p.nb,
+               "factor_levels": st["direct_levels"], "factor_blocks": st["direct_blocks"], "point_products": products}
+        rec.update({"ms_" + n: float(v) for n, v in zip(names, med)})
+        rec.update(ms_call_wall=1e3 * float(np.median(wall)), reps=reps, gpu=gpu_info[:1])
+        print(json.dumps(rec), flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--ba", action="store_true")
     a = ap.parse_args()
     import sim3opt_b200 as s3
     from conftest import make_gpu, make_oracle
     from test_gpu_parity import dense_from_blocks
     gpu_info = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"],
                               capture_output=True, text=True).stdout.strip().splitlines()
+    if a.ba:
+        return ba_main(a, gpu_info)
     for name, g in graphs().items():
         plan = s3.host_direct_plan(len(g["est"]), g["fixed"], g["v0"], g["v1"], max_pairs=60000000)
         p = make_gpu(g, jac=1)
