@@ -206,16 +206,30 @@ int s3o_smallest_eigenvector(s3o_problem *p, int max_iter, double tol, double *x
  * rows/cols: n_pairs Hessian indices (s3o_get_hessian_index; fixed vertices have none); out: n_pairs x d x d,
  * row-major, block (rows[k], cols[k]).  rows == cols == NULL: every diagonal block in Hessian order
  * (n_pairs must equal n_free).  S3O_ERR_SOLVE when H is singular (a connected component without a fixed
- * vertex); S3O_ERR_UNSUPPORTED for BA (s3o_ba_compute_marginals), the partitioned solve, and graphs whose factor
- * exceeds the forced cap.
+ * vertex); S3O_ERR_UNSUPPORTED for BA (s3o_ba_compute_marginals), the partitioned solve, and the NULL form on a
+ * graph whose factor exceeds the forced cap.
  * Every call linearises again at the current estimates, so the result does not depend on what ran before it
  * (g2o uses the H of its last buildSystem, which is one step behind the estimates optimize() returns).  H is
  * factorised by the sparse block Cholesky (a plan under the forced cap of s3o_set_linear_solver(DIRECT) when the
  * linear solver in use has none; the linear solver the LM picks does not change), and the selected inverse gives
  * every block on the pattern of the factor -- all diagonal blocks and every pair joined by an edge -- for about
  * twice the block products of the factorisation.  A pair off that pattern costs d triangular solves for each
- * distinct column vertex among such pairs.  Like s3o_smallest_eigenvector, the call leaves the problem
- * unlinearised (s3o_solve needs s3o_linearize again). */
+ * distinct column vertex among such pairs.
+ * Beyond the forced cap (the 100k- and 1M-pose graphs) explicit pairs take an iterative route instead: the pairs
+ * are grouped by column vertex c, and for each distinct c the d right-hand sides H x = e_(c,m), m = 0..d-1, are
+ * solved by PCG without damping (the multilevel preconditioner for the Sim3, scale-trans and scale kinds under the
+ * difference scale model, block-Jacobi otherwise), each refined until its true residual |e - H x|_2 is at most
+ * S3O_MARGINALS_PCG_TOL (|e| = 1); where fp64 cannot resolve that (the residual's rounding floor eps |H| |x| lies
+ * above it when kappa(H) ~ 1e12), refinement stops once a round no longer halves the residual, provided the
+ * normwise backward error |e - H x| / (|H|_F |x|) is at most 1e-13.  Cost: d PCG solves per distinct column vertex, whatever the number of rows
+ * requested with it.  Block (r, c) is always column c's solve; diagonal blocks come back exactly symmetric,
+ * (X + X^T) / 2.  A solve that misses the tolerance within 20 000 PCG iterations, or breaks down, returns
+ * S3O_ERR_SOLVE naming the column vertex, the component and the residual reached.  The NULL form would take
+ * n_free * d solves there and returns S3O_ERR_UNSUPPORTED: request explicit pairs.  The environment variable
+ * S3O_MARGINALS_ROUTE=pcg takes the iterative route on any graph (to compare both routes on one H).  The LM's
+ * state (lambda, its scalars, the preconditioner choice) and the solver statistics are the same after the call.
+ * Like s3o_smallest_eigenvector, the call leaves the problem unlinearised (s3o_solve needs s3o_linearize again). */
+#define S3O_MARGINALS_PCG_TOL 1e-10
 int s3o_compute_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out);
 
 /* ---- the hot call (replaces optimizer.optimize(n)) ------------------------------------- */

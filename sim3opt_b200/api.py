@@ -199,7 +199,11 @@ class Problem:
     def marginals(self, pairs=None):
         """Marginal covariances (g2o SparseOptimizer::computeMarginals): blocks of H^-1, H the undamped Gauss-Newton
         Hessian at the current estimates.  pairs=None: the (n_free, d, d) diagonal blocks in Hessian order; otherwise
-        an (m, 2) array of Hessian-index pairs (row, col) -> (m, d, d)."""
+        an (m, 2) array of Hessian-index pairs (row, col) -> (m, d, d).
+        Within the sparse Cholesky's forced cap the blocks come from the selected inverse of its factor.  Beyond it
+        (s100k, S1M) only explicit pairs are served, by d PCG solves per distinct column vertex, each refined to a
+        true residual |e - H x| <= 1e-10 (S3O_MARGINALS_PCG_TOL); pairs=None raises there.  S3O_MARGINALS_ROUTE=pcg
+        in the environment takes the iterative route on any graph."""
         self.build_structure()
         if pairs is None:
             out = np.zeros((self.num_free, self.d, self.d))

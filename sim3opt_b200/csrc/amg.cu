@@ -1664,7 +1664,7 @@ int update_values_t(s3o_problem *p, double lambda) {
 // direction p = (zJ + P0 x_1) + beta p.  z holds zJ = D^-1 r on entry and is not completed -- nothing needs z
 // itself.  init: first application of a solve (p = z).
 template <int D>
-int apply_t(s3o_problem *p, int init) {
+int apply_t(s3o_problem *p, int init, double tol, int max_iter) {
     AmgState *st = p->amg;
     const int nl = (int)st->lev.size();
     const DevScalars *sc = p->d_sc;
@@ -1828,7 +1828,7 @@ int apply_t(s3o_problem *p, int init) {
         int dgrid = (L.n * D + NT - 1) / NT;
         if (dgrid > 148) dgrid = 148;
         if (dgrid < 1) dgrid = 1;
-        amg_coarse_dot_kernel<NT><<<dgrid, NT, 0, s>>>(L.n * D, L.r, L.x, p->d_partials, p->d_sc, init, p->pcg_tol, p->pcg_max_iter);
+        amg_coarse_dot_kernel<NT><<<dgrid, NT, 0, s>>>(L.n * D, L.r, L.x, p->d_partials, p->d_sc, init, tol, max_iter);
         amg_prolong0_kernel<D, NT><<<grid, NT, 0, s>>>(rows, L.agg, L.rel, L.pad_fine, L.x, p->d_z, p->d_p, sc, init);
         launches += 2;
         trace_mark(p, "coarse dot + fine prolong");
@@ -1853,8 +1853,8 @@ int amg_update_values(s3o_problem *p, double lambda) {
     S3O_AMG_DISPATCH((update_values_t<7, S3O_KIND_SIM3>(p, lambda)), (update_values_t<4, S3O_KIND_SCALE_TRANS>(p, lambda)),
                      (update_values_t<1, S3O_KIND_SCALE>(p, lambda)))
 }
-int amg_apply(s3o_problem *p, int init) {
-    S3O_AMG_DISPATCH(apply_t<7>(p, init), apply_t<4>(p, init), apply_t<1>(p, init))
+int amg_apply(s3o_problem *p, int init, double tol, int max_iter) {
+    S3O_AMG_DISPATCH(apply_t<7>(p, init, tol, max_iter), apply_t<4>(p, init, tol, max_iter), apply_t<1>(p, init, tol, max_iter))
 }
 #undef S3O_AMG_DISPATCH
 
@@ -1862,6 +1862,9 @@ void amg_counts(const s3o_problem *p, int64_t *rebuilds, int64_t *reuses) {
     if (!rebuilds || !reuses) { if (p->amg) p->amg->rebuilds = p->amg->reuses = 0; return; }
     *rebuilds = p->amg ? p->amg->rebuilds : 0;
     *reuses = p->amg ? p->amg->reuses : 0;
+}
+void amg_set_counts(s3o_problem *p, int64_t rebuilds, int64_t reuses) {
+    if (p->amg) { p->amg->rebuilds = rebuilds; p->amg->reuses = reuses; }
 }
 void amg_invalidate_frames(s3o_problem *p) { if (p->amg) { p->amg->frames_valid = false; p->amg->lin_changed = true; } }
 

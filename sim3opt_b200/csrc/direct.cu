@@ -15,6 +15,7 @@
 
 #include <algorithm>
 #include <climits>
+#include <cstring>
 
 #include "direct.h"
 #include "problem.h"
@@ -700,28 +701,44 @@ void free_marginal_arrays(DirectState *S) {
 
 }  // namespace
 
-// Plan, buffers and pair lists of one marginals call (see problem.h).
-int marginals_open(s3o_problem *p, const char *who, int n_pairs, const int32_t *rows, const int32_t *cols, MarginalsRun *R) {
-    // the plan: the linear solver's own when it has one (the same analysis, only the size limits differ), otherwise
-    // one under the forced cap kept for the marginals -- the choice of the linear solver does not move
-    DirectState *S = nullptr;
+// The plan of the marginals: the linear solver's own when it has one (the same analysis, only the size limits
+// differ), otherwise one under the forced cap kept for the marginals -- the choice of the linear solver does not move.
+// *S = nullptr when the factor exceeds the forced cap (the analysis is run once and its verdict kept).
+static int marginals_plan(s3o_problem *p, DirectState **S) {
+    *S = nullptr;
     int rc;
     if (p->linsolver != S3O_LINSOLVER_PCG) {
         if ((rc = direct_setup(p))) return rc;
-        if (direct_available(p)) S = p->direct;
+        if (direct_available(p)) { *S = p->direct; return S3O_OK; }
     }
+    if (!p->direct) p->direct = new DirectState();
+    DirectState *&M = p->direct->marg;
+    if (!M) {
+        M = new DirectState();
+        if ((rc = plan_and_upload(p, M, kForcedMaxPairs, INT_MAX))) { delete M; M = nullptr; return rc; }
+    }
+    if (M->available) *S = M;
+    return S3O_OK;
+}
+
+int marginals_iterative(s3o_problem *p, bool *iterative) {
+    // S3O_MARGINALS_ROUTE=pcg: the iterative route also where the factor fits (both routes on the same H)
+    const char *route = getenv("S3O_MARGINALS_ROUTE");
+    if (route && !strcmp(route, "pcg")) { *iterative = true; return S3O_OK; }
+    DirectState *S = nullptr;
+    const int rc = marginals_plan(p, &S);
+    *iterative = !rc && !S;
+    return rc;
+}
+
+// Plan, buffers and pair lists of one marginals call (see problem.h).
+int marginals_open(s3o_problem *p, const char *who, int n_pairs, const int32_t *rows, const int32_t *cols, MarginalsRun *R) {
+    DirectState *S = nullptr;
+    int rc;
+    if ((rc = marginals_plan(p, &S))) return rc;
     if (!S) {
-        if (!p->direct) p->direct = new DirectState();
-        DirectState *&M = p->direct->marg;
-        if (!M) {
-            M = new DirectState();
-            if ((rc = plan_and_upload(p, M, kForcedMaxPairs, INT_MAX))) { delete M; M = nullptr; return rc; }
-        }
-        if (!M->available) {
-            set_error("%s: the factor of this graph needs more than %lld block products", who, kForcedMaxPairs);
-            return S3O_ERR_UNSUPPORTED;
-        }
-        S = M;
+        set_error("%s: the factor of this graph needs more than %lld block products", who, kForcedMaxPairs);
+        return S3O_ERR_UNSUPPORTED;
     }
     const DirectPlan &Pl = S->plan;
     const int n = Pl.n, d = p->d, dd = d * d;

@@ -239,6 +239,40 @@ int do_solve(s3o_problem *p, double lambda, int *status, int *iters, double *rel
             return S3O_ERR_UNSUPPORTED;
         }
     }
+    bool amg = false;
+    int rc;
+    if (wants_multilevel(p)) {
+        if ((rc = amg_setup(p))) return rc;
+        amg = amg_levels(p) > 0;
+    }
+    if ((rc = pcg_prepare(p, lambda, amg))) return rc;
+    if ((rc = pcg_iterate(p, lambda, amg, p->pcg_tol, p->pcg_max_iter))) return rc;
+    // AUTO on a small graph: block-Jacobi until a solve turns out to be ill-conditioned (small lambda on
+    // a long chain), the multilevel correction from the next solve on
+    // (and back once the multilevel solves get so cheap -- large lambda -- that its setup dominates)
+    if (p->precond == S3O_PRECOND_AUTO && (p->kind == S3O_KIND_SIM3 || p->kind == S3O_KIND_SCALE_TRANS)) {
+        if (!amg && p->h_sc->iters > 256) p->auto_multilevel = true;
+        else if (amg && p->auto_multilevel && p->h_sc->iters <= 8) p->auto_multilevel = false;
+    }
+    if (status) *status = p->h_sc->done ? p->h_sc->done : 2;
+    if (iters) *iters = p->h_sc->iters;
+    if (rel_res) *rel_res = p->h_sc->rr0 > 0 ? std::sqrt(p->h_sc->rr / p->h_sc->rr0) : 0.0;
+    return S3O_OK;
+}
+
+void hessian_product(s3o_problem *p, const double *x) { run_spmv(p, struct_view(p), 0.0, x, 0); }
+
+// Block-Jacobi inverses of (H + lambda I) and, with the multilevel correction, its Galerkin operators.
+int pcg_prepare(s3o_problem *p, double lambda, bool amg) {
+    launch_precond(p->d, p->d_H, p->d_rowptr, own_rows(p), lambda, p->d_Minv, p->d_sc, p->stream);
+    int rc = check_launch(p, 1);
+    if (!rc && amg) rc = amg_update_values(p, lambda);
+    return rc;
+}
+
+// PCG on (H + lambda I) x = p->d_b from x = 0, x in p->d_x, to the relative recurrence residual tol or max_iter
+// iterations; the verdict in p->h_sc (done, iters, rr, rr0).
+int pcg_iterate(s3o_problem *p, double lambda, bool amg, double tol, int max_iter) {
     const int nf = own_rows(p), d = p->d;
     const int dist = p->dist ? 1 : 0;
     const StructDev s = struct_view(p);
@@ -261,26 +295,19 @@ int do_solve(s3o_problem *p, double lambda, int *status, int *iters, double *rel
         }
         return S3O_OK;
     };
-    bool amg = false;
     int rc;
-    if (wants_multilevel(p)) {
-        if ((rc = amg_setup(p))) return rc;
-        amg = amg_levels(p) > 0;
-    }
-    launch_precond(d, p->d_H, p->d_rowptr, nf, lambda, p->d_Minv, p->d_sc, p->stream);
-    if (amg && (rc = amg_update_values(p, lambda))) return rc;
     // with the multilevel correction the vector kernels leave r.z to amg_apply (like the partitioned
     // solve leaves it to the all-reduce)
     const int defer = dist || amg;
-    launch_pcg_init(d, nf, p->d_b, p->d_Minv, p->d_x, p->d_r, p->d_z, p->d_p, p->d_partials, p->d_sc, p->pcg_tol,
-                    p->pcg_max_iter, defer, p->stream);
-    rc = check_launch(p, 2);
+    launch_pcg_init(d, nf, p->d_b, p->d_Minv, p->d_x, p->d_r, p->d_z, p->d_p, p->d_partials, p->d_sc, tol,
+                    max_iter, defer, p->stream);
+    rc = check_launch(p, 1);
     if (rc) return rc;
     if (amg) {      // restriction, V-cycle, r.z (riding on the r_1 all-gather when partitioned), p = z
-        if ((rc = amg_apply(p, 1))) return rc;
+        if ((rc = amg_apply(p, 1, tol, max_iter))) return rc;
     } else if (dist) {
         if ((rc = allreduce_sum(p, &p->d_sc->rz_new, 2))) return rc;
-        launch_pcg_fin_init(p->d_sc, p->pcg_tol, p->pcg_max_iter, p->stream);
+        launch_pcg_fin_init(p->d_sc, tol, max_iter, p->stream);
         p->stats.kernel_launches += 1;
     }
     // Iterations are launched in batches between host checks of the convergence flag; an iteration launched after
@@ -308,7 +335,7 @@ int do_solve(s3o_problem *p, double lambda, int *status, int *iters, double *rel
                               p->d_sc, defer, p->stream);
             trace_mark(p, "pcg_update");
             if (amg) {      // ... r.z, beta and p = z + beta p included
-                if ((rc = amg_apply(p, 0))) return rc;
+                if ((rc = amg_apply(p, 0, tol, max_iter))) return rc;
                 if (p->trace_state == 2) { trace_mark(p, "end"); p->trace_state = 3; }
                 continue;
             }
@@ -347,22 +374,12 @@ int do_solve(s3o_problem *p, double lambda, int *status, int *iters, double *rel
             }
         }
         p->spmv_ev_used = 0;
-        if (p->h_sc->done || launched >= p->pcg_max_iter + batch) break;
+        if (p->h_sc->done || launched >= max_iter + batch) break;
         batch = launched < 16 ? std::max(2, launched / 2) : std::min(64, launched);
     }
     p->stats.pcg_iterations += p->h_sc->iters;
     p->last_pcg_iters = p->h_sc->iters;
     if (p->h_sc->done != 1) p->stats.pcg_unconverged += 1;      // iteration cap or breakdown: the step is inexact
-    // AUTO on a small graph: block-Jacobi until a solve turns out to be ill-conditioned (small lambda on
-    // a long chain), the multilevel correction from the next solve on
-    // (and back once the multilevel solves get so cheap -- large lambda -- that its setup dominates)
-    if (p->precond == S3O_PRECOND_AUTO && (p->kind == S3O_KIND_SIM3 || p->kind == S3O_KIND_SCALE_TRANS)) {
-        if (!amg && p->h_sc->iters > 256) p->auto_multilevel = true;
-        else if (amg && p->auto_multilevel && p->h_sc->iters <= 8) p->auto_multilevel = false;
-    }
-    if (status) *status = p->h_sc->done ? p->h_sc->done : 2;
-    if (iters) *iters = p->h_sc->iters;
-    if (rel_res) *rel_res = p->h_sc->rr0 > 0 ? std::sqrt(p->h_sc->rr / p->h_sc->rr0) : 0.0;
     return S3O_OK;
 }
 }  // namespace s3o
@@ -1655,17 +1672,24 @@ int s3o_compute_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, cons
                 return S3O_ERR_SOLVE;
             }
     }
+    // the selected inverse of the sparse Cholesky factor, or PCG solves of the requested block columns where that
+    // factor exceeds the forced cap (marginals_pcg.cu)
+    bool iterative = false;
+    if ((rc = marginals_iterative(p, &iterative))) return rc;
     cudaEventRecord(p->ev[0], p->stream);
     if ((rc = do_linearize(p))) return rc;
     cudaEventRecord(p->ev[1], p->stream);
-    rc = direct_marginals(p, n_pairs, rows, cols, out, p->ev + 2);
+    rc = iterative ? pcg_marginals(p, n_pairs, rows, cols, out, p->ev + 2) : direct_marginals(p, n_pairs, rows, cols, out, p->ev + 2);
     direct_invalidate(p);
     p->linearized = false;          // as after s3o_optimize: the next solve linearises again
     if (rc) return rc;
     if (getenv("S3O_MARGINALS_TRACE")) {     // per-phase CUDA-event times (tools/marginals_probe.py)
         float ms[4] = {};
         for (int k = 0; k < 4; ++k) cudaEventElapsedTime(&ms[k], p->ev[k], p->ev[k + 1]);
-        fprintf(stderr, "s3o_compute_marginals: linearize %.4f factor %.4f selinv %.4f gather %.4f ms\n", ms[0], ms[1], ms[2], ms[3]);
+        if (iterative)
+            fprintf(stderr, "s3o_compute_marginals: linearize %.4f precond %.4f solves %.4f symmetrize %.4f ms\n", ms[0], ms[1], ms[2], ms[3]);
+        else
+            fprintf(stderr, "s3o_compute_marginals: linearize %.4f factor %.4f selinv %.4f gather %.4f ms\n", ms[0], ms[1], ms[2], ms[3]);
     }
     return S3O_OK;
 }

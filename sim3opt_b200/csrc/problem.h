@@ -157,6 +157,12 @@ int alloc_linear_system(s3o_problem *p);                      // H, b, x, r, z, 
 // factor is small (s3o_set_linear_solver), PCG otherwise.  defer_sync: the exact path does not wait for the
 // device; *status stays 0 and the caller reads DevScalars::done after its own sync_scalars.
 int do_solve(s3o_problem *p, double lambda, int *status, int *iters, double *rel_res, bool defer_sync = false);
+// The PCG of do_solve in two steps, shared with the iterative marginals: pcg_prepare forms the block-Jacobi inverses
+// of (H + lambda I) and, when amg, the multilevel operators; pcg_iterate solves (H + lambda I) x = p->d_b from x = 0
+// into p->d_x, to the relative recurrence residual tol or max_iter iterations, and leaves its verdict in p->h_sc.
+int pcg_prepare(s3o_problem *p, double lambda, bool amg);
+int pcg_iterate(s3o_problem *p, double lambda, bool amg, double tol, int max_iter);
+void hessian_product(s3o_problem *p, const double *x);   // q1 and T of H x (lambda = 0; completed by the column owner)
 
 // ---- sparse block Cholesky (direct.cu, direct_host.cpp) ---------------------------------------
 int direct_setup(s3o_problem *p);                     // symbolic analysis + upload, once per structure
@@ -188,6 +194,14 @@ struct MarginalsRun {
 int marginals_open(s3o_problem *p, const char *who, int n_pairs, const int32_t *rows, const int32_t *cols, MarginalsRun *run);
 int marginals_factor(s3o_problem *p, const MarginalsRun &run, cudaEvent_t *ev);
 int marginals_pick(s3o_problem *p, const MarginalsRun &run, int n_pairs);
+// Which route serves a pose-graph marginals call: the iterative one (*iterative) when the factor exceeds the forced
+// cap, or when S3O_MARGINALS_ROUTE=pcg asks for it.
+int marginals_iterative(s3o_problem *p, bool *iterative);
+// Iterative route (marginals_pcg.cu): for each distinct column vertex c of the explicit pairs, d PCG solves
+// H x = e_(c,m) without damping, refined until the true residual |e - H x| <= S3O_MARGINALS_PCG_TOL.  Reuses the LM's
+// PCG work vectors and scalars; puts back what the LM carries across calls and the solver statistics.  ev (may be
+// nullptr): 3 events recorded after the preconditioner set-up, the solves and the gather.
+int pcg_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev);
 // Launches a persistent kernel whose CTAs synchronise through grid_barrier (gridbar.cuh).  The kernel's LAST argument
 // is a GridBarrier; args[nargs - 1] must point to a GridBarrier that this call fills.
 inline int launch_persistent(s3o_problem *p, const void *func, int grid, int block, void **args, int nargs, size_t smem = 0) {
@@ -220,7 +234,8 @@ void amg_counts(const s3o_problem *p, int64_t *rebuilds, int64_t *reuses);
 void amg_invalidate_frames(s3o_problem *p);           // the linearisation point moved
 int amg_update_frames(s3o_problem *p);
 int amg_update_values(s3o_problem *p, double lambda); // Galerkin operators for (H + lambda I)
-int amg_apply(s3o_problem *p, int init);              // z += P0 V(P0^T r), r.z and the PCG scalars
+int amg_apply(s3o_problem *p, int init, double tol, int max_iter);   // z += P0 V(P0^T r), r.z and the PCG scalars
+void amg_set_counts(s3o_problem *p, int64_t rebuilds, int64_t reuses);
 
 // ---- bundle adjustment hooks (ba.cu), called from the C ABI in problem.cu --------------------
 void ba_destroy(s3o_problem *p);

@@ -10,7 +10,13 @@ One JSON line per graph.
 two cameras fixed, Huber 2.5), split into linearise, Schur complement, factorisation, selected inverse, point phase and
 gather.  Also prints sum_l |O(l)|^2, the 6x6-by-6x3 products of the point phase.
 
-    python tools/marginals_probe.py [--ba] [--reps 50] [--warmup 5]
+--pcg: the iterative route on the graphs beyond the sparse Cholesky's cap, s100k (synth.sphere(100, 1000)) and S1M
+(synth.sphere(1000, 1000)).  The first call (one column vertex) includes the forced-cap plan analysis that finds the
+factor too large; then one call each with 1, 2 and 8 column vertices (the diagonal block and one far row per column).
+Per call: host time and CUDA-event time of the solves per column vertex, PCG iterations per right-hand side,
+refinement rounds and the largest true residual.
+
+    python tools/marginals_probe.py [--ba | --pcg] [--reps 50] [--warmup 5]
 """
 import argparse
 import json
@@ -89,11 +95,48 @@ def ba_main(a, gpu_info):
         print(json.dumps(rec), flush=True)
 
 
+def pcg_main(gpu_info):
+    import re
+    from conftest import make_gpu
+    from sim3opt_b200 import synth
+    col_re = re.compile(r"column (\d+) \(vertex \d+\): PCG iterations ([\d ]+), refinement rounds (\d+), true residual ([^,\s]+), backward error (\S+)")
+    for name, laps in (("s100k", 100), ("S1M", 1000)):
+        g = synth.sphere(laps, 1000, seed=42)
+        p = make_gpu(g, jac=1)
+        p.build_structure()
+        nf = p.num_free
+
+        def call(cols):
+            pairs = np.array([(c, c) for c in cols] + [((c + nf // 2) % nf, c) for c in cols], np.int32)
+            with StderrCapture() as cap:
+                t0 = time.perf_counter()
+                p.marginals(pairs)
+                wall = time.perf_counter() - t0
+            cols_out = [m.groups() for m in col_re.finditer(cap.text)]
+            phase = [line for line in cap.text.splitlines() if line.startswith("s3o_compute_marginals: linearize")][-1]
+            ms = [float(x) for x in phase.split()[2:9:2]]
+            its = [int(x) for c in cols_out for x in c[1].split()]
+            return {"columns": len(cols), "ms_call_wall": 1e3 * wall, "ms_wall_per_column": 1e3 * wall / len(cols),
+                    "ms_linearize": ms[0], "ms_precond": ms[1], "ms_solves_per_column": ms[2] / len(cols),
+                    "pcg_iters_per_rhs_mean": float(np.mean(its)), "pcg_iters_per_rhs_max": int(np.max(its)),
+                    "refinement_rounds_max": max(int(c[2]) for c in cols_out),
+                    "true_residual_max": max(float(c[3]) for c in cols_out),
+                    "backward_error_max": max(float(c[4]) for c in cols_out)}
+
+        rng = np.random.default_rng(1)
+        rec = {"graph": name, "free": nf, "gpu": gpu_info[:1]}
+        rec["first_call"] = call([nf - 1])          # includes the forced-cap plan analysis
+        for k in (1, 2, 8):
+            rec[f"cols_{k}"] = call(sorted(rng.choice(nf, k, replace=False).tolist()))
+        print(json.dumps(rec), flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--ba", action="store_true")
+    ap.add_argument("--pcg", action="store_true")
     a = ap.parse_args()
     import sim3opt_b200 as s3
     from conftest import make_gpu, make_oracle
@@ -102,6 +145,8 @@ def main():
                               capture_output=True, text=True).stdout.strip().splitlines()
     if a.ba:
         return ba_main(a, gpu_info)
+    if a.pcg:
+        return pcg_main(gpu_info)
     for name, g in graphs().items():
         plan = s3.host_direct_plan(len(g["est"]), g["fixed"], g["v0"], g["v1"], max_pairs=60000000)
         p = make_gpu(g, jac=1)
