@@ -191,6 +191,32 @@ int s3o_hessian_multiply(s3o_problem *p, double lambda, const double *x, double 
  * all-gathered inside, so the call is collective and leaves identical estimates on every rank. */
 int s3o_update(s3o_problem *p, const double *x);
 
+/* Read-outs of the multilevel preconditioner, for tests that check it piece by piece against a host reference.
+ * Pose-graph kinds on one GPU only (S3O_ERR_UNSUPPORTED for BA and the partitioned solve); S3O_ERR_INVALID before
+ * s3o_linearize.  They change no estimate, neither H nor b; they do count in the multilevel rebuild / reuse statistics.
+ * s3o_multilevel_prepare runs the set-up s3o_solve runs for (H + lambda I) -- the hierarchy, the Galerkin operators,
+ * the smoother inverses and the coarsest inverse -- and describes the cycle the PCG will take.  info (cap >= 9 + 3 *
+ * levels; 9 + 3 * 12 always suffices): [0] coarse levels (0: block-Jacobi only), [1] K-cycle depth, [2] mask of the
+ * K-cycle levels, [3] first level of the cooperative kernel, [4] first level of the V-cycle's tail kernel, [5] dense
+ * coarsest inverse, [6] inverted by the cooperative kernel, [7] SMs the cooperative kernels may use, [8] grid of the
+ * cooperative cycle kernel (0: V-cycle), then per level l: [9+3l] vertices, [10+3l] blocks, [11+3l] 8-lane groups per
+ * block row in the cooperative kernel (0: not in it).  Coarse level l (from 0) holds its operator and the transfer to
+ * it from the next finer level (l = 0: from the free vertices). */
+int s3o_multilevel_prepare(s3o_problem *p, double lambda, int32_t *info, int cap);
+/* Level l as the last s3o_multilevel_prepare left it; every array may be NULL.  agg: n_fine aggregate of every vertex
+ * of the finer level; root_vid: n vertex id of every aggregate's root; rowptr (n+1) / colidx (blocks): full BSR
+ * pattern, columns ascending; A: blocks x d x d row-major; Dinv: n x d x d inverses of the diagonal blocks; rel:
+ * n_fine x 13 frames of the transfer, S_i S_root^-1 as [R row-major, t, s] (scale-trans, scale: R_i R_root^T and
+ * s_i / s_root, t = 0). */
+int s3o_get_multilevel_level(s3o_problem *p, int level, int32_t *agg, int32_t *root_vid, int32_t *rowptr,
+                             int32_t *colidx, double *A, double *Dinv, double *rel);
+/* inv: (n d) x (n d) row-major dense inverse of the coarsest operator (S3O_ERR_INVALID when it has none) */
+int s3o_get_multilevel_coarsest_inverse(s3o_problem *p, double *inv);
+/* z = M^-1 r (n_free * d each) through the kernels of one PCG iteration, after the set-up for (H + lambda I):
+ * D^-1 r + P0 x1 with the multilevel preconditioner, D^-1 r with block-Jacobi or without coarse levels.  Overwrites
+ * the PCG work vectors. */
+int s3o_apply_preconditioner(s3o_problem *p, double lambda, const double *r, double *z);
+
 /* Eigenvector of the smallest eigenvalue of H = J^T Omega J at the current estimates, by inverse
  * iteration with the PCG solver (replaces the dense Eigen::JacobiSVD null-vector solve of the
  * stepwise scale initialisation, kitti_surf.cpp:887-934: H of the 1-DoF scale graph with no fixed

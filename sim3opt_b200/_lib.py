@@ -72,6 +72,10 @@ SYMBOLS = {
     "s3o_solve": (C.c_int, [C.c_void_p, C.c_double, _dp, C.POINTER(C.c_int), _dp]),
     "s3o_hessian_multiply": (C.c_int, [C.c_void_p, C.c_double, _dp, _dp]),
     "s3o_update": (C.c_int, [C.c_void_p, _dp]),
+    "s3o_multilevel_prepare": (C.c_int, [C.c_void_p, C.c_double, _ip, C.c_int]),
+    "s3o_get_multilevel_level": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _ip, _ip, _dp, _dp, _dp]),
+    "s3o_get_multilevel_coarsest_inverse": (C.c_int, [C.c_void_p, _dp]),
+    "s3o_apply_preconditioner": (C.c_int, [C.c_void_p, C.c_double, _dp, _dp]),
     "s3o_smallest_eigenvector": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, _dp, _dp, C.POINTER(C.c_int)]),
     "s3o_compute_marginals": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _dp]),
     "s3o_optimize": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.POINTER(C.c_int), _dp, _dp, _dp, C.c_int]),

@@ -188,6 +188,46 @@ class Problem:
         x = _f64(x)
         self._check(self.L.s3o_update(self.h, _d(x)))
 
+    # ---- multilevel preconditioner read-outs (for tests) --------------------------
+    def multilevel_prepare(self, lam):
+        """Set-up of the preconditioner for (H + lam I), as s3o_solve runs it; returns the cycle plan (dict).
+        The level read-outs below refer to this call's set-up."""
+        info = np.zeros(9 + 3 * 12, np.int32)
+        self._check(self.L.s3o_multilevel_prepare(self.h, float(lam), info.ctypes.data_as(_ip), len(info)))
+        nl = int(info[0])
+        lv = info[9:9 + 3 * nl].reshape(nl, 3)
+        self._ml = dict(n_levels=nl, kdepth=int(info[1]), kmask=int(info[2]), coop_first=int(info[3]), lt=int(info[4]),
+                        dense=int(info[5]), dense_coop=int(info[6]), coop_grid=int(info[7]), grid=int(info[8]),
+                        n=[int(v) for v in lv[:, 0]], nblk=[int(v) for v in lv[:, 1]], G=[int(v) for v in lv[:, 2]],
+                        n_free=self.stats()["n_free"])
+        return dict(self._ml)
+
+    def multilevel_level(self, level):
+        """Coarse level `level` of the last multilevel_prepare: dict of agg, root_vid, rowptr, colidx, A (blocks, d, d),
+        Dinv (n, d, d) and rel (n_fine, 13)."""
+        m, d = self._ml, self.d
+        n, nb = m["n"][level], m["nblk"][level]
+        nfine = m["n_free"] if level == 0 else m["n"][level - 1]
+        out = dict(agg=np.zeros(nfine, np.int32), root_vid=np.zeros(n, np.int32), rowptr=np.zeros(n + 1, np.int32),
+                   colidx=np.zeros(nb, np.int32), A=np.zeros((nb, d, d)), Dinv=np.zeros((n, d, d)), rel=np.zeros((nfine, 13)))
+        self._check(self.L.s3o_get_multilevel_level(
+            self.h, int(level), *(out[k].ctypes.data_as(_ip) for k in ("agg", "root_vid", "rowptr", "colidx")),
+            *(_d(out[k]) for k in ("A", "Dinv", "rel"))))
+        return out
+
+    def multilevel_coarsest_inverse(self):
+        N = self._ml["n"][-1] * self.d
+        inv = np.zeros((N, N))
+        self._check(self.L.s3o_get_multilevel_coarsest_inverse(self.h, _d(inv)))
+        return inv
+
+    def apply_preconditioner(self, lam, r):
+        """z = M^-1 r through the kernels of one PCG iteration, after the set-up for (H + lam I)."""
+        r = _f64(r).reshape(-1)
+        z = np.zeros_like(r)
+        self._check(self.L.s3o_apply_preconditioner(self.h, float(lam), _d(r), _d(z)))
+        return z
+
     def smallest_eigenvector(self, max_iter=50, tol=1e-12):
         """(x, lambda_min, lambda_max, iterations) of H at the current estimates (stepwise scale init)."""
         self.build_structure()

@@ -30,6 +30,7 @@ constexpr int kCoarsestMaxBig = 128;    // large graphs: the hierarchy stops at 
 constexpr int kBigGraph = 20000;        // free vertices from which the deep-hierarchy settings apply
 constexpr int kMaxLevels = 12;
 constexpr double kOmega = 0.7;          // damping of the block-Jacobi smoother on the coarse levels
+constexpr int kPlanHeader = 9;          // amg_plan_info: entries before the per-level (n, nblk, G) triples
 
 struct LevelDev {       // transfer level l -> l+1 plus operator and vectors of level l+1
     int n_fine = 0, n = 0, nblk = 0, nub = 0, pad_fine = 0;
@@ -1313,6 +1314,24 @@ amg_coop_kernel(const __grid_constant__ CoopParams P, double omega, const DevSca
     }
 }
 
+// V-cycle: first level handled by the cluster tail kernel (a large coarsest level: the tail still runs its sweeps)
+int tail_first(const AmgState *st) {
+    const int nl = (int)st->lev.size();
+    int lt = 0;
+    while (lt < nl && st->lev[lt].n > kTailRows) ++lt;
+    return lt == nl ? nl - 1 : lt;
+}
+// K-cycle: grid of the cooperative kernel entered at level l, and the 8-lane groups that share one block row of an
+// n-row level on that grid (as many as the grid has to spare)
+int coop_grid_at(const AmgState *st, int l) {
+    const int grid = (st->lev[l].n * 8 + kCoopThreads - 1) / kCoopThreads;
+    return std::max(8, std::min(grid, st->coop_grid));
+}
+int coop_row_groups(int grid, int n) {
+    const long long lanes = (long long)grid * kCoopThreads;
+    return (long long)n * 32 <= lanes ? 4 : ((long long)n * 16 <= lanes ? 2 : 1);
+}
+
 template <class T>
 int up(s3o_problem *p, T **dst, const std::vector<T> &src) { return upload(p, dst, src); }
 
@@ -1672,9 +1691,7 @@ int apply_t(s3o_problem *p, int init, double tol, int max_iter) {
     cudaStream_t s = p->stream;
     int launches = 0;
     auto rows = [](int n) { return (n + 15) / 16; };
-    int lt = 0;                 // first level handled by the one-CTA tail kernel
-    while (lt < nl && st->lev[lt].n > kTailRows) ++lt;
-    if (lt == nl) lt = nl - 1;  // a large coarsest level: the tail kernel still runs its smoothing sweeps
+    const int lt = tail_first(st);
     {   // fine residual -> level 1
         LevelDev &L = st->lev[0];
         amg_restrict_kernel<D><<<(L.n + 15) / 16, 128, 0, s>>>(L.n, L.mem_ptr, L.mem_idx, L.rel, L.pad_fine, p->d_r, L.r, sc, chk);
@@ -1744,12 +1761,8 @@ int apply_t(s3o_problem *p, int init, double tol, int max_iter) {
                 int chk_ = chk;
                 GridBarrier gb{};
                 void *args[] = { &P, &omega, (void *)&sc, &chk_, &gb };
-                int grid = (L.n * 8 + kCoopThreads - 1) / kCoopThreads;
-                grid = std::max(8, std::min(grid, st->coop_grid));
-                for (int k = 0; k < P.nlev; ++k) {      // a block row is shared by as many 8-lane groups as the grid has to spare
-                    const long long lanes = (long long)grid * kCoopThreads, n = P.lev[k].n;
-                    P.lev[k].G = n * 32 <= lanes ? 4 : (n * 16 <= lanes ? 2 : 1);
-                }
+                const int grid = coop_grid_at(st, l);
+                for (int k = 0; k < P.nlev; ++k) P.lev[k].G = coop_row_groups(grid, P.lev[k].n);
                 if (launch_persistent(p, (const void *)amg_coop_kernel<D>, grid, kCoopThreads, args, 5)) rc_inner = S3O_ERR_CUDA;
                 ++launches;
                 trace_mark(p, "cooperative kernel");
@@ -1867,5 +1880,78 @@ void amg_set_counts(s3o_problem *p, int64_t rebuilds, int64_t reuses) {
     if (p->amg) { p->amg->rebuilds = rebuilds; p->amg->reuses = reuses; }
 }
 void amg_invalidate_frames(s3o_problem *p) { if (p->amg) { p->amg->frames_valid = false; p->amg->lin_changed = true; } }
+
+// ---- read-outs of the hierarchy for tests (s3o_multilevel_prepare, s3o_get_multilevel_*) ---------------------
+int amg_plan_info(const s3o_problem *p, bool active, int32_t *info, int cap) {
+    const AmgState *st = active ? p->amg : nullptr;
+    const int nl = st ? (int)st->lev.size() : 0;
+    if (cap < kPlanHeader + 3 * nl) { set_error("s3o_multilevel_prepare: info needs %d entries", kPlanHeader + 3 * nl); return S3O_ERR_INVALID; }
+    for (int k = 0; k < cap; ++k) info[k] = 0;
+    if (nl == 0) return S3O_OK;
+    const int grid = st->kdepth > 0 ? coop_grid_at(st, st->coop_first) : 0;
+    info[0] = nl; info[1] = st->kdepth; info[2] = (int32_t)st->kmask; info[3] = st->coop_first; info[4] = tail_first(st);
+    info[5] = st->dense; info[6] = st->dense_coop; info[7] = st->coop_grid; info[8] = grid;
+    for (int l = 0; l < nl; ++l) {
+        info[kPlanHeader + 3 * l] = st->lev[l].n;
+        info[kPlanHeader + 3 * l + 1] = st->lev[l].nblk;
+        info[kPlanHeader + 3 * l + 2] = (grid && l >= st->coop_first) ? coop_row_groups(grid, st->lev[l].n) : 0;
+    }
+    return S3O_OK;
+}
+
+namespace {
+template <class T>
+int download(s3o_problem *p, T *dst, const T *src, size_t count) {
+    if (dst && count) S3O_CUDA(cudaMemcpyAsync(dst, src, count * sizeof(T), cudaMemcpyDeviceToHost, p->stream));
+    return S3O_OK;
+}
+}  // namespace
+
+int amg_read_level(s3o_problem *p, int level, int32_t *agg, int32_t *root_vid, int32_t *rowptr, int32_t *colidx,
+                   double *A, double *Dinv, double *rel) {
+    const AmgState *st = p->amg;
+    if (!st || level < 0 || level >= (int)st->lev.size()) {
+        set_error("s3o_get_multilevel_level: no level %d (%d levels prepared)", level, st ? (int)st->lev.size() : 0);
+        return S3O_ERR_INVALID;
+    }
+    const LevelDev &L = st->lev[level];
+    const int D = p->d, S = D * (D + 1) / 2;
+    std::vector<double> dpk(Dinv ? (size_t)L.n * S : 0), rpl(rel ? (size_t)NREL * L.pad_fine : 0);
+    int rc = download(p, agg, L.agg, (size_t)L.n_fine);
+    rc = rc ? rc : download(p, root_vid, L.vid, (size_t)L.n);
+    rc = rc ? rc : download(p, rowptr, L.rowptr, (size_t)L.n + 1);
+    rc = rc ? rc : download(p, colidx, L.colidx, (size_t)L.nblk);
+    rc = rc ? rc : download(p, A, L.A, (size_t)L.nblk * DD);
+    rc = rc ? rc : download(p, dpk.data(), L.Dinv, dpk.size());
+    rc = rc ? rc : download(p, rpl.data(), L.rel, rpl.size());
+    if (rc) return rc;
+    S3O_CUDA(cudaStreamSynchronize(p->stream));
+    if (Dinv) {         // packed upper triangle (sym_off) -> d x d
+        for (int I = 0; I < L.n; ++I)
+            for (int r = 0; r < D; ++r)
+                for (int c = 0; c < D; ++c) {
+                    const int lo = std::min(r, c), hi = std::max(r, c);
+                    Dinv[((size_t)I * D + r) * D + c] = dpk[(size_t)I * S + lo * D - lo * (lo - 1) / 2 + (hi - lo)];
+                }
+    }
+    if (rel)            // [13][pad_fine] planes -> [n_fine][13]
+        for (int i = 0; i < L.n_fine; ++i)
+            for (int k = 0; k < NREL; ++k) rel[(size_t)i * NREL + k] = rpl[(size_t)k * L.pad_fine + i];
+    return S3O_OK;
+}
+
+int amg_read_coarsest_inverse(s3o_problem *p, double *inv) {
+    const AmgState *st = p->amg;
+    if (!st || st->lev.empty() || !st->dense) {
+        set_error("s3o_get_multilevel_coarsest_inverse: no dense inverse of the coarsest level (%s)",
+                  !st || st->lev.empty() ? "no levels prepared" : "more than 128 vertices: smoothed instead");
+        return S3O_ERR_INVALID;
+    }
+    const size_t N = (size_t)st->lev.back().n * p->d;
+    int rc = download(p, inv, (const double *)st->d_dense, N * N);
+    if (rc) return rc;
+    S3O_CUDA(cudaStreamSynchronize(p->stream));
+    return S3O_OK;
+}
 
 }  // namespace s3o

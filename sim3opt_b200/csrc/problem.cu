@@ -1348,6 +1348,71 @@ int s3o_hessian_multiply(s3o_problem *p, double lambda, const double *x, double 
     return S3O_OK;
 }
 
+namespace {
+int multilevel_hook_check(s3o_problem *p, const char *who) {
+    if (!p) { set_error("%s: no problem", who); return S3O_ERR_INVALID; }
+    if (p->kind == S3O_KIND_BA || p->kind == 100) { set_error("%s: pose-graph problems only", who); return S3O_ERR_UNSUPPORTED; }
+    if (p->dist) { set_error("%s: not available in the partitioned solve", who); return S3O_ERR_UNSUPPORTED; }
+    if (!p->built || !p->linearized) { set_error("%s: call s3o_linearize first", who); return S3O_ERR_INVALID; }
+    cudaSetDevice(p->device);
+    return S3O_OK;
+}
+// the preconditioner set-up of do_solve; *amg: the multilevel correction is on
+int multilevel_hook_prepare(s3o_problem *p, double lambda, bool *amg) {
+    int rc;
+    *amg = false;
+    if (wants_multilevel(p)) {
+        if ((rc = amg_setup(p))) return rc;
+        *amg = amg_levels(p) > 0;
+    }
+    return pcg_prepare(p, lambda, *amg);
+}
+}  // namespace
+
+int s3o_multilevel_prepare(s3o_problem *p, double lambda, int32_t *info, int cap) {
+    int rc = multilevel_hook_check(p, "s3o_multilevel_prepare");
+    bool amg = false;
+    if (rc || (rc = multilevel_hook_prepare(p, lambda, &amg))) return rc;
+    S3O_CUDA(cudaStreamSynchronize(p->stream));
+    return info ? s3o::amg_plan_info(p, amg, info, cap) : S3O_OK;
+}
+
+int s3o_get_multilevel_level(s3o_problem *p, int level, int32_t *agg, int32_t *root_vid, int32_t *rowptr,
+                             int32_t *colidx, double *A, double *Dinv, double *rel) {
+    int rc = multilevel_hook_check(p, "s3o_get_multilevel_level");
+    return rc ? rc : s3o::amg_read_level(p, level, agg, root_vid, rowptr, colidx, A, Dinv, rel);
+}
+
+int s3o_get_multilevel_coarsest_inverse(s3o_problem *p, double *inv) {
+    int rc = multilevel_hook_check(p, "s3o_get_multilevel_coarsest_inverse");
+    if (!rc && !inv) { set_error("s3o_get_multilevel_coarsest_inverse: inv is NULL"); rc = S3O_ERR_INVALID; }
+    return rc ? rc : s3o::amg_read_coarsest_inverse(p, inv);
+}
+
+int s3o_apply_preconditioner(s3o_problem *p, double lambda, const double *r, double *z) {
+    int rc = multilevel_hook_check(p, "s3o_apply_preconditioner");
+    if (!rc && (!r || !z)) { set_error("s3o_apply_preconditioner: r or z is NULL"); rc = S3O_ERR_INVALID; }
+    bool amg = false;
+    if (rc || (rc = multilevel_hook_prepare(p, lambda, &amg))) return rc;
+    const int nf = p->S.nf, d = p->d;
+    const size_t bytes = (size_t)nf * d * sizeof(double);
+    double *d_rhs = nullptr;
+    if ((rc = dev_alloc(&d_rhs, (size_t)nf * d))) return rc;
+    // what one PCG iteration runs: z = D^-1 r (p = z), then with the multilevel correction p = z + P0 V(P0^T r)
+    cudaError_t e = cudaMemcpyAsync(d_rhs, r, bytes, cudaMemcpyHostToDevice, p->stream);
+    if (e == cudaSuccess) {
+        launch_pcg_init(d, nf, d_rhs, p->d_Minv, p->d_x, p->d_r, p->d_z, p->d_p, p->d_partials, p->d_sc, p->pcg_tol,
+                        p->pcg_max_iter, amg ? 1 : 0, p->stream);
+        rc = check_launch(p, 1);
+        if (!rc && amg) rc = amg_apply(p, 1, p->pcg_tol, p->pcg_max_iter);
+        if (!rc) e = cudaMemcpyAsync(z, p->d_p, bytes, cudaMemcpyDeviceToHost, p->stream);
+        if (!rc && e == cudaSuccess) e = cudaStreamSynchronize(p->stream);
+    }
+    dev_free(d_rhs);
+    if (!rc && e != cudaSuccess) { set_error("s3o_apply_preconditioner: %s", cudaGetErrorString(e)); rc = S3O_ERR_CUDA; }
+    return rc;
+}
+
 int s3o_update(s3o_problem *p, const double *x) {
     if (!p || !x) return S3O_ERR_INVALID;
     cudaSetDevice(p->device);

@@ -236,6 +236,11 @@ int amg_update_frames(s3o_problem *p);
 int amg_update_values(s3o_problem *p, double lambda); // Galerkin operators for (H + lambda I)
 int amg_apply(s3o_problem *p, int init, double tol, int max_iter);   // z += P0 V(P0^T r), r.z and the PCG scalars
 void amg_set_counts(s3o_problem *p, int64_t rebuilds, int64_t reuses);
+// read-outs for tests (layouts: include/sim3opt_b200.h, s3o_multilevel_prepare and s3o_get_multilevel_*)
+int amg_plan_info(const s3o_problem *p, bool active, int32_t *info, int cap);
+int amg_read_level(s3o_problem *p, int level, int32_t *agg, int32_t *root_vid, int32_t *rowptr, int32_t *colidx,
+                   double *A, double *Dinv, double *rel);
+int amg_read_coarsest_inverse(s3o_problem *p, double *inv);
 
 // ---- bundle adjustment hooks (ba.cu), called from the C ABI in problem.cu --------------------
 void ba_destroy(s3o_problem *p);
