@@ -217,6 +217,21 @@ int s3o_get_multilevel_coarsest_inverse(s3o_problem *p, double *inv);
  * the PCG work vectors. */
 int s3o_apply_preconditioner(s3o_problem *p, double lambda, const double *r, double *z);
 
+/* Read-outs of the DIRECT linear solver (sparse block Cholesky), for tests that check its schedule and its factor
+ * against a host reference.  They work on a problem (after s3o_build_structure) and on a s3o_linsolver handle (after
+ * its first solve); S3O_ERR_UNSUPPORTED in the partitioned solve.  The plan read is the one the factorisations run on:
+ * the linear solver's own, otherwise the one kept for the marginal covariances (S3O_ERR_UNSUPPORTED when there is
+ * neither).  Its arrays (perm, cptr, brow, src, ...) are those of s3o_host_direct_plan for the same graph.
+ * s3o_direct_schedule runs the symbolic analysis if it has not run yet.  info (cap >= 6 + 2 * rounds): [0] block
+ * columns n, [1] elimination rounds, [2] blocks of L, [3] CTAs of the cooperative launch (<= 1: one CTA), [4] leading
+ * rounds run on the whole grid (the rest runs on CTA 0), [5] SMs the cooperative launch may use, then per round r:
+ * [6+2r] columns, [7+2r] blocks of L. */
+int s3o_direct_schedule(s3o_problem *p, int32_t *info, int cap);
+/* The factor the last numeric factorisation on that plan left (undefined before the first one), in elimination order:
+ * L: blocks x d x d row-major, block t = L(brow[t], column of t) with the pivot blocks lower triangular; Linv: n x d x d,
+ * the inverse of each pivot block as the factorisation computed it.  Either may be NULL. */
+int s3o_get_direct_factor(s3o_problem *p, double *L, double *Linv);
+
 /* Eigenvector of the smallest eigenvalue of H = J^T Omega J at the current estimates, by inverse
  * iteration with the PCG solver (replaces the dense Eigen::JacobiSVD null-vector solve of the
  * stepwise scale initialisation, kitti_surf.cpp:887-934: H of the 1-DoF scale graph with no fixed

@@ -76,6 +76,8 @@ SYMBOLS = {
     "s3o_get_multilevel_level": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _ip, _ip, _dp, _dp, _dp]),
     "s3o_get_multilevel_coarsest_inverse": (C.c_int, [C.c_void_p, _dp]),
     "s3o_apply_preconditioner": (C.c_int, [C.c_void_p, C.c_double, _dp, _dp]),
+    "s3o_direct_schedule": (C.c_int, [C.c_void_p, _ip, C.c_int]),
+    "s3o_get_direct_factor": (C.c_int, [C.c_void_p, _dp, _dp]),
     "s3o_smallest_eigenvector": (C.c_int, [C.c_void_p, C.c_int, C.c_double, _dp, _dp, _dp, C.POINTER(C.c_int)]),
     "s3o_compute_marginals": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _dp]),
     "s3o_optimize": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.POINTER(C.c_int), _dp, _dp, _dp, C.c_int]),

@@ -228,6 +228,16 @@ class Problem:
         self._check(self.L.s3o_apply_preconditioner(self.h, float(lam), _d(r), _d(z)))
         return z
 
+    # ---- DIRECT linear solver read-outs (for tests) --------------------------------
+    def direct_schedule(self):
+        """Schedule of the sparse block Cholesky (s3o_direct_schedule): dict of n, rounds, blocks, grid (CTAs of the
+        cooperative launch, <= 1: one CTA), wide (leading rounds on the grid), sms, and per round cols / blocks."""
+        return _direct_schedule(self.L, self.h, self._check)
+
+    def direct_factor(self):
+        """(L (blocks, d, d), Linv (n, d, d)) the last numeric factorisation left, elimination order."""
+        return _direct_factor(self.L, self.h, self._check, self.d)
+
     def smallest_eigenvector(self, max_iter=50, tol=1e-12):
         """(x, lambda_min, lambda_max, iterations) of H at the current estimates (stepwise scale init)."""
         self.build_structure()
@@ -417,6 +427,35 @@ class LinearSolver:
         if rc not in (0, -6):
             raise S3OError(f"s3o error {rc}: {self.L.s3o_last_error().decode()}")
         return rc, x, method.value, its.value
+
+    def _check(self, rc):
+        if rc != 0:
+            raise S3OError(f"s3o error {rc}: {self.L.s3o_last_error().decode()}")
+
+    def direct_schedule(self):
+        """Problem.direct_schedule for the pattern of the last solve."""
+        return _direct_schedule(self.L, self.h, self._check)
+
+    def direct_factor(self):
+        """Problem.direct_factor: the factor of the last solve's (A + lambda I)."""
+        return _direct_factor(self.L, self.h, self._check, self.d)
+
+
+def _direct_schedule(L, h, check):
+    head = np.zeros(6, np.int32)
+    check(L.s3o_direct_schedule(h, head.ctypes.data_as(_ip), len(head)))
+    info = np.zeros(6 + 2 * int(head[1]), np.int32)
+    check(L.s3o_direct_schedule(h, info.ctypes.data_as(_ip), len(info)))
+    lv = info[6:].reshape(-1, 2)
+    return dict(n=int(info[0]), rounds=int(info[1]), blocks=int(info[2]), grid=int(info[3]), wide=int(info[4]),
+                sms=int(info[5]), cols=[int(v) for v in lv[:, 0]], level_blocks=[int(v) for v in lv[:, 1]])
+
+
+def _direct_factor(L, h, check, d):
+    s = _direct_schedule(L, h, check)
+    Lb, Linv = np.zeros((s["blocks"], d, d)), np.zeros((s["n"], d, d))
+    check(L.s3o_get_direct_factor(h, _d(Lb), _d(Linv)))
+    return Lb, Linv
 
 
 def host_direct_plan(n_vertices, fixed, v0, v1, max_pairs=0):

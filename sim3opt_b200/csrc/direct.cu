@@ -8,9 +8,11 @@
 //     pivot   Cholesky of the level's d x d diagonal blocks, inverse of the triangular factor kept
 //     scale   sub-diagonal blocks of the level's columns times L_kk^-T
 //   forward / backward substitution level by level (8-lane group per block row, shuffles inside the group)
-// Every block has one writer and a fixed summation order: bitwise reproducible.  Small factors (the KITTI-size
-// graphs) run in ONE CTA with __syncthreads between phases -- the whole solve is one launch and no
-// host round trip; larger ones run as a cooperative grid (one CTA per SM) with grid barriers.
+// Every block has one writer and a fixed summation order: bitwise reproducible.  The whole solve is one launch and no
+// host round trip.  A factor whose every round is narrow runs in ONE CTA with __syncthreads between phases; otherwise
+// the leading wide rounds run on a cooperative grid (at most one CTA per SM) with grid barriers and the narrow tail on
+// CTA 0 (see plan_and_upload).  The KITTI-size graphs take the grid: on a 148-SM B200 K1 runs 4 of its 11 rounds on
+// 28 CTAs and K118 11 of its 26 rounds on 21 CTAs (Sim3); the scale graph of K118 (d = 1) stays in one CTA.
 #include <cooperative_groups.h>
 
 #include <algorithm>
@@ -841,6 +843,49 @@ int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int
     S3O_CUDA(cudaStreamSynchronize(p->stream));
     p->stats.d2h_bytes += (int64_t)n_pairs * dd * 8 + 4;
     if (failed) { set_error("s3o_compute_marginals: the Hessian is not positive definite (a pivot of its factorisation failed)"); return S3O_ERR_SOLVE; }
+    return S3O_OK;
+}
+
+// ---- read-outs for tests (s3o_direct_schedule, s3o_get_direct_factor) -------------------------------------------
+// The plan the factorisations of p run on: the linear solver's own, otherwise the one kept for the marginals (the
+// choice marginals_plan makes).
+static DirectState *plan_in_use(s3o_problem *p) {
+    if (!p->direct) return nullptr;
+    if (p->linsolver != S3O_LINSOLVER_PCG && p->direct->available) return p->direct;
+    DirectState *M = p->direct->marg;
+    return M && M->available ? M : nullptr;
+}
+
+int direct_schedule(s3o_problem *p, int32_t *info, int cap) {
+    int rc;
+    if (p->linsolver != S3O_LINSOLVER_PCG && (rc = direct_setup(p))) return rc;
+    const DirectState *S = plan_in_use(p);
+    if (!S) { set_error("s3o_direct_schedule: no factorisation plan (the PCG is in use and no marginals ran, or the factor exceeds the cap)"); return S3O_ERR_UNSUPPORTED; }
+    const DirectPlan &P = S->plan;
+    int sms = 0;
+    switch (p->d) {
+    case 7: sms = coop_capacity<7>(p->device); break;
+    case 6: sms = coop_capacity<6>(p->device); break;
+    case 4: sms = coop_capacity<4>(p->device); break;
+    case 1: sms = coop_capacity<1>(p->device); break;
+    }
+    const int32_t head[6] = { P.n, P.nlev, (int32_t)P.brow.size(), S->coop_grid, S->wide_levels, sms };
+    for (int k = 0; k < 6 && k < cap; ++k) info[k] = head[k];
+    for (int l = 0; l < P.nlev && 7 + 2 * l < cap; ++l) {
+        info[6 + 2 * l] = P.lev_ptr[l + 1] - P.lev_ptr[l];
+        info[7 + 2 * l] = P.cptr[P.lev_ptr[l + 1]] - P.cptr[P.lev_ptr[l]];
+    }
+    return S3O_OK;
+}
+
+int direct_read_factor(s3o_problem *p, double *L, double *Linv) {
+    const DirectState *S = plan_in_use(p);
+    if (!S) { set_error("s3o_get_direct_factor: no factorisation plan"); return S3O_ERR_UNSUPPORTED; }
+    const size_t dd = (size_t)p->d * p->d, nL = S->plan.brow.size(), n = (size_t)S->plan.n;
+    if (L) S3O_CUDA(cudaMemcpyAsync(L, S->d_L, sizeof(double) * nL * dd, cudaMemcpyDeviceToHost, p->stream));
+    if (Linv) S3O_CUDA(cudaMemcpyAsync(Linv, S->d_Linv, sizeof(double) * n * dd, cudaMemcpyDeviceToHost, p->stream));
+    S3O_CUDA(cudaStreamSynchronize(p->stream));
+    p->stats.d2h_bytes += (int64_t)(((L ? nL : 0) + (Linv ? n : 0)) * dd * 8);
     return S3O_OK;
 }
 

@@ -1389,6 +1389,27 @@ int s3o_get_multilevel_coarsest_inverse(s3o_problem *p, double *inv) {
     return rc ? rc : s3o::amg_read_coarsest_inverse(p, inv);
 }
 
+namespace {
+int direct_hook_check(s3o_problem *p, const char *who) {
+    if (!p) { set_error("%s: no problem", who); return S3O_ERR_INVALID; }
+    if (p->dist) { set_error("%s: not available in the partitioned solve", who); return S3O_ERR_UNSUPPORTED; }
+    if (!p->built) { set_error("%s: no structure yet (s3o_build_structure, or a first s3o_linsolver_solve)", who); return S3O_ERR_INVALID; }
+    cudaSetDevice(p->device);
+    return S3O_OK;
+}
+}  // namespace
+
+int s3o_direct_schedule(s3o_problem *p, int32_t *info, int cap) {
+    int rc = direct_hook_check(p, "s3o_direct_schedule");
+    if (!rc && (!info || cap < 6)) { set_error("s3o_direct_schedule: info must hold at least 6 ints"); rc = S3O_ERR_INVALID; }
+    return rc ? rc : s3o::direct_schedule(p, info, cap);
+}
+
+int s3o_get_direct_factor(s3o_problem *p, double *L, double *Linv) {
+    int rc = direct_hook_check(p, "s3o_get_direct_factor");
+    return rc ? rc : s3o::direct_read_factor(p, L, Linv);
+}
+
 int s3o_apply_preconditioner(s3o_problem *p, double lambda, const double *r, double *z) {
     int rc = multilevel_hook_check(p, "s3o_apply_preconditioner");
     if (!rc && (!r || !z)) { set_error("s3o_apply_preconditioner: r or z is NULL"); rc = S3O_ERR_INVALID; }

@@ -170,6 +170,10 @@ bool direct_available(const s3o_problem *p);          // false: the factor would
 int direct_solve(s3o_problem *p, double lambda, bool reuse_factor);
 void direct_invalidate(s3o_problem *p);               // H changed
 void direct_destroy(s3o_problem *p);
+// read-outs for tests (s3o_direct_schedule, s3o_get_direct_factor): the plan the factorisations run on -- the linear
+// solver's, else the marginals' -- and the factor its last numeric factorisation left
+int direct_schedule(s3o_problem *p, int32_t *info, int cap);
+int direct_read_factor(s3o_problem *p, double *L, double *Linv);
 // Marginal covariances: blocks (rows[k], cols[k]) of H^-1 (Hessian indices, validated by the caller) for the H in
 // p->d_H, into out (n_pairs x d x d); rows == cols == nullptr: the n_pairs = n_free diagonal blocks.  Factorises H on
 // the linear solver's plan, or on a plan under the forced cap kept for the marginals (the choice of the linear solver
