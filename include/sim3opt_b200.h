@@ -383,6 +383,25 @@ int s3o_linsolver_destroy(s3o_linsolver *s);
 int s3o_linsolver_solve(s3o_linsolver *s, int n_block_cols, const int32_t *colptr, const int32_t *rowidx,
                         const double *blocks, int column_major, double lambda, const double *b, double *x,
                         int *method /* out, may be NULL: s3o_linear_solver used */, int *pcg_iterations /* may be NULL */);
+/* g2o LinearSolver<M>::solvePattern(spinv, blockIndices, A) / solveBlocks(blocks, A): blocks of A^-1 for the symmetric
+ * positive-definite matrix A given exactly as to s3o_linsolver_solve (upper block-CCS, row- or column-major d x d
+ * blocks), WITHOUT damping.  rows/cols: n_pairs block indices in [0, n_block_cols); out: n_pairs x d x d row-major.
+ * rows == cols == NULL: every diagonal block (solveBlocks; n_pairs must equal n_block_cols).
+ * The semantics are those of s3o_compute_marginals with A in place of the linearised H: A is factorised by the sparse
+ * block Cholesky on the handle's own plan (AUTO, DIRECT) or, when it has none, on a plan under the forced cap (the
+ * handle's choice of linear solver does not move); pairs on the pattern of the factor come from its selected inverse,
+ * pairs off it from d triangular solves per distinct column; diagonal blocks come back exactly symmetric.  Beyond the
+ * forced cap, or with S3O_MARGINALS_ROUTE=pcg, explicit pairs take the PCG route (block-Jacobi preconditioner, refined
+ * to S3O_MARGINALS_PCG_TOL) and the NULL form returns S3O_ERR_UNSUPPORTED.  The pattern cache is the one of
+ * s3o_linsolver_solve: either call may come first, and a call with the last call's pattern keeps the structure, the
+ * plan and the buffers.  There is no graph, hence no gauge check: a singular A shows as a failed pivot.
+ * Returns S3O_ERR_INVALID for a malformed CCS, an index out of range, the NULL form with n_pairs != n_block_cols, or a
+ * handle that is not a s3o_linsolver; S3O_ERR_SOLVE when a pivot fails (A is not positive definite) or a PCG solve
+ * misses its tolerance.  Every later s3o_linsolver_solve on the handle computes what it would have computed without
+ * this call, and the statistics direct_solves and pcg_iterations are unchanged by it. */
+int s3o_linsolver_solve_pattern(s3o_linsolver *s, int n_block_cols, const int32_t *colptr, const int32_t *rowidx,
+                                const double *blocks, int column_major, int n_pairs, const int32_t *rows,
+                                const int32_t *cols, double *out);
 
 /* ---- statistics ------------------------------------------------------------------------ */
 typedef struct s3o_stats {

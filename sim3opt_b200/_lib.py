@@ -103,6 +103,7 @@ SYMBOLS = {
     "s3o_linsolver_create": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "s3o_linsolver_destroy": (C.c_int, [C.c_void_p]),
     "s3o_linsolver_solve": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _dp, C.c_int, C.c_double, _dp, _dp, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "s3o_linsolver_solve_pattern": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _dp, C.c_int, C.c_int, _ip, _ip, _dp]),
     "s3o_get_stats": (C.c_int, [C.c_void_p, C.POINTER(Stats)]),
     "s3o_reset_stats": (C.c_int, [C.c_void_p]),
     "s3o_estimate_sigma_squared": (C.c_int, [C.c_void_p, C.c_int, _dp]),

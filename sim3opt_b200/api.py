@@ -428,6 +428,28 @@ class LinearSolver:
             raise S3OError(f"s3o error {rc}: {self.L.s3o_last_error().decode()}")
         return rc, x, method.value, its.value
 
+    def marginals(self, colptr, rowidx, blocks, pairs=None, column_major=False):
+        """Blocks of A^-1 without damping (g2o LinearSolver::solvePattern / solveBlocks), A given as to solve().
+        pairs=None: the (n, d, d) diagonal blocks; otherwise an (m, 2) array of block-index pairs (row, col) ->
+        (m, d, d).  Same routes as Problem.marginals (selected inverse of the sparse Cholesky factor, PCG beyond its
+        forced cap or with S3O_MARGINALS_ROUTE=pcg); raises S3OError on a negative status."""
+        colptr = np.ascontiguousarray(colptr, np.int32)
+        rowidx = np.ascontiguousarray(rowidx, np.int32)
+        blocks = _f64(blocks)
+        n = len(colptr) - 1
+        if pairs is None:
+            m, rows, cols = n, None, None
+        else:
+            pairs = np.asarray(pairs, np.int32).reshape(-1, 2)
+            rows, cols = np.ascontiguousarray(pairs[:, 0]), np.ascontiguousarray(pairs[:, 1])
+            m = len(pairs)
+        out = np.zeros((m, self.d, self.d))
+        self._check(self.L.s3o_linsolver_solve_pattern(
+            self.h, n, colptr.ctypes.data_as(_ip), rowidx.ctypes.data_as(_ip), _d(blocks), 1 if column_major else 0, m,
+            None if rows is None else rows.ctypes.data_as(_ip), None if cols is None else cols.ctypes.data_as(_ip),
+            _d(out)))
+        return out
+
     def _check(self, rc):
         if rc != 0:
             raise S3OError(f"s3o error {rc}: {self.L.s3o_last_error().decode()}")

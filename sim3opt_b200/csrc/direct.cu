@@ -830,9 +830,10 @@ int marginals_pick(s3o_problem *p, const MarginalsRun &R, int n_pairs) {
 }
 
 // Marginal covariances for the H in p->d_H (see problem.h).
-int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev) {
+int direct_marginals(s3o_problem *p, const char *who, int n_pairs, const int32_t *rows, const int32_t *cols, double *out,
+                     cudaEvent_t *ev) {
     MarginalsRun R;
-    int rc = marginals_open(p, "s3o_compute_marginals", n_pairs, rows, cols, &R);
+    int rc = marginals_open(p, who, n_pairs, rows, cols, &R);
     if (rc) return rc;
     if ((rc = marginals_factor(p, R, ev)) || (rc = marginals_pick(p, R, n_pairs))) return rc;
     if (ev) cudaEventRecord(ev[2], p->stream);
@@ -842,7 +843,7 @@ int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int
     S3O_CUDA(cudaMemcpyAsync(&failed, R.fail, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
     S3O_CUDA(cudaStreamSynchronize(p->stream));
     p->stats.d2h_bytes += (int64_t)n_pairs * dd * 8 + 4;
-    if (failed) { set_error("s3o_compute_marginals: the Hessian is not positive definite (a pivot of its factorisation failed)"); return S3O_ERR_SOLVE; }
+    if (failed) { set_error("%s: the Hessian is not positive definite (a pivot of its factorisation failed)", who); return S3O_ERR_SOLVE; }
     return S3O_OK;
 }
 

@@ -154,8 +154,7 @@ struct DevBuf {     // device allocations of one call
 };
 
 template <int D>
-int run(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev) {
-    const char *who = "s3o_compute_marginals";
+int run(s3o_problem *p, const char *who, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev) {
     if (!rows) {
         set_error("%s: the factor of this graph exceeds the sparse Cholesky's cap of block products, and every diagonal "
                   "block by PCG would take n_free * d = %lld solves; request explicit pairs", who, (long long)p->S.nf * D);
@@ -195,9 +194,10 @@ int run(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, d
     };
     if ((rc = h2d(d_crow, crow)) || (rc = h2d(d_cdst, cdst)) || (rc = h2d(d_diag, diag))) return rc;
 
-    // preconditioner at lambda = 0, once for every solve of the call
+    // preconditioner at lambda = 0, once for every solve of the call (a linear-solver handle has no estimates, hence
+    // no gauge frames to build the multilevel hierarchy on: block-Jacobi there)
     bool amg = false;
-    if (p->kind != S3O_KIND_BA && p->scale_model == S3O_SCALE_MODEL_DIFFERENCE) {
+    if (p->kind != S3O_KIND_BA && p->kind != kKindLinear && p->scale_model == S3O_SCALE_MODEL_DIFFERENCE) {
         if ((rc = amg_setup(p))) return rc;
         amg = amg_levels(p) > 0;
     }
@@ -216,6 +216,7 @@ int run(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, d
     if (ev) cudaEventRecord(ev[0], p->stream);
 
     const bool trace = getenv("S3O_MARGINALS_TRACE") != nullptr;
+    if (trace) fprintf(stderr, "%s: preconditioner %s\n", who, amg ? "multilevel" : "block-Jacobi");
     const StructDev s = struct_view(p);
     const int vgrid = grid_for(nd), rgrid = grid_for(nd);
     const double tol = S3O_MARGINALS_PCG_TOL;
@@ -271,7 +272,7 @@ int run(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, d
             worst_back = std::max(worst_back, back);
         }
         if (trace) {
-            fprintf(stderr, "s3o_compute_marginals: column %d (vertex %d): PCG iterations", c, p->S.free2v[c]);
+            fprintf(stderr, "%s: column %d (vertex %d): PCG iterations", who, c, p->S.free2v[c]);
             for (int m = 0; m < D; ++m) fprintf(stderr, " %d", its[m]);
             fprintf(stderr, ", refinement rounds %d, true residual %.3e, backward error %.3e\n", rounds_max, worst, worst_back);
         }
@@ -291,13 +292,15 @@ int run(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, d
 
 }  // namespace
 
-int pcg_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev) {
+int pcg_marginals(s3o_problem *p, const char *who, int n_pairs, const int32_t *rows, const int32_t *cols, double *out,
+                  cudaEvent_t *ev) {
     switch (p->d) {
-    case 7: return run<7>(p, n_pairs, rows, cols, out, ev);
-    case 4: return run<4>(p, n_pairs, rows, cols, out, ev);
-    case 1: return run<1>(p, n_pairs, rows, cols, out, ev);
+    case 7: return run<7>(p, who, n_pairs, rows, cols, out, ev);
+    case 6: return run<6>(p, who, n_pairs, rows, cols, out, ev);     // a linear-solver handle of 6x6 blocks
+    case 4: return run<4>(p, who, n_pairs, rows, cols, out, ev);
+    case 1: return run<1>(p, who, n_pairs, rows, cols, out, ev);
     }
-    set_error("s3o_compute_marginals: block dimension %d", p->d);
+    set_error("%s: block dimension %d", who, p->d);
     return S3O_ERR_UNSUPPORTED;
 }
 

@@ -511,9 +511,6 @@ int s3o_device_count(void) {
     return n;
 }
 
-// kind of the handle behind s3o_linsolver_*: a block system only (no graph, no estimates)
-static constexpr int kKindLinear = 100;
-
 static int create_impl(int kind, int linear_dim, int device, s3o_problem **out) {
     if (!out) { set_error("s3o_create: out is NULL"); return S3O_ERR_INVALID; }
     *out = nullptr;
@@ -586,11 +583,14 @@ int s3o_linsolver_create(int device, int block_dim, s3o_linsolver **out) {
 
 int s3o_linsolver_destroy(s3o_linsolver *p) { return s3o_destroy(p); }
 
-int s3o_linsolver_solve(s3o_linsolver *p, int n, const int32_t *colptr, const int32_t *rowidx, const double *blocks,
-                        int column_major, double lambda, const double *b, double *x, int *method, int *pcg_iterations) {
-    if (!p || p->kind != kKindLinear || n < 0 || !colptr || (n > 0 && (!rowidx || !blocks || !b || !x))) { set_error("s3o_linsolver_solve: bad arguments"); return S3O_ERR_INVALID; }
-    if (n == 0) return S3O_OK;
-    cudaSetDevice(p->device);
+// A of a linear-solver call (n > 0 block columns, upper block-CCS) onto the handle: validates the CCS, keeps the
+// structure, the factorisation plan and the buffers when the pattern is the last call's and rebuilds them otherwise,
+// reorders the blocks into BSR-upper order (row-major d x d) and uploads them to p->d_H.  Errors are reported as
+// "<who>: ...".  ms_host (may be nullptr): host time of the checks and the reordering; ev_copy (may be nullptr):
+// recorded before the copy.
+static int linsolver_upload(s3o_problem *p, const char *who, int n, const int32_t *colptr, const int32_t *rowidx,
+                            const double *blocks, int column_major, double *ms_host, cudaEvent_t ev_copy) {
+    const auto t0 = std::chrono::steady_clock::now();
     const int d = p->d, dd = d * d, nb = colptr[n];
     // same pattern as the last call (LinearSolver::init() once, solve() per LM trial): keep structure and plan
     bool same = p->built && p->S.nf == n && p->S.nb == nb &&
@@ -604,18 +604,18 @@ int s3o_linsolver_solve(s3o_linsolver *p, int n, const int32_t *colptr, const in
             for (int k = colptr[c]; k < colptr[c + 1]; ++k) {
                 const int r = rowidx[k];
                 if (r < 0 || r > c || (k > colptr[c] && r <= rowidx[k - 1])) {
-                    set_error("s3o_linsolver_solve: column %d is not an upper block-CCS column (rows ascending, row <= column)", c);
+                    set_error("%s: column %d is not an upper block-CCS column (rows ascending, row <= column)", who, c);
                     return S3O_ERR_INVALID;
                 }
                 if (r == c) diag = true;
                 else { v0.push_back(r); v1.push_back(c); }
             }
-            if (!diag) { set_error("s3o_linsolver_solve: column %d has no diagonal block", c); return S3O_ERR_INVALID; }
+            if (!diag) { set_error("%s: column %d has no diagonal block", who, c); return S3O_ERR_INVALID; }
         }
         p->nv = n;
         p->fixed.assign(n, 0);
         build_structure_host(n, nullptr, (int)v0.size(), v0.data(), v1.data(), p->S);
-        if (p->S.nb != nb || memcmp(p->S.ccs_rowidx.data(), rowidx, sizeof(int32_t) * nb) != 0) { set_error("s3o_linsolver_solve: pattern mismatch"); return S3O_ERR_INVALID; }
+        if (p->S.nb != nb || memcmp(p->S.ccs_rowidx.data(), rowidx, sizeof(int32_t) * nb) != 0) { set_error("%s: pattern mismatch", who); return S3O_ERR_INVALID; }
         int rc = upload_structure_arrays(p, n);
         rc = rc ? rc : alloc_linear_system(p);
         if (rc) { free_structure(p); return rc; }
@@ -632,13 +632,27 @@ int s3o_linsolver_solve(s3o_linsolver *p, int n, const int32_t *colptr, const in
             for (int r = 0; r < d; ++r)
                 for (int cc = 0; cc < d; ++cc) dst[r * d + cc] = src[cc * d + r];
     }
+    if (ms_host) *ms_host = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (ev_copy) cudaEventRecord(ev_copy, p->stream);
     S3O_CUDA(cudaMemcpyAsync(p->d_H, H.data(), H.size() * sizeof(double), cudaMemcpyHostToDevice, p->stream));
-    S3O_CUDA(cudaMemcpyAsync(p->d_b, b, (size_t)n * d * sizeof(double), cudaMemcpyHostToDevice, p->stream));
-    p->stats.h2d_bytes += (int64_t)((H.size() + (size_t)n * d) * sizeof(double));
-    p->linearized = true;
+    p->stats.h2d_bytes += (int64_t)(H.size() * sizeof(double));
     direct_invalidate(p);
+    return S3O_OK;
+}
+
+int s3o_linsolver_solve(s3o_linsolver *p, int n, const int32_t *colptr, const int32_t *rowidx, const double *blocks,
+                        int column_major, double lambda, const double *b, double *x, int *method, int *pcg_iterations) {
+    if (!p || p->kind != kKindLinear || n < 0 || !colptr || (n > 0 && (!rowidx || !blocks || !b || !x))) { set_error("s3o_linsolver_solve: bad arguments"); return S3O_ERR_INVALID; }
+    if (n == 0) return S3O_OK;
+    cudaSetDevice(p->device);
+    int rc = linsolver_upload(p, "s3o_linsolver_solve", n, colptr, rowidx, blocks, column_major, nullptr, nullptr);
+    if (rc) return rc;
+    const int d = p->d;
+    S3O_CUDA(cudaMemcpyAsync(p->d_b, b, (size_t)n * d * sizeof(double), cudaMemcpyHostToDevice, p->stream));
+    p->stats.h2d_bytes += (int64_t)((size_t)n * d * sizeof(double));
+    p->linearized = true;
     int status = 0, iters = 0;
-    int rc = do_solve(p, lambda, &status, &iters, nullptr);
+    rc = do_solve(p, lambda, &status, &iters, nullptr);
     if (rc) return rc;
     S3O_CUDA(cudaMemcpyAsync(x, p->d_x, (size_t)n * d * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
     S3O_CUDA(cudaStreamSynchronize(p->stream));
@@ -647,6 +661,51 @@ int s3o_linsolver_solve(s3o_linsolver *p, int n, const int32_t *colptr, const in
     if (pcg_iterations) *pcg_iterations = iters;
     if (status == 3) { set_error("s3o_linsolver_solve: the matrix is not positive definite (pivot / PCG breakdown)"); return S3O_ERR_SOLVE; }
     if (status == 2) { set_error("s3o_linsolver_solve: PCG hit the iteration cap"); return S3O_ERR_SOLVE; }
+    return S3O_OK;
+}
+
+// g2o LinearSolver<M>::solvePattern / solveBlocks: blocks of A^-1 by s3o_compute_marginals' machinery, with the
+// caller's A in place of the linearised H.  A later s3o_linsolver_solve uploads its own A and b and factorises again.
+int s3o_linsolver_solve_pattern(s3o_linsolver *p, int n, const int32_t *colptr, const int32_t *rowidx,
+                                const double *blocks, int column_major, int n_pairs, const int32_t *rows,
+                                const int32_t *cols, double *out) {
+    const char *who = "s3o_linsolver_solve_pattern";
+    if (!p || p->kind != kKindLinear || n < 0 || !colptr || (n > 0 && (!rowidx || !blocks)) || n_pairs < 0 ||
+        (!rows != !cols) || (n_pairs > 0 && !out)) {
+        set_error("%s: bad arguments (a s3o_linsolver handle, an upper block-CCS A, pairs or NULL)", who);
+        return S3O_ERR_INVALID;
+    }
+    if (!rows && n_pairs != n) { set_error("%s: the diagonal blocks need n_pairs = n_block_cols = %d", who, n); return S3O_ERR_INVALID; }
+    for (int k = 0; rows && k < n_pairs; ++k)
+        if (rows[k] < 0 || rows[k] >= n || cols[k] < 0 || cols[k] >= n) {
+            set_error("%s: pair %d (%d, %d) is not a pair of block indices in [0, %d)", who, k, rows[k], cols[k], n);
+            return S3O_ERR_INVALID;
+        }
+    if (n == 0) return S3O_OK;
+    cudaSetDevice(p->device);
+    double ms_host = 0;
+    int rc = linsolver_upload(p, who, n, colptr, rowidx, blocks, column_major, &ms_host, p->ev[0]);
+    if (rc) return rc;
+    cudaEventRecord(p->ev[1], p->stream);
+    // the selected inverse of the sparse Cholesky factor, or PCG solves of the requested block columns where that
+    // factor exceeds the forced cap (marginals_pcg.cu)
+    bool iterative = false;
+    if ((rc = marginals_iterative(p, &iterative))) return rc;
+    rc = iterative ? pcg_marginals(p, who, n_pairs, rows, cols, out, p->ev + 2)
+                   : direct_marginals(p, who, n_pairs, rows, cols, out, p->ev + 2);
+    direct_invalidate(p);
+    p->linearized = false;
+    if (rc) return rc;
+    if (getenv("S3O_MARGINALS_TRACE")) {     // host reordering, then CUDA-event times (tools/marginals_probe.py --linsolver)
+        float ms[4] = {};
+        for (int k = 0; k < 4; ++k) cudaEventElapsedTime(&ms[k], p->ev[k], p->ev[k + 1]);
+        if (iterative)
+            fprintf(stderr, "%s: reorder %.4f upload %.4f precond %.4f solves %.4f symmetrize %.4f ms\n", who, ms_host,
+                    ms[0], ms[1], ms[2], ms[3]);
+        else
+            fprintf(stderr, "%s: reorder %.4f upload %.4f factor %.4f selinv %.4f gather %.4f ms\n", who, ms_host, ms[0],
+                    ms[1], ms[2], ms[3]);
+    }
     return S3O_OK;
 }
 
@@ -1765,7 +1824,8 @@ int s3o_compute_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, cons
     cudaEventRecord(p->ev[0], p->stream);
     if ((rc = do_linearize(p))) return rc;
     cudaEventRecord(p->ev[1], p->stream);
-    rc = iterative ? pcg_marginals(p, n_pairs, rows, cols, out, p->ev + 2) : direct_marginals(p, n_pairs, rows, cols, out, p->ev + 2);
+    rc = iterative ? pcg_marginals(p, "s3o_compute_marginals", n_pairs, rows, cols, out, p->ev + 2)
+                   : direct_marginals(p, "s3o_compute_marginals", n_pairs, rows, cols, out, p->ev + 2);
     direct_invalidate(p);
     p->linearized = false;          // as after s3o_optimize: the next solve linearises again
     if (rc) return rc;

@@ -30,6 +30,9 @@ struct AmgState;  // multilevel preconditioner (amg.cu)
 struct DirectState;  // sparse block Cholesky (direct.cu)
 struct DirectPlan;   // its symbolic analysis (direct.h)
 
+// kind of the handle behind s3o_linsolver_*: a block system only (no graph, no estimates)
+constexpr int kKindLinear = 100;
+
 }  // namespace s3o
 
 using s3o::Comm;
@@ -178,8 +181,10 @@ int direct_read_factor(s3o_problem *p, double *L, double *Linv);
 // p->d_H, into out (n_pairs x d x d); rows == cols == nullptr: the n_pairs = n_free diagonal blocks.  Factorises H on
 // the linear solver's plan, or on a plan under the forced cap kept for the marginals (the choice of the linear solver
 // does not change), then runs the selected inverse.  Leaves p->d_b / p->d_x / p->d_sc untouched and no factor held.
-// ev (may be nullptr): 3 events recorded after the factorisation, the selected inverse and the gather.
-int direct_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev);
+// ev (may be nullptr): 3 events recorded after the factorisation, the selected inverse and the gather.  Errors are
+// reported as "<who>: ..." (the C-ABI entry that called it).
+int direct_marginals(s3o_problem *p, const char *who, int n_pairs, const int32_t *rows, const int32_t *cols, double *out,
+                     cudaEvent_t *ev);
 // The same call in steps, so that the BA marginals (ba.cu) can run their point phase on the selected inverse:
 //   marginals_open    plan choice, first-call buffers and gather lists, the requested pairs' lists (host + upload);
 //                     errors are reported as "<who>: ..."
@@ -204,8 +209,11 @@ int marginals_iterative(s3o_problem *p, bool *iterative);
 // Iterative route (marginals_pcg.cu): for each distinct column vertex c of the explicit pairs, d PCG solves
 // H x = e_(c,m) without damping, refined until the true residual |e - H x| <= S3O_MARGINALS_PCG_TOL.  Reuses the LM's
 // PCG work vectors and scalars; puts back what the LM carries across calls and the solver statistics.  ev (may be
-// nullptr): 3 events recorded after the preconditioner set-up, the solves and the gather.
-int pcg_marginals(s3o_problem *p, int n_pairs, const int32_t *rows, const int32_t *cols, double *out, cudaEvent_t *ev);
+// nullptr): 3 events recorded after the preconditioner set-up, the solves and the gather.  Preconditioner: multilevel
+// for the pose-graph kinds under the difference scale model, block-Jacobi otherwise (a linear-solver handle has no
+// estimates to build a hierarchy on).  Errors are reported as "<who>: ...".
+int pcg_marginals(s3o_problem *p, const char *who, int n_pairs, const int32_t *rows, const int32_t *cols, double *out,
+                  cudaEvent_t *ev);
 // Launches a persistent kernel whose CTAs synchronise through grid_barrier (gridbar.cuh).  The kernel's LAST argument
 // is a GridBarrier; args[nargs - 1] must point to a GridBarrier that this call fills.
 inline int launch_persistent(s3o_problem *p, const void *func, int grid, int block, void **args, int nargs, size_t smem = 0) {

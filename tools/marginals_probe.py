@@ -16,7 +16,12 @@ factor too large; then one call each with 1, 2 and 8 column vertices (the diagon
 Per call: host time and CUDA-event time of the solves per column vertex, PCG iterations per right-hand side,
 refinement rounds and the largest true residual.
 
-    python tools/marginals_probe.py [--ba | --pcg] [--reps 50] [--warmup 5]
+--linsolver: s3o_linsolver_solve_pattern (every diagonal block) on a s3o_linsolver handle for the same four graphs, fed
+the H that a problem linearised at the graph's estimates (s3o_get_hessian, g2o block-CCS order), split into the host
+checks and reordering of A, its host-to-device copy, factorisation, selected inverse and gather; beside it the same
+graph's s3o_compute_marginals phases, taken in the same process.
+
+    python tools/marginals_probe.py [--ba | --pcg | --linsolver] [--reps 50] [--warmup 5]
 """
 import argparse
 import json
@@ -131,12 +136,46 @@ def pcg_main(gpu_info):
         print(json.dumps(rec), flush=True)
 
 
+def linsolver_main(a, gpu_info):
+    import sim3opt_b200 as s3
+    from conftest import make_gpu
+    names = ["reorder", "upload", "factor", "selinv", "gather"]
+    for name, g in graphs().items():
+        p = make_gpu(g, jac=1)
+        H, _ = p.linearize()
+        colptr, rowidx = p.build_structure()
+        ls = s3.LinearSolver(p.d)
+        rec = {"graph": name, "free": len(colptr) - 1, "blocks_A": len(rowidx), "bytes_A": H.nbytes}
+        for who, call in (("s3o_linsolver_solve_pattern:", lambda: ls.marginals(colptr, rowidx, H)),
+                          ("s3o_compute_marginals:", p.marginals)):
+            for _ in range(a.warmup):
+                call()
+            wall = []
+            with StderrCapture() as cap:
+                for _ in range(a.reps):
+                    t0 = time.perf_counter()
+                    call()
+                    wall.append(time.perf_counter() - t0)
+            lines = [line.split() for line in cap.text.splitlines() if line.startswith(who)]
+            assert len(lines) == a.reps, cap.text[-2000:]
+            med = np.median(np.array([[float(x) for x in w[2:-1:2]] for w in lines]), 0)
+            if who.startswith("s3o_linsolver"):
+                rec.update({"ms_" + n: float(v) for n, v in zip(names, med)})
+                rec["ms_call_wall"] = 1e3 * float(np.median(wall))
+            else:       # linearize, factor, selinv, gather of the problem's call
+                rec.update({"problem_ms_" + n: float(v) for n, v in zip(["linearize"] + names[2:], med)})
+                rec["problem_ms_call_wall"] = 1e3 * float(np.median(wall))
+        rec.update(reps=a.reps, gpu=gpu_info[:1])
+        print(json.dumps(rec), flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--ba", action="store_true")
     ap.add_argument("--pcg", action="store_true")
+    ap.add_argument("--linsolver", action="store_true")
     a = ap.parse_args()
     import sim3opt_b200 as s3
     from conftest import make_gpu, make_oracle
@@ -147,6 +186,8 @@ def main():
         return ba_main(a, gpu_info)
     if a.pcg:
         return pcg_main(gpu_info)
+    if a.linsolver:
+        return linsolver_main(a, gpu_info)
     for name, g in graphs().items():
         plan = s3.host_direct_plan(len(g["est"]), g["fixed"], g["v0"], g["v1"], max_pairs=60000000)
         p = make_gpu(g, jac=1)
