@@ -11,6 +11,8 @@
 // usage: kitti_pgo direct   <dataDir> <outFile> [--all-loops] [--iters N] [--numeric] [--pcg-tol T] [--precision P]
 //                           [--marginals FILE]
 //        kitti_pgo stepwise <dataDir> <outFile> [--all-loops] [--stages 2|3] [--no-stepwise] [--iters N] [--marginals FILE]
+//        kitti_pgo online   <dataDir> <outFile> [--all-loops] [--step K] [--iters N] [--precision P]
+//                           (key frames replayed one by one; grown with updateInitialization every K)
 //        kitti_pgo dry-run  <dataDir> [--all-loops]        (no GPU: loads, builds, prints structure sizes)
 //        kitti_pgo align    <resultFile> <gtPoseFile> [--only-scale]   (kitti_surf.cpp:1381-1452: Umeyama + RMSE)
 //        kitti_pgo reproject <keyFrameDir> <resultFile> <out.bal>       (drawPTAMPoints.cpp:285-456: map -> BAL)
@@ -33,7 +35,7 @@ namespace {
 struct Options {
     string mode, dataDir, outFile, marginalsFile;
     bool oneConstraint = true, stepwise = true, numeric = false;
-    int stages = 2, iters = 100, precision = 6;
+    int stages = 2, iters = 100, precision = 6, step = 10;
     double pcgTol = 1e-13;
     int pcgMaxIter = 100000;
 };
@@ -186,6 +188,66 @@ int runDirect(const Options &o) {
     });
     profiler.stop("sim3_direct");
     std::cout << "Execution time:\n sim3 direct optimization: " << profiler.ms["sim3_direct"] << " ms (optimize " << profiler.ms["optimize"] << " ms)\n";
+    return 0;
+}
+
+// online: the key frames replayed one by one, as a SLAM back-end receives them.  Step k adds key frame k, its
+// odometry edge (k, k-1) and every loop edge whose two key frames now exist; every --step K key frames the graph is
+// grown on the device (updateInitialization) and optimised with optimize(--iters, true).
+int runOnline(const Options &o) {
+    vector<KeyFrame> kfs;
+    vector<Sim3Constraint> loops;
+    if (!loadProblem(o, kfs, loops)) return 2;
+    g2o::SparseOptimizer optimizer;
+    configure(optimizer, o);
+    const Eigen::Matrix<double, 7, 7> matLambdasim = Eigen::Matrix<double, 7, 7>::Identity();
+    vector<g2o::Sim3> vScw(kfs.size());
+    for (const KeyFrame &kf : kfs) vScw[kf.mnFrameId] = g2o::Sim3(kf.GetRotation(), kf.GetTranslation(), 1.0);
+    g2o::HyperGraph::VertexSet vset;
+    g2o::HyperGraph::EdgeSet eset;
+    auto edge = [&](int id0, int id1, const g2o::Sim3 &m) {
+        vio::EdgeSim3 *e = new vio::EdgeSim3();
+        e->setVertex(1, optimizer.vertex(id1));
+        e->setVertex(0, optimizer.vertex(id0));
+        e->setMeasurement(m);
+        e->information() = matLambdasim;
+        optimizer.addEdge(e);
+        eset.insert(e);
+    };
+    Timer profiler;
+    bool initialised = false;
+    int merges = 0, total_iters = 0;
+    for (size_t k = 0; k < kfs.size(); ++k) {
+        const int id = kfs[k].mnFrameId;
+        vio::VertexSim3Expmap *v = new vio::VertexSim3Expmap();
+        v->setEstimate(vScw[id]);
+        v->setFixed(id == 0);
+        v->setId(id);
+        optimizer.addVertex(v);
+        vset.insert(v);
+        if (k > 0) edge(id, kfs[k - 1].mnFrameId, vScw[kfs[k - 1].mnFrameId] * vScw[id].inverse());
+        for (const Sim3Constraint &c : loops)
+            if (std::max(c.trans_id1, c.trans_id2) == id) edge(c.trans_id1, c.trans_id2, c.mean);
+        if ((k + 1) % o.step != 0 && k + 1 != kfs.size()) continue;
+        profiler.profile("grow");
+        const bool ok = initialised ? optimizer.updateInitialization(vset, eset) : optimizer.initializeOptimization();
+        profiler.stop("grow");
+        if (!ok) { std::cerr << "update / initialize: " << optimizer.lastError() << "\n"; return 3; }
+        initialised = true;
+        vset.clear();
+        eset.clear();
+        profiler.profile("optimize");
+        const int iters = optimizer.optimize(o.iters, true);
+        profiler.stop("optimize");
+        if (iters < 0) { std::cerr << "optimize: " << optimizer.lastError() << "\n"; return 3; }
+        total_iters += iters;
+        ++merges;
+    }
+    report("online", optimizer, total_iters);
+    std::cout << "online: merges " << merges << " grow " << profiler.ms["grow"] << " ms optimize " << profiler.ms["optimize"] << " ms\n";
+    writeResult(o, kfs, "% sim3 optimization result: kf id, sw2i, scaled tiinw, ri2w(qxyzw):", [&](int id) {
+        return static_cast<vio::VertexSim3Expmap *>(optimizer.vertex(id))->estimate();
+    });
     return 0;
 }
 
@@ -351,7 +413,7 @@ int runReproject(const string &keyFrameDir, const string &resultFile, const stri
 int main(int argc, char **argv) {
     Options o;
     if (argc < 3) {
-        std::cerr << "usage: kitti_pgo direct|stepwise|dry-run <dataDir> [<outFile>] [--all-loops] [--stages 2|3] [--no-stepwise]"
+        std::cerr << "usage: kitti_pgo direct|stepwise|online|dry-run <dataDir> [<outFile>] [--all-loops] [--stages 2|3] [--no-stepwise] [--step K]"
                      " [--iters N] [--numeric] [--pcg-tol T] [--precision P] [--marginals FILE]\n";
         return 1;
     }
@@ -378,6 +440,7 @@ int main(int argc, char **argv) {
         else if (a == "--numeric") o.numeric = true;
         else if (a == "--stages" && k + 1 < argc) o.stages = std::atoi(argv[++k]);
         else if (a == "--iters" && k + 1 < argc) o.iters = std::atoi(argv[++k]);
+        else if (a == "--step" && k + 1 < argc) o.step = std::max(1, std::atoi(argv[++k]));
         else if (a == "--precision" && k + 1 < argc) o.precision = std::atoi(argv[++k]);
         else if (a == "--pcg-tol" && k + 1 < argc) o.pcgTol = std::atof(argv[++k]);
         else if (a == "--marginals" && k + 1 < argc) o.marginalsFile = argv[++k];
@@ -395,6 +458,7 @@ int main(int argc, char **argv) {
     }
     if (o.mode == "direct" || o.mode == "dry-run") return runDirect(o);
     if (o.mode == "stepwise") return runStepwise(o);
+    if (o.mode == "online") return runOnline(o);
     std::cerr << "unknown mode " << o.mode << "\n";
     return 1;
 }

@@ -143,6 +143,30 @@ int s3o_set_pcg(s3o_problem *p, double rel_tol, int max_iter);
 int s3o_set_preconditioner(s3o_problem *p, int kind /* s3o_preconditioner */);
 int s3o_set_linear_solver(s3o_problem *p, int kind /* s3o_linear_solver */);
 
+/* ---- growing a built graph (g2o updateInitialization + BlockSolver::updateStructure) ----
+ * s3o_add_vertices appends n vertices with ids nv .. nv+n-1, in the layouts of s3o_set_vertices (aux is required for
+ * SCALE_TRANS, and is given for every vertex or for none).  s3o_add_edges appends n edges, with the layouts and the
+ * checks of s3o_set_edges against the current vertex count; their caller edge ids continue from the current count.
+ * The existing estimates stay on the device (copied there to the new plane pitch); only the appended arrays are
+ * uploaded.  Getters and s3o_set_estimates see the new vertex count at once.
+ *
+ * The next s3o_build_structure -- or any call that needs the structure, as for a first build -- merges the appended
+ * elements on the device.  The problem is then indistinguishable, bit for bit, from a fresh one of the same kind and
+ * settings built from the concatenated vertex and edge arrays, whose estimates are this problem's current estimates
+ * followed by the appended ones: structure, Hessian indices (appended free vertices take n_free, n_free+1, ...),
+ * chi2, edge errors, H and b, solves, s3o_optimize and the marginals.  An appended edge sorts after the existing edges
+ * of the same vertex pair.  As with s3o_set_vertices, the merge drops the LM continuation state, the estimate snapshot
+ * and the AUTO preconditioner's switch; the factorisation plan is analysed again at the next solve, the multilevel
+ * hierarchy is rebuilt.  Cumulative counters of s3o_stats continue.
+ *
+ * Information matrices: a NULL info counts as identity once any edge has one; the merged graph keeps the diagonal
+ * representation only while every matrix is diagonal, as s3o_set_edges would.  Before the first build, appending is
+ * the same as having passed the concatenated arrays to s3o_set_vertices / s3o_set_edges.  n = 0 changes nothing.
+ * S3O_ERR_UNSUPPORTED for bundle adjustment and in the partitioned solve, S3O_ERR_INVALID for bad arguments; a
+ * rejected call leaves the problem as it was.  Removing elements or changing a vertex's fixed flag needs a new build. */
+int s3o_add_vertices(s3o_problem *p, int n, const double *est, const uint8_t *fixed, const double *aux);
+int s3o_add_edges(s3o_problem *p, int n, const int32_t *v0, const int32_t *v1, const double *meas, const double *info);
+
 /* ---- structure (replaces initializeOptimization + BlockSolver::buildStructure) -------- */
 int s3o_build_structure(s3o_problem *p, int *n_free, int *n_blocks);
 /* g2o-order upper block-CCS of Hpp: colptr[n_free+1], rowidx[n_blocks] (rows <= col, ascending) */

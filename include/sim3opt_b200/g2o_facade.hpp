@@ -28,6 +28,7 @@
 #include <cstdio>
 #include <map>
 #include <memory>
+#include <set>
 #include <string>
 #include <utility>
 #include <vector>
@@ -383,6 +384,12 @@ private:
     int max_trials_ = 10, lm_trials_ = 0;
 };
 
+// ---- g2o::HyperGraph's element sets (std::set of pointers, as in g2o) ---------------------------
+struct HyperGraph {
+    typedef std::set<Vertex *> VertexSet;
+    typedef std::set<Edge *> EdgeSet;
+};
+
 // ---- g2o::SparseOptimizer ----------------------------------------------------------------------
 class SparseOptimizer {
 public:
@@ -519,12 +526,87 @@ public:
         if (s3o_get_hessian_index(problem_, hidx.data()) != S3O_OK) return fail(s3o_last_error());
         for (int k = 0; k < n; ++k) order_[k]->hessian_index_ = hidx[k];
         n_free_ = nf; n_blocks_ = nb;
+        n_edges_init_ = edges_.size();
+        initialized_ = true;
+        return true;
+    }
+
+    // SparseOptimizer::updateInitialization [EXT g2o] + BlockSolver::updateStructure: grows the built problem by the
+    // vertices and edges added since the last (re)initialisation, which vset / eset must list exactly (otherwise false,
+    // with lastError()).  The library merges them on the device (s3o_add_vertices / s3o_add_edges): the existing
+    // graph is not uploaded again.  New vertices are appended in id order and new edges in addEdge order; g2o iterates
+    // its pointer-ordered sets instead, so only the summation order inside an H block with several new edges can
+    // differ from g2o's.  A new vertex whose id is below an existing one keeps its place after the existing vertices
+    // (initializeOptimization() numbers by id).  Pose graphs only: bundle adjustment graphs return false, as g2o's
+    // BlockSolver::updateStructure does for marginalised vertices.  Then optimize(n, true).
+    bool updateInitialization(HyperGraph::VertexSet &vset, HyperGraph::EdgeSet &eset) {
+        if (!problem_) return fail("updateInitialization: initializeOptimization() has not succeeded");
+        if (kind_ == S3O_KIND_BA) return fail("updateInitialization: bundle adjustment graphs are rebuilt by initializeOptimization()");
+        std::vector<Vertex *> nv;
+        for (auto &kv : vertices_)
+            if (!dense_.count(kv.first)) nv.push_back(kv.second);      // id order
+        if (nv.size() != vset.size()) return fail("updateInitialization: the vertex set is not the vertices added since the last initialisation");
+        for (Vertex *v : nv)
+            if (!vset.count(v)) return fail("updateInitialization: the vertex set is not the vertices added since the last initialisation");
+        const size_t e0 = n_edges_init_, ne = edges_.size() - e0;
+        if (ne != eset.size()) return fail("updateInitialization: the edge set is not the edges added since the last initialisation");
+        for (size_t k = e0; k < edges_.size(); ++k)
+            if (!eset.count(edges_[k])) return fail("updateInitialization: the edge set is not the edges added since the last initialisation");
+        for (Vertex *v : nv)
+            if (v->s3oKind() != kind_) return fail("updateInitialization: vertex kind does not match the graph");
+        const RobustKernel *rk = nullptr;
+        for (size_t k = 0; k < edges_.size(); ++k) {
+            if (k >= e0 && edges_[k]->s3oKind() != kind_) return fail("updateInitialization: edge kind does not match the graph");
+            if (!robustConsistent(edges_[k], (int)k, rk)) return fail("updateInitialization: the library applies ONE robust kernel to all edges; set the same kernel (kind and delta) on every edge or on none");
+        }
+        // vertices: estimates, fixed flags, aux rotations
+        const int n = (int)nv.size(), n0 = (int)order_.size();
+        std::vector<double> est((size_t)n * est_dim_), aux;
+        std::vector<uint8_t> fixed(n);
+        double q4[4];
+        for (int k = 0; k < n; ++k) {
+            nv[k]->packEstimate(&est[(size_t)k * est_dim_]);
+            fixed[k] = nv[k]->fixed() ? 1 : 0;
+            if (nv[k]->packAux(q4)) {
+                if (aux.empty()) aux.assign((size_t)n * 4, 0.0);
+                for (int c = 0; c < 4; ++c) aux[(size_t)k * 4 + c] = q4[c];
+            }
+        }
+        if (s3o_add_vertices(problem_, n, est.data(), fixed.data(), aux.empty() ? nullptr : aux.data()) != S3O_OK)
+            return fail(s3o_last_error());
+        for (int k = 0; k < n; ++k) { dense_[nv[k]->id()] = n0 + k; order_.push_back(nv[k]); }
+        est_.resize(order_.size() * est_dim_);
+        // edges: endpoints, measurements, information (NULL while all new ones are identity: the library writes identity)
+        std::vector<int32_t> v0(ne), v1(ne);
+        std::vector<double> meas(ne * est_dim_), info;
+        bool identity = true;
+        for (size_t k = 0; k < ne; ++k) identity = identity && edges_[e0 + k]->informationIsIdentity();
+        if (!identity) info.resize(ne * dim_ * dim_);
+        for (size_t k = 0; k < ne; ++k) {
+            Edge *e = edges_[e0 + k];
+            v0[k] = dense_[e->vertex(0)->id()];
+            v1[k] = dense_[e->vertex(1)->id()];
+            e->packMeasurement(&meas[k * est_dim_]);
+            if (!identity) e->packInformation(&info[k * dim_ * dim_]);
+        }
+        if (s3o_add_edges(problem_, (int)ne, v0.data(), v1.data(), meas.data(), identity ? nullptr : info.data()) != S3O_OK)
+            return fail(s3o_last_error());
+        if (rk && s3o_set_robust(problem_, rk->s3oKind(), rk->delta()) != S3O_OK) return fail(s3o_last_error());
+        n_edges_init_ = edges_.size();
+        int nf = 0, nb = 0;
+        if (s3o_build_structure(problem_, &nf, &nb) != S3O_OK) return fail(s3o_last_error());
+        std::vector<int32_t> hidx(order_.size());
+        if (s3o_get_hessian_index(problem_, hidx.data()) != S3O_OK) return fail(s3o_last_error());
+        for (size_t k = 0; k < order_.size(); ++k) order_[k]->hessian_index_ = hidx[k];
+        n_free_ = nf; n_blocks_ = nb;
         initialized_ = true;
         return true;
     }
 
     // SparseOptimizer::optimize [EXT g2o], call site kitti_surf.cpp:675.  Returns the number of
-    // iterations performed, 0 when the first iteration fails, -1 when not initialised.
+    // iterations performed, 0 when the first iteration fails, -1 when not initialised.  online (after
+    // updateInitialization) changes nothing here: as in g2o's Levenberg, the structure is already up to date and the LM
+    // starts from lambda init at its first iteration.
     int optimize(int iterations, bool /*online*/ = false) {
         if (!initialized_ || !problem_) { error_ = "optimize: initializeOptimization() has not succeeded"; return -1; }
         if (iterations <= 0) return 0;
@@ -714,6 +796,7 @@ private:
     std::vector<double> est_, pts_, hist_;
     std::string error_;
     bool verbose_ = false, initialized_ = false;
+    size_t n_edges_init_ = 0;          // edges_ the problem holds (the rest were added since the last (re)initialisation)
     int device_ = 0, kind_ = 0, est_dim_ = 0, dim_ = 0, n_free_ = 0, n_free_points_ = 0, n_blocks_ = 0;
     int jac_mode_ = S3O_JAC_ANALYTIC, math_mode_ = S3O_MATH_REFERENCE, pcg_max_iter_ = 0;
     double jac_h_ = 1e-9, pcg_tol_ = 0, stop_gain_ = 0, chi2_ = 0;

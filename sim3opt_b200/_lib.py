@@ -47,6 +47,8 @@ SYMBOLS = {
     "s3o_host_partition": (C.c_int, [C.c_int, _up, C.c_int, _ip, _ip, C.c_int, C.c_int, _ip, _ip, _ip, _ip, _ip, _ip, _ip, _ip]),
     "s3o_set_vertices": (C.c_int, [C.c_void_p, C.c_int, _dp, _up, _dp]),
     "s3o_set_edges": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _dp, _dp]),
+    "s3o_add_vertices": (C.c_int, [C.c_void_p, C.c_int, _dp, _up, _dp]),
+    "s3o_add_edges": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _dp, _dp]),
     "s3o_set_estimates": (C.c_int, [C.c_void_p, _dp]),
     "s3o_set_robust": (C.c_int, [C.c_void_p, C.c_int, C.c_double]),
     "s3o_set_jacobian_mode": (C.c_int, [C.c_void_p, C.c_int, C.c_double]),

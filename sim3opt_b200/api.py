@@ -96,6 +96,31 @@ class Problem:
             infop = _d(info)
         self._check(self.L.s3o_set_edges(self.h, self.ne, v0.ctypes.data_as(_ip), v1.ctypes.data_as(_ip), _d(meas), infop))
 
+    def add_vertices(self, est, fixed=None, aux=None):
+        """Append vertices (ids nv, nv+1, ...); the next build_structure merges them into the built graph."""
+        est = _f64(est).reshape(-1, self.est_dim)
+        n = est.shape[0]
+        fx = np.zeros(n, np.uint8) if fixed is None else np.ascontiguousarray(fixed, np.uint8)
+        auxp = None
+        if aux is not None:
+            aux = _f64(aux).reshape(n, 4)
+            auxp = _d(aux)
+        self._check(self.L.s3o_add_vertices(self.h, n, _d(est), fx.ctypes.data_as(_up), auxp))
+        self.nv += n
+
+    def add_edges(self, v0, v1, meas, info=None):
+        """Append edges (caller ids continue from ne); the next build_structure merges them into the built graph."""
+        v0 = np.ascontiguousarray(v0, np.int32)
+        v1 = np.ascontiguousarray(v1, np.int32)
+        n = len(v0)
+        meas = _f64(meas).reshape(-1, self.est_dim)
+        infop = None
+        if info is not None:
+            info = _f64(info).reshape(n, self.d, self.d)
+            infop = _d(info)
+        self._check(self.L.s3o_add_edges(self.h, n, v0.ctypes.data_as(_ip), v1.ctypes.data_as(_ip), _d(meas), infop))
+        self.ne += n
+
     def set_estimates(self, est):
         est = _f64(est).reshape(self.nv, self.est_dim)
         self._check(self.L.s3o_set_estimates(self.h, _d(est)))

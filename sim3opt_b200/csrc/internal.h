@@ -84,6 +84,29 @@ struct DeviceStructure {
 };
 int build_structure_device(cudaStream_t st, int nv, const uint8_t *fixed, const int32_t *hidx_in, int nfree_in, int ne,
                            const int32_t *v0, const int32_t *v1, HostStructure &S, DeviceStructure *keep = nullptr);
+// Device merge of appended vertices and edges into a built structure (s3o_add_vertices / s3o_add_edges, merged by
+// s3o_build_structure).  S, keep and the edge records out equal what build_structure_device and the edge packing give
+// for the concatenated arrays, bit for bit: appended free vertices are numbered n_free_old, n_free_old + 1, ..., and
+// an appended edge sorts after the built edges with the same key.  The built arrays are read, not freed.
+struct StructureMerge {
+    // the built structure: vertices, free vertices, active edges, caller edges; device arrays in sorted order
+    int nv_old = 0, nf_old = 0, na_old = 0, ne_old = 0;
+    const int32_t *hidx = nullptr, *sv0 = nullptr, *sv1 = nullptr, *perm = nullptr;
+    // appended: vertices nv_old..nv-1 (fixed flags, host) and caller edges ne_old..ne-1 (endpoints, host)
+    int nv = 0, ne = 0;
+    const uint8_t *fixed_new = nullptr;
+    const int32_t *v0_new = nullptr, *v1_new = nullptr;
+    // edge records.  Information representations: 0 none (identity), 1 diagonal, 2 full.  Built: SoA planes at pitch
+    // ne_pad_old (d planes when diagonal, d(d+1)/2 packed upper triangles when full).  Appended: caller order, AoS
+    // (est_dim measurement entries; d or d*d information entries), already in the merged representation info_rep.
+    int est_dim = 0, d = 0, ne_pad_old = 0, info_rep_old = 0, info_rep = 0;
+    const double *meas = nullptr, *info = nullptr, *meas_new = nullptr, *info_new = nullptr;
+    // out: the merged records at pitch pad32(active edges) in info_rep (the caller frees them), and the bytes copied
+    // from the host (fixed flags and endpoints of the appended elements)
+    double *meas_out = nullptr, *info_out = nullptr;
+    int64_t h2d_bytes = 0;
+};
+int merge_structure_device(cudaStream_t st, StructureMerge &M, HostStructure &S, DeviceStructure &keep);
 
 // Vertex-range partition of the free vertices across `world` ranks (SURVEY.md section 8e).
 // Rank r owns global Hessian indices [r*seg, min((r+1)*seg, nf)), seg = ceil(nf/world).

@@ -51,10 +51,10 @@ void launch_unpack_vertices(const double *soa, int n, int n_pad, int dim, double
 // information matrix is packed to its upper triangle (row-major, r<=c).
 __global__ void pack_edges_kernel(const double *__restrict__ meas_aos, const double *__restrict__ info_aos,
                                   const int32_t *__restrict__ perm, int ne, int ne_pad, int est_dim, int d, int info_diag,
-                                  double *__restrict__ meas, double *__restrict__ info) {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= ne) return;
-    const size_t o = (size_t)perm[t];
+                                  double *__restrict__ meas, double *__restrict__ info, const int32_t *__restrict__ dst) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= ne) return;
+    const size_t o = (size_t)perm[i], t = dst ? (size_t)dst[i] : (size_t)i;
     for (int k = 0; k < est_dim; ++k) meas[(size_t)k * ne_pad + t] = meas_aos[o * est_dim + k];
     if (info_aos && info_diag) {         // d diagonal entries per edge in, d planes out
         for (int r = 0; r < d; ++r) info[(size_t)r * ne_pad + t] = info_aos[o * d + r];
@@ -65,9 +65,24 @@ __global__ void pack_edges_kernel(const double *__restrict__ meas_aos, const dou
     }
 }
 void launch_pack_edges(const double *meas_aos, const double *info_aos, const int32_t *perm, int ne, int ne_pad,
-                       int est_dim, int d, int info_diag, double *meas, double *info, cudaStream_t st) {
+                       int est_dim, int d, int info_diag, double *meas, double *info, cudaStream_t st, const int32_t *dst) {
     if (ne == 0) return;
-    pack_edges_kernel<<<(ne + 127) / 128, 128, 0, st>>>(meas_aos, info_aos, perm, ne, ne_pad, est_dim, d, info_diag, meas, info);
+    pack_edges_kernel<<<(ne + 127) / 128, 128, 0, st>>>(meas_aos, info_aos, perm, ne, ne_pad, est_dim, d, info_diag, meas, info, dst);
+}
+
+__global__ void convert_info_kernel(const double *__restrict__ src, int n, int d, int rep_src, int rep_dst,
+                                    double *__restrict__ dst) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    for (int r = 0; r < d; ++r) {
+        const double diag = rep_src == 1 ? src[(size_t)k * d + r] : 1.0;
+        if (rep_dst == 1) { dst[(size_t)k * d + r] = diag; continue; }
+        for (int c = 0; c < d; ++c) dst[((size_t)k * d + r) * d + c] = r == c ? diag : 0.0;
+    }
+}
+void launch_convert_info(const double *src, int n, int d, int rep_src, int rep_dst, double *dst, cudaStream_t st) {
+    if (n == 0) return;
+    convert_info_kernel<<<(n + 127) / 128, 128, 0, st>>>(src, n, d, rep_src, rep_dst, dst);
 }
 
 // ======================================================================================

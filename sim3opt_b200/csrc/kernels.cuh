@@ -65,8 +65,13 @@ constexpr int kMaxPartials = 4096;
 // ---- packing ---------------------------------------------------------------------------
 void launch_pack_vertices(const double *aos, int n, int n_pad, int dim, double *soa, cudaStream_t st);
 void launch_unpack_vertices(const double *soa, int n, int n_pad, int dim, double *aos, cudaStream_t st);
+// record perm[t] of the caller-ordered AoS staging to sorted position t, or to dst[t] when dst is given
 void launch_pack_edges(const double *meas_aos, const double *info_aos, const int32_t *perm, int ne, int ne_pad,
-                       int est_dim, int d, int info_diag, double *meas, double *info, cudaStream_t st);
+                       int est_dim, int d, int info_diag, double *meas, double *info, cudaStream_t st,
+                       const int32_t *dst = nullptr);
+// AoS information records of n edges from representation rep_src (0: src ignored, identity; 1: d diagonal entries)
+// to rep_dst (1: d diagonal entries; 2: d x d matrices)
+void launch_convert_info(const double *src, int n, int d, int rep_src, int rep_dst, double *dst, cudaStream_t st);
 
 // ---- per-edge --------------------------------------------------------------------------
 void launch_chi2(const GraphDev &g, double *partials, DevScalars *sc, cudaStream_t st);

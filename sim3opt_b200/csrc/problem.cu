@@ -99,6 +99,9 @@ void free_structure(s3o_problem *p) {
     dev_free(p->d_rowptr); dev_free(p->d_colidx); dev_free(p->d_blk_row); dev_free(p->d_blk_ebeg);
     dev_free(p->d_blk_eend); dev_free(p->d_colT_ptr); dev_free(p->d_colT_blk); dev_free(p->d_inc_ptr);
     dev_free(p->d_inc_ent); dev_free(p->d_e_blk); dev_free(p->d_tile_row); dev_free(p->d_blk_src); dev_free(p->d_multi_blk);
+    dev_free(p->d_perm);
+    // on a built problem the staging holds only appended edges, which mean nothing without the structure they extend
+    if (p->built) { dev_free(p->d_meas_aos); dev_free(p->d_info_aos); }
     dev_free(p->d_ghidx); dev_free(p->d_send_idx); dev_free(p->d_primary); dev_free(p->d_sendbuf); dev_free(p->d_xg);
     dev_free(p->d_H); dev_free(p->d_b); dev_free(p->d_x); dev_free(p->d_r); dev_free(p->d_z); dev_free(p->d_p);
     dev_free(p->d_q1); dev_free(p->d_T); dev_free(p->d_Minv); dev_free(p->d_scratch);
@@ -156,10 +159,18 @@ int sync_scalars(s3o_problem *p) {
 
 namespace {
 
+// vertices or edges appended (s3o_add_vertices / s3o_add_edges) since the structure was built
+bool has_pending(const s3o_problem *p) {
+    return p->built && p->kind <= S3O_KIND_SCALE && (p->nv != p->S.nv || p->ne != p->S.ne);
+}
+
 int ensure_built(s3o_problem *p) {
-    if (p->built) return S3O_OK;
+    if (p->built && !has_pending(p)) return S3O_OK;
     return s3o_build_structure(p, nullptr, nullptr);
 }
+
+// information representation: 0 none (identity), 1 diagonal, 2 full
+inline int info_rep(bool has_info, bool info_diag) { return has_info ? (info_diag ? 1 : 2) : 0; }
 
 bool uses_spmv4(const s3o_problem *p) {
     const int ntiles = (int)p->S.tile_row.size() - 1;
@@ -902,6 +913,34 @@ int s3o_get_vertices_slice(s3o_problem *p, double *est_slice) {
     return S3O_OK;
 }
 
+// Diagonal information matrices (the usual case) are kept as their d diagonal entries.  One threaded pass over the
+// caller's n matrices checks the off-diagonal entries and extracts the diagonals at the same time (the buffer is left
+// uninitialised so that its pages are first touched by the threads that fill them).  Returns the n x d diagonals when
+// every matrix is diagonal, else null.
+static std::unique_ptr<double[]> scan_info_diagonals(int d, int n, const double *info) {
+    const int dd = d * d;
+    const unsigned hw = std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
+    std::unique_ptr<double[]> diag(new double[(size_t)n * d]);
+    double *dst = diag.get();
+    std::vector<char> nondiag(hw, 0);
+    std::vector<std::thread> th;
+    for (unsigned w = 0; w < hw; ++w)
+        th.emplace_back([&, w]() {
+            const size_t lo = (size_t)n * w / hw, hi = (size_t)n * (w + 1) / hw;
+            for (size_t k = lo; k < hi && !nondiag[w]; ++k) {
+                const double *M = info + k * dd;
+                for (int e = 0; e < dd; ++e) {
+                    const int r = e / d, c = e - r * d;
+                    if (r == c) dst[k * d + r] = M[e];
+                    else if (M[e] != 0.0) { nondiag[w] = 1; break; }
+                }
+            }
+        });
+    for (auto &t : th) t.join();
+    for (char f : nondiag) if (f) diag.reset();
+    return diag;
+}
+
 int s3o_set_edges(s3o_problem *p, int n, const int32_t *v0, const int32_t *v1, const double *meas, const double *info) {
     if (!p || n < 0 || (n > 0 && (!v0 || !v1 || !meas))) { set_error("s3o_set_edges: bad arguments"); return S3O_ERR_INVALID; }
     if (p->kind == S3O_KIND_BA) { set_error("s3o_set_edges: a BA problem takes s3o_ba_set_observations"); return S3O_ERR_INVALID; }
@@ -917,33 +956,10 @@ int s3o_set_edges(s3o_problem *p, int n, const int32_t *v0, const int32_t *v1, c
     p->user_ne = n;
     p->has_info = info != nullptr;
     p->info_diag = false;
-    // Diagonal information matrices (the usual case) are kept as their d diagonal entries.  One threaded pass over
-    // the caller's matrices checks the off-diagonal entries and extracts the diagonals at the same time (the buffer
-    // is left uninitialised so that its pages are first touched by the threads that fill them).
     std::unique_ptr<double[]> info_diag_host;
     if (info && n > 0) {
-        const int dd = p->d * p->d, d = p->d;
-        const unsigned hw = std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
-        info_diag_host.reset(new double[(size_t)n * d]);
-        double *dst = info_diag_host.get();
-        std::vector<char> nondiag(hw, 0);
-        std::vector<std::thread> th;
-        for (unsigned w = 0; w < hw; ++w)
-            th.emplace_back([&, w]() {
-                const size_t lo = (size_t)n * w / hw, hi = (size_t)n * (w + 1) / hw;
-                for (size_t k = lo; k < hi && !nondiag[w]; ++k) {
-                    const double *M = info + k * dd;
-                    for (int e = 0; e < dd; ++e) {
-                        const int r = e / d, c = e - r * d;
-                        if (r == c) dst[k * d + r] = M[e];
-                        else if (M[e] != 0.0) { nondiag[w] = 1; break; }
-                    }
-                }
-            });
-        for (auto &t : th) t.join();
-        p->info_diag = true;
-        for (char f : nondiag) if (f) p->info_diag = false;
-        if (!p->info_diag) info_diag_host.reset();
+        info_diag_host = scan_info_diagonals(p->d, n, info);
+        p->info_diag = info_diag_host != nullptr;
     }
     setup_mark("set_edges: info scan");
     std::vector<double> meas_loc, info_loc;
@@ -996,6 +1012,135 @@ int s3o_set_edges(s3o_problem *p, int n, const int32_t *v0, const int32_t *v1, c
     S3O_CUDA(cudaStreamSynchronize(p->stream));
     setup_mark("set_edges: upload");
     p->stats.n_edges = p->user_ne;
+    return S3O_OK;
+}
+
+// ---- growing a graph (g2o SparseOptimizer::updateInitialization) --------------------------------
+static int check_growable(const s3o_problem *p, const char *who) {
+    if (p->kind == S3O_KIND_BA) {
+        set_error("%s: bundle adjustment marginalises its points, and g2o's BlockSolver::updateStructure does not grow such "
+                  "graphs either; build the problem again", who);
+        return S3O_ERR_UNSUPPORTED;
+    }
+    if (p->kind > S3O_KIND_SCALE) { set_error("%s: not a pose-graph problem", who); return S3O_ERR_INVALID; }
+    if (p->dist) { set_error("%s: the partitioned solve cannot grow its graph; call s3o_set_vertices / s3o_set_edges", who); return S3O_ERR_UNSUPPORTED; }
+    return S3O_OK;
+}
+
+int s3o_add_vertices(s3o_problem *p, int n, const double *est, const uint8_t *fixed, const double *aux) {
+    if (!p || n < 0 || (n > 0 && !est)) { set_error("s3o_add_vertices: bad arguments"); return S3O_ERR_INVALID; }
+    int rc = check_growable(p, "s3o_add_vertices");
+    if (rc) return rc;
+    if (p->kind == S3O_KIND_SCALE_TRANS && !aux && n > 0) { set_error("s3o_add_vertices: SCALE_TRANS needs aux rotations"); return S3O_ERR_INVALID; }
+    if (n == 0) return S3O_OK;
+    if (!p->d_est[0]) return s3o_set_vertices(p, n, est, fixed, aux);
+    if (p->nv > 0 && p->has_aux != (aux != nullptr)) { set_error("s3o_add_vertices: aux must be given for every vertex or for none"); return S3O_ERR_INVALID; }
+    cudaSetDevice(p->device);
+    const int nv_old = p->nv, nv = nv_old + n, pad = pad32(nv), ed = p->est_dim;
+    // planes at the pitch of a fresh s3o_set_vertices; the current estimates are copied on the device
+    double *est_new[2] = { nullptr, nullptr }, *aux_new = nullptr, *tmp = nullptr;
+    auto release = [&]() { dev_free(est_new[0]); dev_free(est_new[1]); dev_free(aux_new); dev_free(tmp); };
+    rc = dev_alloc(&est_new[0], (size_t)pad * ed);
+    rc = rc ? rc : dev_alloc(&est_new[1], (size_t)pad * ed);
+    rc = rc ? rc : dev_alloc(&tmp, (size_t)n * std::max(ed, aux ? 4 : 0));
+    if (aux) rc = rc ? rc : dev_alloc(&aux_new, (size_t)pad * 4);
+    if (rc) { release(); return rc; }
+    cudaStream_t st = p->stream;
+    cudaMemsetAsync(est_new[0], 0, (size_t)pad * ed * sizeof(double), st);
+    cudaMemsetAsync(est_new[1], 0, (size_t)pad * ed * sizeof(double), st);
+    cudaMemcpy2DAsync(est_new[0], (size_t)pad * sizeof(double), p->d_est[p->cur], (size_t)p->nv_pad * sizeof(double),
+                      (size_t)nv_old * sizeof(double), ed, cudaMemcpyDeviceToDevice, st);
+    cudaMemcpyAsync(tmp, est, (size_t)n * ed * sizeof(double), cudaMemcpyHostToDevice, st);
+    launch_pack_vertices(tmp, n, pad, ed, est_new[0] + nv_old, st);
+    if (aux) {
+        cudaMemsetAsync(aux_new, 0, (size_t)pad * 4 * sizeof(double), st);
+        cudaMemcpy2DAsync(aux_new, (size_t)pad * sizeof(double), p->d_aux, (size_t)p->nv_pad * sizeof(double),
+                          (size_t)nv_old * sizeof(double), 4, cudaMemcpyDeviceToDevice, st);
+        cudaMemcpyAsync(tmp, aux, (size_t)n * 4 * sizeof(double), cudaMemcpyHostToDevice, st);
+        launch_pack_vertices(tmp, n, pad, 4, aux_new + nv_old, st);
+    }
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    dev_free(tmp);
+    if (e != cudaSuccess) { release(); set_error("s3o_add_vertices: %s", cudaGetErrorString(e)); return S3O_ERR_CUDA; }
+    dev_free(p->d_est[0]); dev_free(p->d_est[1]); dev_free(p->d_aux);
+    p->d_est[0] = est_new[0]; p->d_est[1] = est_new[1]; p->d_aux = aux_new;
+    p->cur = 0;
+    p->nv = nv;
+    p->nv_pad = pad;
+    p->fixed.resize(nv, 0);
+    if (fixed) memcpy(p->fixed.data() + nv_old, fixed, n);
+    // what s3o_set_vertices drops: the LM state, the snapshot (at the old pitch) and the staging buffer (sized by nv)
+    p->lm_valid = false;
+    p->linearized = false;
+    dev_free(p->d_est_snap);
+    dev_free(p->d_stage);
+    p->stats.h2d_bytes += (int64_t)n * ed * sizeof(double) + (aux ? (int64_t)n * 32 : 0);
+    p->stats.kernel_launches += aux ? 2 : 1;
+    p->stats.n_vertices = nv;
+    return S3O_OK;
+}
+
+int s3o_add_edges(s3o_problem *p, int n, const int32_t *v0, const int32_t *v1, const double *meas, const double *info) {
+    if (!p || n < 0 || (n > 0 && (!v0 || !v1 || !meas))) { set_error("s3o_add_edges: bad arguments"); return S3O_ERR_INVALID; }
+    int rc = check_growable(p, "s3o_add_edges");
+    if (rc) return rc;
+    for (int k = 0; k < n; ++k)
+        if (v0[k] < 0 || v0[k] >= p->nv || v1[k] < 0 || v1[k] >= p->nv || v0[k] == v1[k]) {
+            set_error("s3o_add_edges: edge %d has invalid vertices (%d,%d), n_vertices=%d", k, v0[k], v1[k], p->nv);
+            return S3O_ERR_INVALID;
+        }
+    if (n == 0) return S3O_OK;
+    if (!p->built && p->ne > 0 && !p->d_meas_aos) { set_error("s3o_add_edges: the edges were consumed; call s3o_set_edges again"); return S3O_ERR_INVALID; }
+    cudaSetDevice(p->device);
+    setup_mark(nullptr);
+    // information representation of the grown graph: a NULL matrix counts as identity once any edge has one
+    std::unique_ptr<double[]> diag_host;
+    if (info) diag_host = scan_info_diagonals(p->d, n, info);
+    const int rep_old = p->ne > 0 ? info_rep(p->has_info, p->info_diag) : 0;
+    const int rep_new = info ? (diag_host ? 1 : 2) : 0;
+    const int rep = (rep_old == 0 && rep_new == 0) ? 0 : std::max(std::max(rep_old, 1), std::max(rep_new, 1));
+    setup_mark("add_edges: info scan");
+    // new staging = the staged records (in rep_old, converted to rep) followed by the appended ones
+    const int staged = p->built ? p->ne - p->S.ne : p->ne, d = p->d, ed = p->est_dim;
+    const int w = rep == 1 ? d : d * d, w_new = rep_new == 1 ? d : d * d;
+    const double *isrc = rep_new == 1 ? diag_host.get() : info;
+    double *meas_s = nullptr, *info_s = nullptr, *tmp = nullptr;
+    auto release = [&]() { dev_free(meas_s); dev_free(info_s); dev_free(tmp); };
+    rc = dev_alloc(&meas_s, (size_t)(staged + n) * ed);
+    if (rep) rc = rc ? rc : dev_alloc(&info_s, (size_t)(staged + n) * w);
+    if (rep_new && rep_new != rep) rc = rc ? rc : dev_alloc(&tmp, (size_t)n * w_new);
+    if (rc) { release(); return rc; }
+    cudaStream_t st = p->stream;
+    if (staged) cudaMemcpyAsync(meas_s, p->d_meas_aos, (size_t)staged * ed * sizeof(double), cudaMemcpyDeviceToDevice, st);
+    cudaMemcpyAsync(meas_s + (size_t)staged * ed, meas, (size_t)n * ed * sizeof(double), cudaMemcpyHostToDevice, st);
+    if (rep) {
+        if (staged && rep_old == rep) cudaMemcpyAsync(info_s, p->d_info_aos, (size_t)staged * w * sizeof(double), cudaMemcpyDeviceToDevice, st);
+        else if (staged) launch_convert_info(rep_old ? p->d_info_aos : nullptr, staged, d, rep_old, rep, info_s, st);
+        double *dst = info_s + (size_t)staged * w;
+        if (rep_new == rep) cudaMemcpyAsync(dst, isrc, (size_t)n * w * sizeof(double), cudaMemcpyHostToDevice, st);
+        else {
+            if (rep_new) cudaMemcpyAsync(tmp, isrc, (size_t)n * w_new * sizeof(double), cudaMemcpyHostToDevice, st);
+            launch_convert_info(tmp, n, d, rep_new, rep, dst, st);
+        }
+    }
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    dev_free(tmp);
+    if (e != cudaSuccess) { release(); set_error("s3o_add_edges: %s", cudaGetErrorString(e)); return S3O_ERR_CUDA; }
+    dev_free(p->d_meas_aos); dev_free(p->d_info_aos);
+    p->d_meas_aos = meas_s;
+    p->d_info_aos = info_s;
+    p->has_info = rep > 0;
+    p->info_diag = rep == 1;
+    p->v0.insert(p->v0.end(), v0, v0 + n);
+    p->v1.insert(p->v1.end(), v1, v1 + n);
+    p->ne += n;
+    p->user_ne = p->ne;
+    p->linearized = false;
+    p->stats.h2d_bytes += (int64_t)n * ed * sizeof(double) + (rep_new ? (int64_t)n * w_new * sizeof(double) : 0);
+    p->stats.n_edges = p->ne;
+    setup_mark("add_edges: upload");
     return S3O_OK;
 }
 
@@ -1077,6 +1222,59 @@ int s3o_set_pcg(s3o_problem *p, double rel_tol, int max_iter) {
     if (!p) return S3O_ERR_INVALID;
     if (rel_tol > 0) p->pcg_tol = rel_tol;
     if (max_iter > 0) p->pcg_max_iter = max_iter;
+    return S3O_OK;
+}
+
+// g2o BlockSolver::updateStructure: merges the vertices and edges appended since the last build into the built
+// structure on the device (structure_dev.cu), then rebuilds what a fresh build derives from it -- H and the vectors,
+// the SpMV tiles, the multilevel hierarchy -- and drops the factorisation plan and the LM state, as s3o_set_vertices
+// does.  The existing edges' records never cross PCIe.
+static int merge_structure(s3o_problem *p) {
+    setup_mark(nullptr);
+    StructureMerge M;
+    const HostStructure &S0 = p->S;
+    M.nv_old = S0.nv; M.nf_old = S0.nf; M.na_old = S0.ne_act; M.ne_old = S0.ne;
+    M.hidx = p->d_hidx; M.sv0 = p->d_sv0; M.sv1 = p->d_sv1; M.perm = p->d_perm;
+    M.nv = p->nv; M.ne = p->ne;
+    M.fixed_new = p->fixed.data() + M.nv_old;
+    M.v0_new = p->v0.data() + M.ne_old; M.v1_new = p->v1.data() + M.ne_old;
+    M.est_dim = p->est_dim; M.d = p->d; M.ne_pad_old = p->ne_pad;
+    M.info_rep_old = p->built_info_rep; M.info_rep = info_rep(p->has_info, p->info_diag);
+    M.meas = p->d_meas; M.info = p->d_info; M.meas_new = p->d_meas_aos; M.info_new = p->d_info_aos;
+    HostStructure S;
+    DeviceStructure dev;
+    int rc = merge_structure_device(p->stream, M, S, dev);
+    if (rc) return rc;
+    p->stats.h2d_bytes += M.h2d_bytes;
+    free_structure(p);          // the old arrays, the staging, the factorisation plan and the hierarchy
+    p->S = std::move(S);
+    p->d_hidx = dev.hidx; p->d_sv0 = dev.sv0; p->d_sv1 = dev.sv1; p->d_blk_ebeg = dev.blk_ebeg; p->d_blk_eend = dev.blk_eend;
+    p->d_blk_src = dev.blk_src; p->d_multi_blk = dev.multi_blk; p->d_inc_ptr = dev.inc_ptr; p->d_inc_ent = dev.inc_ent;
+    p->d_e_blk = dev.e_blk; p->d_rowptr = dev.rowptr; p->d_colidx = dev.colidx; p->d_blk_row = dev.blk_row;
+    p->d_colT_ptr = dev.colT_ptr; p->d_colT_blk = dev.colT_blk; p->d_perm = dev.perm;
+    p->d_meas = M.meas_out;
+    p->d_info = M.info_out;
+    p->built_info_rep = M.info_rep;
+    p->ne_pad = pad32(p->S.ne_act);
+    p->lm_valid = false;
+    dev_free(p->d_est_snap);
+    rc = upload_structure_arrays(p, p->S.nf, true);
+    rc = rc ? rc : alloc_linear_system(p);
+    rc = rc ? rc : dev_alloc(&p->d_scratch, (size_t)p->ne_pad * scratch_stride(p->d));
+    if (rc) { free_structure(p); return rc; }
+    cudaMemsetAsync(p->d_x, 0, (size_t)p->S.nf * p->d * sizeof(double), p->stream);
+    cudaError_t e = cudaStreamSynchronize(p->stream);
+    if (e != cudaSuccess || (e = cudaGetLastError()) != cudaSuccess) {
+        set_error("s3o_build_structure (merge): %s", cudaGetErrorString(e));
+        free_structure(p);
+        return S3O_ERR_CUDA;
+    }
+    p->stats.kernel_launches += 1;
+    setup_mark("merge: uploads + allocations");
+    p->built = true;
+    p->stats.n_free = p->S.nf; p->stats.n_blocks = p->S.nb;
+    if (wants_multilevel(p) && (rc = amg_setup(p))) return rc;
+    setup_mark("merge: hierarchy");
     return S3O_OK;
 }
 
@@ -1166,7 +1364,8 @@ int s3o_build_structure(s3o_problem *p, int *n_free, int *n_blocks) {
         }
         cudaMemsetAsync(p->d_x, 0, nfd * sizeof(double), p->stream);
         cudaError_t e = cudaStreamSynchronize(p->stream);
-        dev_free(d_perm);
+        p->d_perm = d_perm;
+        p->built_info_rep = info_rep(p->has_info, p->info_diag);
         if (e != cudaSuccess || (e = cudaGetLastError()) != cudaSuccess) {
             set_error("s3o_build_structure: %s", cudaGetErrorString(e));
             free_structure(p);
@@ -1181,6 +1380,9 @@ int s3o_build_structure(s3o_problem *p, int *n_free, int *n_blocks) {
         // the aggregation hierarchy is structure work too: build it here rather than inside the first solve
         if (wants_multilevel(p) && (rc = amg_setup(p))) return rc;
         setup_mark("structure: hierarchy total");
+    } else if (has_pending(p)) {
+        int rc = merge_structure(p);
+        if (rc) return rc;
     }
     if (n_free) *n_free = p->S.nf;
     if (n_blocks) *n_blocks = p->S.nb;
@@ -1272,6 +1474,7 @@ int s3o_host_direct_plan(int n_vertices, const uint8_t *fixed, int n_edges, cons
 }
 
 int s3o_get_structure(s3o_problem *p, int32_t *colptr, int32_t *rowidx) {
+    if (p && has_pending(p)) { cudaSetDevice(p->device); int rc = ensure_built(p); if (rc) return rc; }
     if (!p || !p->built) { set_error("s3o_get_structure: structure not built"); return S3O_ERR_INVALID; }
     if (colptr) memcpy(colptr, p->S.ccs_colptr.data(), sizeof(int32_t) * (p->S.nf + 1));
     if (rowidx) memcpy(rowidx, p->S.ccs_rowidx.data(), sizeof(int32_t) * p->S.nb);
@@ -1279,6 +1482,7 @@ int s3o_get_structure(s3o_problem *p, int32_t *colptr, int32_t *rowidx) {
 }
 
 int s3o_get_hessian_index(s3o_problem *p, int32_t *hidx) {
+    if (p && has_pending(p)) { cudaSetDevice(p->device); int rc = ensure_built(p); if (rc) return rc; }
     if (!p || !p->built || !hidx) { set_error("s3o_get_hessian_index: structure not built"); return S3O_ERR_INVALID; }
     memcpy(hidx, p->S.hidx.data(), sizeof(int32_t) * p->nv);
     return S3O_OK;
@@ -1454,7 +1658,7 @@ int direct_hook_check(s3o_problem *p, const char *who) {
     if (p->dist) { set_error("%s: not available in the partitioned solve", who); return S3O_ERR_UNSUPPORTED; }
     if (!p->built) { set_error("%s: no structure yet (s3o_build_structure, or a first s3o_linsolver_solve)", who); return S3O_ERR_INVALID; }
     cudaSetDevice(p->device);
-    return S3O_OK;
+    return ensure_built(p);
 }
 }  // namespace
 

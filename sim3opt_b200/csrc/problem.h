@@ -49,7 +49,10 @@ struct s3o_problem {
     std::vector<uint8_t> fixed;
     std::vector<int32_t> v0, v1;
     bool has_info = false, has_aux = false, info_diag = false;
-    double *d_meas_aos = nullptr, *d_info_aos = nullptr;  // caller-ordered staging until the structure is built
+    // caller-ordered staging of the edge records until the structure is built; on a built problem, of the edges
+    // appended since (s3o_add_edges), until the next build merges them.  has_info / info_diag describe the staged
+    // records and, once merged or built, the whole graph
+    double *d_meas_aos = nullptr, *d_info_aos = nullptr;
     // device graph
     int nv_pad = 0, ne_pad = 0;
     double *d_est[2] = { nullptr, nullptr };
@@ -64,6 +67,8 @@ struct s3o_problem {
     int32_t *d_colT_ptr = nullptr, *d_colT_blk = nullptr, *d_inc_ptr = nullptr, *d_inc_ent = nullptr, *d_e_blk = nullptr;
     int32_t *d_tile_row = nullptr;
     int32_t *d_blk_src = nullptr, *d_multi_blk = nullptr;
+    int32_t *d_perm = nullptr;              // [ne_act] sorted position -> caller edge (read by the merge)
+    int built_info_rep = 0;                 // information in d_info: 0 none, 1 diagonal planes, 2 packed triangles
     // partitioned solve (one process per GPU, NCCL): s3o_set_comm
     Comm comm;
     bool dist = false;
